@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — 2-opt move evaluations per second on the BASELINE.json headline workload.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (config.workload): synthetic uniform EUC_2D instance uni<n> (n = 100000, SURVEY.md §8(c) generator),
 nearest-neighbour start tour built on the GPU, best-improvement 2-opt with on-the-fly distances.
@@ -19,12 +19,17 @@ obtained by replaying the committed single-GPU move log tests/golden/uni100000_b
 --impl reference times the reference's own CPU code (oracle/_ref: its calc_dist and x_udir_pos driven over rows of one
 best-improvement scan exactly like src/tabusearch.c:126-156, all host threads) on the same instance and start tour, and the
 stock single-thread alg_2opt_tabu() on uni2000 next to it.
+--dump-outputs DIR writes what the timed passes returned to a caller (tour and cost after the last step, pass counters) as
+float64 .npy files, so that two builds can be compared output for output on the same seeded inputs.
+Nothing is written into the repository tree; the CPU nearest-neighbour tour of an uncommitted size is cached in the
+system's temporary directory.
 """
 import argparse
 import hashlib
 import json
 import os
 import sys
+import tempfile
 import threading
 import time
 
@@ -33,6 +38,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ from the imports below
 
 METRIC = "2opt_move_evals_per_sec"
 UNIT = "evals/s"
@@ -54,7 +60,11 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip ga_batch / matrix roofline / per-pass breakdown")
     ap.add_argument("--rows-per-thread", type=int, default=0)
     ap.add_argument("--tile-cols", type=int, default=0)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed path's outputs of its last step as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def workload_config(n: int) -> dict:
@@ -245,16 +255,26 @@ def start_tour_cpu_or_cached(xy, n):
     fixture = os.path.join(ROOT, "tests", "golden", f"nn_uni{n}.npz")
     if os.path.exists(fixture):
         return np.load(fixture)["succ"].astype(np.int32)
-    cache = os.path.join(ROOT, "gpurun_out", f"nn_uni{n}.npy")
+    cache = nn_cache_path(n)
     if os.path.exists(cache):
         return np.load(cache)
     succ, _ = Oracle().nn_tour(xy, 0, 0)
     try:
-        os.makedirs(os.path.dirname(cache), exist_ok=True)
         np.save(cache, succ)
     except OSError:
         pass
     return succ
+
+
+def nn_cache_path(n: int) -> str:
+    return os.path.join(tempfile.gettempdir(), f"tspb200_bench_nn_uni{n}.npy")
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """DIR/<name>.npy for every array, as float64 (tour indices < 2^53 stay exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, dtype=np.float64))
 
 
 class TourFixture:
@@ -347,8 +367,7 @@ def main():
     nn_s = time.perf_counter() - t0
     if rank == 0:
         try:
-            os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-            np.save(os.path.join(ROOT, "gpurun_out", f"nn_uni{n}.npy"), succ0)
+            np.save(nn_cache_path(n), succ0)
         except OSError:
             pass
     fixture = TourFixture(n, succ0)
@@ -383,14 +402,14 @@ def main():
     value = done_passes * pairs / (gpu_ms * 1e-3)
     # the tile shape / grid `value` was measured with (later legs — pruned runs, other sizes — re-plan the tiles)
     shape_value = {k: eng.info(k) for k in ("block_threads", "rows_per_thread", "tile_cols", "grid_bi", "ntiles", "row_shuffle", "tile_rows")}
-    tour_after, _ = eng.tour_download()
+    tour_after, cost_after = eng.tour_download()
     chk_value = fixture.check_after_passes(tour_after, args.warmup + done_passes)
     clocks = sampler.stop(t_region0, t_region1)
 
     # ---- e2e: host buffers through the C-ABI, copies inside the timed region -------------------------------
     h_xy = pinned(xy)
     h_succ = pinned(succ0.astype(np.int32))
-    e2e_passes = max(1, args.steps)
+    e2e_passes = args.steps
     eng.set_instance(h_xy, 0)           # warm-up of the same call sequence
     eng.two_opt(BI, h_succ, 0.0, max_iters=2)
     barrier()
@@ -408,7 +427,7 @@ def main():
     # K calls of tspb200_two_opt(max_iters = 1): each uploads the step's input tour from pinned host memory (4n bytes),
     # runs one pass, downloads the resulting tour and its cost (4n + 8 bytes), which is the next step's input.  The
     # instance (coordinates) stays resident like any constant of the job.
-    step_calls = max(1, min(args.steps, 50))
+    step_calls = args.steps
     cur = h_succ.copy()
     eng.two_opt(BI, cur, 0.0, max_iters=1)
     barrier()
@@ -635,6 +654,9 @@ def main():
     if tlo and tlo.get("pruned", {}).get("tour_check", {}).get("check") == "MISMATCH":
         bad.append("time_to_local_optimum.pruned")
     line["self_check"] = "ok" if not bad else "MISMATCH in " + ", ".join(bad)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tour_succ": tour_after, "tour_cost": [cost_after],
+                                         "pass_stats": [done_passes, moves, st.evals, st.obj_delta]})
     print(json.dumps(line), flush=True)
     eng.close()
     if world > 1:

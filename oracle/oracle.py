@@ -22,6 +22,8 @@ ORACLE_SO = os.path.join(_HERE, "_build", "libtsporacle.so")
 REF_SO = os.path.join(_HERE, "_ref", "libtspref.so")
 #: the same reference objects linked against the product's drop-in symbols (oracle/Makefile, INTEGRATION.md §2)
 REF_GPU_SO = os.path.join(_HERE, "_ref", "libtspref_gpu.so")
+#: the reference's drivers restated on the drop-in header, linked against libtspb200_dropin.so (oracle/dropin_callers.c)
+CALLERS_SO = os.path.join(_HERE, "_build", "libdropin_callers.so")
 
 EUC_2D, MAX_2D, MAN_2D, CEIL_2D, GEO, ATT = 0, 1, 2, 3, 4, 5
 
@@ -187,46 +189,19 @@ class Oracle:
         return ev, sec.value, (bd.value, bi.value, bj.value)
 
 
-class RefLib:
-    """The unmodified reference, compiled.  Raises FileNotFoundError when oracle/_ref is absent."""
+class _InstanceLib:
+    """A library that keeps reference `instance`s through the refshim_* calls and exports the reference's driver symbols."""
 
-    LAYOUT_KEYS = ["sizeof_instance", "off_time_limit", "off_integer_cost", "off_perf_prof", "off_nodes",
-                   "off_num_nodes", "off_weight_type", "off_num_columns", "off_obj_best", "off_edges",
-                   "sizeof_point", "sizeof_edge", "off_verbose", "off_seed"]
-
-    def __init__(self, gpu_link: bool = False):
-        """gpu_link=True loads libtspref_gpu.so: the reference's callers run unmodified, but calc_dist / alg_2opt /
-        alg_2opt_tabu / reverse_path resolve to the product's CUDA-backed definitions (needs a GPU at call time)."""
-        build()
-        so = REF_GPU_SO if gpu_link else REF_SO
-        if not os.path.exists(so):
-            raise FileNotFoundError(so)
-        L = C.CDLL(so)
+    def _bind_instance_calls(self, L):
         L.refshim_new.restype = C.c_void_p
         L.refshim_new.argtypes = [C.c_int, _f64p, C.c_int]
-        L.refshim_parse.restype = C.c_void_p
-        L.refshim_parse.argtypes = [C.c_char_p]
         L.refshim_free.argtypes = [C.c_void_p]
         L.refshim_num_nodes.argtypes = [C.c_void_p]
-        L.refshim_weight_type.argtypes = [C.c_void_p]
         L.refshim_obj.restype = C.c_double
         L.refshim_obj.argtypes = [C.c_void_p]
-        L.refshim_set_obj.argtypes = [C.c_void_p, C.c_double]
-        L.refshim_get_xy.argtypes = [C.c_void_p, _f64p]
         L.refshim_get_succ.argtypes = [C.c_void_p, _i32p]
         L.refshim_set_succ.argtypes = [C.c_void_p, _i32p]
-        L.refshim_dist_matrix.argtypes = [C.c_void_p, _i32p]
-        L.refshim_layout.argtypes = [C.POINTER(C.c_int64), C.c_int]
-        L.refshim_bi_scan_rows_mt.restype = C.c_int64
-        L.refshim_bi_scan_rows_mt.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double),
-                                              C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
-        # the reference's own entry points
-        L.calc_dist.restype = C.c_double
-        L.calc_dist.argtypes = [C.c_int, C.c_int, C.c_void_p]
-        L.greedy.argtypes = [C.c_void_p, C.c_int]
-        L.alg_2opt.argtypes = [C.c_void_p]
         L.alg_2opt_tabu.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int]
-        L.reverse_path.argtypes = [C.c_void_p, C.c_int, C.c_int, _i32p]
         self.L = L
 
     def run_method(self, name: str, xy, wt, time_limit: int = -1):
@@ -244,14 +219,82 @@ class RefLib:
         self.free(h)
         return out
 
+    def new(self, xy, wt):
+        xy = _as_xy(xy)
+        return self.L.refshim_new(len(xy), xy, wt)
+
+    def free(self, h):
+        self.L.refshim_free(h)
+
+    def get_succ(self, h) -> np.ndarray:
+        succ = np.empty(self.L.refshim_num_nodes(h), dtype=np.int32)
+        self.L.refshim_get_succ(h, succ)
+        return succ
+
+    def two_opt_bi(self, xy, wt, succ, skip_edge=None, iter_=1, tenure=1, want_prev=False):
+        """alg_2opt_tabu(inst, skip_edge, stored_prev, iter, tenure); returns (succ, obj_best[, prev])."""
+        h = self.new(xy, wt)
+        n = self.L.refshim_num_nodes(h)
+        self.L.refshim_set_succ(h, np.ascontiguousarray(succ, dtype=np.int32))
+        prev = np.empty(n, dtype=np.int32) if want_prev else None
+        self.L.alg_2opt_tabu(h, skip_edge.ctypes.data if skip_edge is not None else None,
+                             prev.ctypes.data if prev is not None else None, iter_, tenure)
+        out = (self.get_succ(h), self.L.refshim_obj(h)) + ((prev,) if want_prev else ())
+        self.free(h)
+        return out
+
+
+class DropinCallers(_InstanceLib):
+    """oracle/dropin_callers.c -> oracle/_build/libdropin_callers.so: the reference drivers HEU_greedy / HEU_2opt_greedy /
+    HEU_2opt_greedy_iter / HEU_2opt_extramileage restated on top of libtspb200_dropin.so (needs a GPU at call time).
+    Raises FileNotFoundError when it is not built."""
+
+    def __init__(self):
+        build()
+        if not os.path.exists(CALLERS_SO):  # an oracle built before the product library has no callers library yet
+            subprocess.run(["make", "-C", _HERE, "callers"], check=True, stdout=subprocess.DEVNULL)
+        if not os.path.exists(CALLERS_SO):
+            raise FileNotFoundError(CALLERS_SO)
+        self._bind_instance_calls(C.CDLL(CALLERS_SO))
+
+
+class RefLib(_InstanceLib):
+    """The unmodified reference, compiled.  Raises FileNotFoundError when oracle/_ref is absent."""
+
+    LAYOUT_KEYS = ["sizeof_instance", "off_time_limit", "off_integer_cost", "off_perf_prof", "off_nodes",
+                   "off_num_nodes", "off_weight_type", "off_num_columns", "off_obj_best", "off_edges",
+                   "sizeof_point", "sizeof_edge", "off_verbose", "off_seed"]
+
+    def __init__(self, gpu_link: bool = False):
+        """gpu_link=True loads libtspref_gpu.so: the reference's callers run unmodified, but calc_dist / alg_2opt /
+        alg_2opt_tabu / reverse_path resolve to the product's CUDA-backed definitions (needs a GPU at call time)."""
+        build()
+        so = REF_GPU_SO if gpu_link else REF_SO
+        if not os.path.exists(so):
+            raise FileNotFoundError(so)
+        L = C.CDLL(so)
+        self._bind_instance_calls(L)
+        L.refshim_parse.restype = C.c_void_p
+        L.refshim_parse.argtypes = [C.c_char_p]
+        L.refshim_weight_type.argtypes = [C.c_void_p]
+        L.refshim_set_obj.argtypes = [C.c_void_p, C.c_double]
+        L.refshim_get_xy.argtypes = [C.c_void_p, _f64p]
+        L.refshim_dist_matrix.argtypes = [C.c_void_p, _i32p]
+        L.refshim_layout.argtypes = [C.POINTER(C.c_int64), C.c_int]
+        L.refshim_bi_scan_rows_mt.restype = C.c_int64
+        L.refshim_bi_scan_rows_mt.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double),
+                                              C.POINTER(C.c_int64), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
+        # the reference's own entry points
+        L.calc_dist.restype = C.c_double
+        L.calc_dist.argtypes = [C.c_int, C.c_int, C.c_void_p]
+        L.greedy.argtypes = [C.c_void_p, C.c_int]
+        L.alg_2opt.argtypes = [C.c_void_p]
+        L.reverse_path.argtypes = [C.c_void_p, C.c_int, C.c_int, _i32p]
+
     def layout(self) -> dict:
         buf = (C.c_int64 * 32)()
         k = self.L.refshim_layout(buf, 32)
         return {name: int(buf[t]) for t, name in zip(range(k), self.LAYOUT_KEYS)}
-
-    def new(self, xy, wt):
-        xy = _as_xy(xy)
-        return self.L.refshim_new(len(xy), xy, wt)
 
     def parse(self, path: str):
         """Reference TSPLIB parser -> (xy, weight_type). weight_type -1 (unset) is returned as is."""
@@ -263,9 +306,6 @@ class RefLib:
         self.L.refshim_free(h)
         return xy, wt
 
-    def free(self, h):
-        self.L.refshim_free(h)
-
     def dist_matrix(self, xy, wt) -> np.ndarray:
         h = self.new(xy, wt)
         n = len(_as_xy(xy))
@@ -273,11 +313,6 @@ class RefLib:
         self.L.refshim_dist_matrix(h, out)
         self.free(h)
         return out
-
-    def get_succ(self, h) -> np.ndarray:
-        succ = np.empty(self.L.refshim_num_nodes(h), dtype=np.int32)
-        self.L.refshim_get_succ(h, succ)
-        return succ
 
     def nn_tour(self, xy, wt, start=0):
         h = self.new(xy, wt)
@@ -293,18 +328,6 @@ class RefLib:
         self.L.refshim_set_obj(h, obj)
         self.L.alg_2opt(h)
         out = self.get_succ(h), self.L.refshim_obj(h)
-        self.free(h)
-        return out
-
-    def two_opt_bi(self, xy, wt, succ, skip_edge=None, iter_=1, tenure=1, want_prev=False):
-        """alg_2opt_tabu(inst, skip_edge, stored_prev, iter, tenure); returns (succ, obj_best[, prev])."""
-        h = self.new(xy, wt)
-        n = self.L.refshim_num_nodes(h)
-        self.L.refshim_set_succ(h, np.ascontiguousarray(succ, dtype=np.int32))
-        prev = np.empty(n, dtype=np.int32) if want_prev else None
-        self.L.alg_2opt_tabu(h, skip_edge.ctypes.data if skip_edge is not None else None,
-                             prev.ctypes.data if prev is not None else None, iter_, tenure)
-        out = (self.get_succ(h), self.L.refshim_obj(h)) + ((prev,) if want_prev else ())
         self.free(h)
         return out
 

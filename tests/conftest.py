@@ -49,6 +49,22 @@ def goldens():
 
 
 @pytest.fixture(scope="session")
+def reference_outputs():
+    """stored results of the reference's functions on the inputs of the tests that compare with them; their provenance is
+    the file's "source" (tests/golden/make_reference_outputs.py)"""
+    with open(os.path.join(GOLD_DIR, "reference_outputs.json")) as f:
+        return json.load(f)
+
+
+@pytest.fixture(scope="session")
+def reflib_if_built():
+    """the compiled reference when oracle/_ref is built (make -C oracle REF=<checkout>), else None: the tests that check
+    reference_outputs compare with it directly as well"""
+    from oracle.oracle import RefLib, have_ref
+    return RefLib() if have_ref() else None
+
+
+@pytest.fixture(scope="session")
 def instances():
     z = np.load(os.path.join(GOLD_DIR, "instances.npz"))
     out = {}

@@ -1,6 +1,7 @@
 """CPU tests: the oracle restatement (oracle/tsp_oracle.c) against (a) the committed golden fixtures that
 were generated from the unmodified reference, (b) the reference's own published CSV goldens, and (c) the
-compiled reference itself when oracle/_ref is present."""
+stored results of the reference's functions on further inputs (tests/golden/reference_outputs.json, provenance in its
+"source"), and the compiled reference itself when oracle/_ref is built."""
 import hashlib
 
 import numpy as np
@@ -84,52 +85,55 @@ def test_berlin52_move_logs(oracle, instances, goldens):
     assert is_tour(bs) and is_tour(fs)
 
 
-def test_oracle_equals_compiled_reference(oracle, reflib, instances):
+def test_oracle_equals_compiled_reference(oracle, instances, goldens, reference_outputs, reflib_if_built):
+    """the reference's matrix, NN, FI and BI results (goldens.json) and the prev[] alg_2opt_tabu exports (tabusearch.c:173-175)"""
     for nm in ["berlin52", "att48", "ulysses22", "pr299", "gr96"]:
         xy, wt = instances[nm]
-        assert (oracle.dist_matrix(xy, wt) == reflib.dist_matrix(xy, wt)).all()
+        g = goldens["instances"][nm]
+        assert sha(oracle.dist_matrix(xy, wt)) == g["matrix_sha256"], nm
         s1, c1 = oracle.nn_tour(xy, wt, 0)
-        s2, c2 = reflib.nn_tour(xy, wt, 0)
-        assert (s1 == s2).all() and c1 == c2
+        assert sha(s1) == g["nn_sha256"] and c1 == g["nn_cost"], nm
         f1 = oracle.two_opt_fi(xy, wt, s1, c1)
-        f2 = reflib.two_opt_fi(xy, wt, s1, c1)
-        assert (f1[0] == f2[0]).all() and f1[1] == f2[1]
+        assert sha(f1[0]) == g["fi_sha256"] and f1[1] == g["fi_cost"], nm
         b1 = oracle.two_opt_bi(xy, wt, s1, want_prev=True)
-        b2 = reflib.two_opt_bi(xy, wt, s1, want_prev=True)
-        assert (b1[0] == b2[0]).all() and b1[1] == b2[1] and (b1[4] == b2[2]).all()
+        assert sha(b1[0]) == g["bi_sha256"] and b1[1] == g["bi_cost"], nm
+        assert sha(b1[4]) == reference_outputs["bi_prev_sha256"][nm], nm
+        if reflib_if_built:
+            ref = reflib_if_built
+            assert (oracle.dist_matrix(xy, wt) == ref.dist_matrix(xy, wt)).all()
+            b2 = ref.two_opt_bi(xy, wt, s1, want_prev=True)
+            assert (b1[0] == b2[0]).all() and b1[1] == b2[1] and (b1[4] == b2[2]).all()
 
 
-def test_oracle_equals_reference_on_random_tours_and_coords(oracle, reflib):
-    rng = np.random.default_rng(7)
-    for wt, n in [(0, 120), (3, 90), (5, 100), (4, 60)]:
-        if wt == 4:
-            xy = np.round(rng.uniform(-80, 80, size=(n, 2)), 2)
-        else:
-            xy = rng.integers(0, 3000, size=(n, 2)).astype(np.float64)
-            xy[::7] += 0.5  # non-integer but FP32-exact
-        succ = order_to_succ(rng.permutation(n).astype(np.int32))
+def test_oracle_equals_reference_on_random_tours_and_coords(oracle, reference_outputs, reflib_if_built):
+    from golden.make_reference_outputs import random_tour_cases
+    cases = list(random_tour_cases())
+    assert len(cases) == len(reference_outputs["random_tours"]) == 4
+    for (wt, xy, succ), r in zip(cases, reference_outputs["random_tours"]):
+        assert (wt, len(xy)) == (r["wt"], r["n"])
         c = oracle.succ_cost(xy, wt, succ)
         f1 = oracle.two_opt_fi(xy, wt, succ, c)
-        f2 = reflib.two_opt_fi(xy, wt, succ, c)
-        assert (f1[0] == f2[0]).all() and f1[1] == f2[1]
+        assert sha(f1[0]) == r["fi_sha256"] and f1[1] == r["fi_cost"], wt
         b1 = oracle.two_opt_bi(xy, wt, succ)
-        b2 = reflib.two_opt_bi(xy, wt, succ)
-        assert (b1[0] == b2[0]).all() and b1[1] == b2[1]
+        assert sha(b1[0]) == r["bi_sha256"] and b1[1] == r["bi_cost"], wt
+        if reflib_if_built:
+            f2 = reflib_if_built.two_opt_fi(xy, wt, succ, c)
+            b2 = reflib_if_built.two_opt_bi(xy, wt, succ)
+            assert (f1[0] == f2[0]).all() and f1[1] == f2[1] and (b1[0] == b2[0]).all() and b1[1] == b2[1]
 
 
-def test_tabu_mask_restatement(oracle, reflib):
+def test_tabu_mask_restatement(oracle, reference_outputs, reflib_if_built):
     """alg_2opt_tabu with a tabu list: same tour AND same mutated list (lazy expiry, tabusearch.c:83-92)."""
-    rng = np.random.default_rng(11)
-    n = 60
-    xy = rng.integers(0, 1000, size=(n, 2)).astype(np.float64)
-    succ = order_to_succ(rng.permutation(n).astype(np.int32))
-    ncols = n * (n - 1) // 2
-    mask = np.where(rng.random(ncols) < 0.2, rng.integers(1, 30, size=ncols), 0).astype(np.int32)
-    m1, m2 = mask.copy(), mask.copy()
-    b1 = oracle.two_opt_bi(xy, 0, succ, skip_edge=m1, iter_=30, tenure=12)
-    b2 = reflib.two_opt_bi(xy, 0, succ, skip_edge=m2, iter_=30, tenure=12)
-    assert (b1[0] == b2[0]).all() and b1[1] == b2[1]
-    assert (m1 == m2).all()
+    from golden.make_reference_outputs import tabu_mask_case
+    xy, succ, m1 = tabu_mask_case()
+    m2 = m1.copy()
+    r = reference_outputs["tabu_mask"]
+    b1 = oracle.two_opt_bi(xy, 0, succ, skip_edge=m1, iter_=r["iter"], tenure=r["tenure"])
+    assert sha(b1[0]) == r["bi_sha256"] and b1[1] == r["bi_cost"]
+    assert sha(m1) == r["mask_after_sha256"]
+    if reflib_if_built:
+        b2 = reflib_if_built.two_opt_bi(xy, 0, succ, skip_edge=m2, iter_=r["iter"], tenure=r["tenure"])
+        assert (b1[0] == b2[0]).all() and b1[1] == b2[1] and (m1 == m2).all()
 
 
 def test_synthetic_known_answers(oracle):
@@ -173,48 +177,55 @@ def test_large_fixture_spot_check(oracle):
     assert log.tolist() == g["fl3795"]["bi_log"][:3]
 
 
-def test_constructive_restatements_equal_reference_and_csv(oracle, reflib, instances, goldens):
-    """orc_greedy_iter / orc_extra_mileage (reference HEU_Greedy_iter, HEU_extramileage) vs the compiled reference (tour and
-    cost) and vs the published GREEDY_ITER / EXTR_MILE columns."""
+def test_constructive_restatements_equal_reference_and_csv(oracle, instances, goldens, reference_outputs, reflib_if_built):
+    """orc_greedy_iter / orc_extra_mileage (reference HEU_Greedy_iter, HEU_extramileage) vs the stored driver results (tour and
+    cost), the compiled reference when built, and the published GREEDY_ITER / EXTR_MILE columns."""
+    from golden.make_reference_outputs import tiny_extra_mileage_cases
     for nm in ("berlin52", "pr299", "att532", "ulysses22", "gr96", "eil51"):
         xy, wt = instances[nm]
         b, s, c = oracle.greedy_iter(xy, wt)
-        st, rs, rc = reflib.run_method("HEU_Greedy_iter", xy, wt)
-        assert st == 0 and c == rc and (s == rs).all(), nm
+        r = reference_outputs["greedy_iter"][nm]
+        assert c == r["cost"] and sha(s) == r["sha256"], nm
+        if reflib_if_built:
+            st, rs, rc = reflib_if_built.run_method("HEU_Greedy_iter", xy, wt)
+            assert st == 0 and c == rc and (s == rs).all(), nm
         s, c = oracle.extra_mileage(xy, wt)
-        st, rs, rc = reflib.run_method("HEU_extramileage", xy, wt)
-        assert st == 0 and c == rc and (s == rs).all(), nm
+        r = reference_outputs["extra_mileage"][nm]
+        assert c == r["cost"] and sha(s) == r["sha256"], nm
+        if reflib_if_built:
+            st, rs, rc = reflib_if_built.run_method("HEU_extramileage", xy, wt)
+            assert st == 0 and c == rc and (s == rs).all(), nm
         if nm in goldens["reference_csv"]:
             assert c == goldens["reference_csv"][nm]["EXTR_MILE"]
-    rng = np.random.default_rng(4)
-    for n in (2, 3, 5, 30):
-        xy = rng.integers(0, 7, size=(n, 2)).astype(np.float64)  # ties and coincident nodes
+    for n, xy in tiny_extra_mileage_cases():  # ties and coincident nodes
         s, c = oracle.extra_mileage(xy, 0)
-        st, rs, rc = reflib.run_method("HEU_extramileage", xy, 0)
-        assert c == rc and (s == rs).all(), n
+        r = reference_outputs["extra_mileage"][f"ties{n}"]
+        assert c == r["cost"] and sha(s) == r["sha256"], n
+        if reflib_if_built:
+            st, rs, rc = reflib_if_built.run_method("HEU_extramileage", xy, 0)
+            assert c == rc and (s == rs).all(), n
 
 
-def test_vns_kick_restatement_equals_the_reference_kick(oracle, reflib):
+def test_vns_kick_restatement_equals_the_reference_kick(oracle, reference_outputs, reflib_if_built):
     """oracle.vns_kick (indices handed in) against the reference's own kick() (src/vns.c:11), which draws its three indices
     from glibc random(): the draws are replayed with the restated generator.  Seeds whose largest index is n-1 are skipped —
     there the reference reads one element past its tour array."""
-    from tsp_optimization_b200.instances import GlibcRandom, is_tour, uniform_instance
-    n = 300
+    from golden.make_reference_outputs import vns_kick_indices
+    from tsp_optimization_b200.instances import is_tour, uniform_instance
+    n = reference_outputs["vns_kick"]["n"]
     xy = uniform_instance(n)
     succ, _ = oracle.nn_tour(xy, 0, 0)
     compared = 0
     for seed in range(1, 40):
-        g = GlibcRandom(seed)
-        i1 = g.rand_choice(0, n)
-        i2 = i3 = i1
-        while i2 == i1 or abs(i1 - i2) <= 1:
-            i2 = g.rand_choice(0, n)
-        while i3 == i1 or i3 == i2 or abs(i1 - i3) <= 1 or abs(i2 - i3) <= 1:
-            i3 = g.rand_choice(0, n)
-        if max(i1, i2, i3) == n - 1:
+        idx = vns_kick_indices(seed, n)
+        if max(idx) == n - 1:
+            assert str(seed) not in reference_outputs["vns_kick"]["seeds"]
             continue
-        s_ref, c_ref = reflib.vns_kick_stock(xy, 0, succ, seed)
-        s_o, c_o = oracle.vns_kick(xy, 0, succ, i1, i2, i3)
-        assert (s_ref == s_o).all() and c_ref == c_o and is_tour(s_o), seed
+        r = reference_outputs["vns_kick"]["seeds"][str(seed)]
+        s_o, c_o = oracle.vns_kick(xy, 0, succ, *idx)
+        assert sha(s_o) == r["sha256"] and c_o == r["cost"] and is_tour(s_o), seed
+        if reflib_if_built:
+            s_ref, c_ref = reflib_if_built.vns_kick_stock(xy, 0, succ, seed)
+            assert (s_ref == s_o).all() and c_ref == c_o, seed
         compared += 1
     assert compared >= 30
