@@ -175,6 +175,7 @@ struct tspb200_ctx {
     long long opt_time_limit_ms = 0;
     int opt_seed_hint = 1;
     int opt_pdl = 1;
+    int opt_prefilter = -1;           // exhaustive best-improvement scan: stage-1 prefilter on squared distances (-1 auto, 0 off, 1 on)
     int opt_single_block = -1;
     int opt_prune = -1;         // exact tile pruning of the best-improvement scan: -1 auto, 0 off (exhaustive scan), 1 on
     int opt_timing = 0;         // accumulate the per-pass breakdown (scan / tail / exchange wait / apply) on the device
@@ -418,6 +419,9 @@ int tspb200_set_option(tspb200_ctx *ctx, const char *key, int64_t value) {
         ctx->opt_batch_kernel = value ? 1 : 0;
     } else if (k == "pdl") {
         ctx->opt_pdl = value ? 1 : 0;
+    } else if (k == "prefilter") {
+        if (value < -1 || value > 1) return fail(ctx, TSPB200_E_ARG, "prefilter must be -1 (auto), 0 or 1");
+        ctx->opt_prefilter = (int)value;
     } else if (k == "seed_hint") {
         ctx->opt_seed_hint = value < 0 ? 0 : (value > 2 ? 2 : (int)value);
     } else if (k == "tile_cols") {
@@ -457,6 +461,8 @@ int64_t tspb200_get_info(const tspb200_ctx *ctx, const char *key) {
     if (k == "matrix_resident") return ctx->d_mat != nullptr;
     if (k == "matrix_ld") return ctx->mat_ld;
     if (k == "cold_calls") return ctx->h_ctl ? (int64_t)ctx->h_ctl->cold_calls : -1;  // as of the last host sync
+    if (k == "pf_hits") return ctx->h_ctl ? (int64_t)ctx->h_ctl->pf_hits : -1;
+    if (k == "prefilter") return ctx->opt_prefilter;
     if (k == "tiles_scanned") return ctx->h_ctl ? (int64_t)ctx->h_ctl->tiles_scanned : -1;
     // per-pass breakdown accumulated since the tour was uploaded (option "timing"), ns; tm_count = passes accumulated
     if (k.rfind("tm_", 0) == 0 && ctx->h_ctl) {
@@ -719,6 +725,7 @@ static void choose_tile_shape(int n, int num_sms, int world, int opt_T, int opt_
 
 // exact tile pruning pays once a pass is deep enough that skipping tiles outweighs the two extra (tiny) launches
 constexpr int PRUNE_AUTO_MIN_N = 3000;
+constexpr int BI_PREFILTER_MIN_N = 40000;  // exhaustive scans with at least this tour size's pairs per rank use the stage-1 prefilter (see tspb200_bi_run)
 static bool prune_wanted(const tspb200_ctx *ctx) {
     return ctx->opt_prune >= 0 ? ctx->opt_prune == 1 : ctx->n >= PRUNE_AUTO_MIN_N;
 }
@@ -1034,12 +1041,22 @@ int tspb200_bi_run(tspb200_ctx *ctx, int64_t max_passes, tspb200_stats *st) {
     a.fuse_apply = ctx->world == 1 ? (fuse_in_kernel ? 2 : 1) : 0;
     a.seed_hint = ctx->opt_seed_hint;
     a.packed_tail = (path == 0 && packable && ctx->opt_seed_hint < 2) ? 1 : 0;
+    // E: the square-root filter's own FP32 error (< 1.75 eps: two distances, three sums) plus the roundings of the
+    // prefilter's a = ds_p + h, b = ds_q + h and h (< 0.75 eps), DESIGN.md §3
+    a.pf_slack = 4.0f * ctx->eps32;
     a.timing = ctx->opt_timing;
     if (a.timing == 2 && !ctx->d_dbg) CK(cudaMalloc(&ctx->d_dbg, sizeof(unsigned long long) * (2 + 8) * 4096));  // {start, end} + 8 phase stamps per block
     a.dbg = ctx->d_dbg;
     // exact tile pruning: same moves, fewer evaluated pairs (the throughput benchmarks switch it off: "prune" = 0)
     const bool prune = path == 0 && !ctx->tabu_on && ctx->ntr > 0 && prune_wanted(ctx);
     a.pruned = prune ? 1 : 0;
+    // stage-1 prefilter (kernels_bi_scan.cuh): exhaustive scans with a large share of pairs per rank.  Measured on B200
+    // (profiles/r3_prefilter_by_n.jsonl): a pass at n = 100 000 is 15 % faster, one at n = 10 000 slower — a pass of one or a
+    // few waves is latency-bound, and its stage-1 hits (an L2 round trip each) sit on the critical path.  What counts is the
+    // work of this rank, n^2 / (2 world) pairs, so the rule compares that with a single-GPU pass at BI_PREFILTER_MIN_N.
+    // Pruned passes scan only the tiles that hold improving moves, where stage 1 hits too often to pay (DESIGN.md §4.1).
+    const bool pf_auto = (double)n * (double)n >= (double)BI_PREFILTER_MIN_N * BI_PREFILTER_MIN_N * a.world;
+    a.prefilter = (!prune || TSPB_BI_PREFILTER_PRUNED) && (ctx->opt_prefilter == 1 || (ctx->opt_prefilter == -1 && pf_auto)) ? 1 : 0;
     a.row_shuffle = ctx->row_shuffle;
     // multi-GPU: keys travel as NVLink peer stores from the scan kernel (path 0) unless NCCL was asked for
     const bool use_xchg = ctx->world > 1 && path == 0 && ctx->xchg.enabled && ctx->opt_exchange == 0;

@@ -16,9 +16,14 @@
 // (delta, i, j) argmin.  Column records are staged in shared memory by TMA bulk copies (UBLKCP),
 // double-buffered across tiles.
 //
-// Header: the kernel is a template over the block shape and the instance flags (104 instantiations); they are compiled in
+// Stage-1 prefilter (bi_scan_kernel, exhaustive scans of large tours): squared distances against per-row and per-column
+// bounds decide first, without a square root; only its hits meet the square-root filter above (see pf_bound below).
+// bi_scan_sqrt_kernel is the square-root filter alone (pruned passes, smaller shares per rank, option "prefilter" = 0).
+//
+// Header: the kernels are templates over the block shape and the instance flags (104 square-root instantiations, 52 prefilter
+// ones: exhaustive only); they are compiled in
 // four translation units (kernels_bi_s64.cu, kernels_bi_p64.cu, kernels_bi_128.cu, kernels_bi_256.cu) so that a clean build
-// takes about a minute with make -j4 instead of three in one file.  kernels_bi.cu holds the dispatch and the other kernels of a pass.
+// compiles them in parallel (make -j4).  kernels_bi.cu holds the dispatch and the other kernels of a pass.
 #pragma once
 #include "tsp_state.cuh"
 
@@ -40,7 +45,8 @@ __device__ __forceinline__ float dist32(float ax, float ay, float bx, float by) 
 // LAST: how D[R] — the distance from the row just below this thread's rows, i.e. the first row of the next lane — is
 // obtained: 1 = computed here (scalar, the (R+1)-th square root of the column), 2 = taken from the next lane with one
 // shuffle (SHUF kernels: the lanes of a warp own adjacent row groups, so that distance is lane+1's D[0]), 0 = not needed.
-template <int R, bool ATT, int LAST>
+// SQ: return the raw squared distances s = dx^2 + dy^2 (no square root, no ATT scale) for the stage-1 prefilter.
+template <int R, bool ATT, int LAST, bool SQ = false>
 __device__ __forceinline__ void column_dists(const f32x2 (&xr2)[R / 2], const f32x2 (&yr2)[R / 2], float xrl, float yrl,
                                              float cx, float cy, float (&D)[R + 1]) {
     const f32x2 cxx = f2pack(cx, cx), cyy = f2pack(cy, cy);
@@ -49,13 +55,54 @@ __device__ __forceinline__ void column_dists(const f32x2 (&xr2)[R / 2], const f3
         f32x2 dx = f2sub(xr2[k], cxx);
         f32x2 dy = f2sub(yr2[k], cyy);
         f32x2 s = f2fma(dy, dy, f2mul(dx, dx));
+        if (SQ) {
+            D[2 * k] = f2lo(s);
+            D[2 * k + 1] = f2hi(s);
+            continue;
+        }
         if (ATT) s = f2mul(s, f2pack(0.1f, 0.1f));
         D[2 * k] = sqrt_approx(f2lo(s));
         D[2 * k + 1] = sqrt_approx(f2hi(s));
     }
-    if (LAST == 1) D[R] = dist32<ATT>(xrl, yrl, cx, cy);
-    else if (LAST == 2) D[R] = __shfl_down_sync(0xffffffffu, D[0], 1);
-    else D[R] = 0.f;
+    if (LAST == 1) {
+        if (SQ) {
+            const float dx = xrl - cx, dy = yrl - cy;
+            D[R] = fmaf(dy, dy, dx * dx);
+        } else {
+            D[R] = dist32<ATT>(xrl, yrl, cx, cy);
+        }
+    } else if (LAST == 2) {
+        D[R] = __shfl_down_sync(0xffffffffu, D[0], 1);
+    } else {
+        D[R] = 0.f;
+    }
+}
+
+// ---- stage-1 prefilter (option "prefilter", DESIGN.md §3) ----------------------------------------------------
+// The FP32 filter above asks D1 + D2 <= ds_p + ds_q + thr (D1 = D(p,q), D2 = D(p+1,q+1)) and needs a square root per
+// distance.  With a = ds_p + h, b = ds_q + h, h = (thr + E) / 2, every pair that filter can pass has d1 + d2 <= a + b
+// (d = the real distance between the FP32 coordinates; E bounds the filter's own FP32 error and the roundings of a, b),
+// hence, since a + b >= d1 + d2 >= 0,
+//     s1 + s2 = d1^2 + d2^2 <= (d1 + d2)^2 <= (a + b)^2 <= 2 a|a| + 2 b|b|        (s = dx^2 + dy^2; ATT: d^2 = s / 10)
+// — the last step is 2a^2 + 2b^2 - (a+b)^2 = (a-b)^2 >= 0 for a, b >= 0 and, for b < 0 <= a + b, (a - 3b)(a + b) >= 0.
+// Stage 1 tests  (s1 + cp_p) + s2 <= C_q  with the row constant cp_p = -pf_bound(ds_p) and the column constant
+// C_q = pf_bound(ds_q): squared distances only, no MUFU.  pf_bound(x) >= 2g (x + h)|x + h| (g = 1, ATT: 10) with a relative
+// slack PF_REL that covers every FP32 rounding of the squared domain and an absolute one (PF_ABS) for flushed denormals.
+// Padding rows / columns (ds = -BIG) give cp = +inf / C = -inf: never a hit, never a NaN.
+// Stage 2 re-runs the square-root filter on the hitting lane's R x BI_CB block (bi_refilter_warp); only what survives it
+// reaches bi_cold_warp, so the exact path sees the same pairs as without the prefilter.
+//
+// PF_REL: the roundings of s (dx, dx^2, the FMA: < 4.1 ulp relative), of the two sums (< 2.1 ulp of |s1| + |s2| + |cp|) and
+// of each constant (< 3 ulp) add up to < 12 ulp = 2^-20.4 of 2g (a^2 + b^2); inflating both bounds by 2^-16 of themselves
+// gains 2g (a^2 + b^2) 2^-16, ~20x that.  PF_ABS: flush-to-zero can move a product or a sum by < 2^-126 each.
+constexpr float PF_REL = 0x1p-16f;
+constexpr float PF_ABS = 0x1p-100f;
+
+// upper bound of 2g (ds + h)|ds + h|, g = 10 for ATT (its distances are sqrt(s / 10)), else 1
+template <bool ATT>
+__device__ __forceinline__ float pf_bound(float ds, float h) {
+    const float a = ds + h;
+    return fmaf(a * (ATT ? 20.f : 2.f), fmaf(PF_REL, a, fabsf(a)), PF_ABS);
 }
 
 // ---- cold path ------------------------------------------------------------------------------------------
@@ -67,7 +114,8 @@ __device__ __forceinline__ void column_dists(const f32x2 (&xr2)[R / 2], const f3
 // shuffles.  A hit costs a few hundred cycles instead of a serial walk over 32 pairs by a single lane.
 constexpr int BI_CB = 4;  // columns per filter check
 
-template <int R, bool ATT, bool EXACT32>
+// PF: called from the prefilter kernel, whose column records hold C_q instead of ds_q (read from rec instead)
+template <int R, bool ATT, bool EXACT32, bool PF>
 __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
                                              int jj0, float thr) {
     const int lane = threadIdx.x & 31;
@@ -80,8 +128,9 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
         if (idx < R * BI_CB && q >= p + 2 && q <= n - 1 && !(p == 0 && q == n - 1)) {  // reference tabusearch.c:134
             const float4 rp = __ldg(&rec[p]), rp1 = __ldg(&rec[p + 1]);  // row records: one L2 round trip for the warp
             const float4 c0 = sc[jj0 + c], c1 = sc[jj0 + c + 1];
+            const float dsq = PF ? __ldg(&rec[q].z) : c0.z;
             const float qv = (dist32<ATT>(rp.x, rp.y, c0.x, c0.y) - rp.z) + dist32<ATT>(rp1.x, rp1.y, c1.x, c1.y);
-            if (qv <= thr + c0.z) {
+            if (qv <= thr + dsq) {
                 const int u = node_of(rp), v = node_of(c0);
                 long long d1, d2;
                 if (EXACT32) {
@@ -91,7 +140,7 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
                     d1 = exact_dist(I.metric, I.pt64[u], I.pt64[v]);
                     d2 = exact_dist(I.metric, I.pt64[node_of(rp1)], I.pt64[node_of(c1)]);
                 }
-                const long long delta = d1 + d2 - (long long)rp.z - (long long)c0.z;
+                const long long delta = d1 + d2 - (long long)rp.z - (long long)dsq;
                 if (delta < 0) {
                     MoveKey k;
                     k.delta = (int)delta; k.i = min(u, v); k.j = max(u, v); k.pad = 0;
@@ -102,6 +151,27 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
     }
     __syncwarp();
     return key_warp_min(best);
+}
+
+// Stage 2 of the prefilter: does any pair of the R x BI_CB block pass bi_cold_warp's square-root filter?  Same pairs,
+// same expression, one pair per lane; inline, so the kernel's own code keeps the MUFU.SQRT of the filter.  Warp-uniform.
+template <int R, bool ATT>
+__device__ __forceinline__ bool bi_refilter_warp(const float4 *rec, const float4 *sc, int n, int p0, int Q0, int jj0, float thr) {
+    const int lane = threadIdx.x & 31;
+    bool pass = false;
+#pragma unroll
+    for (int base = 0; base < R * BI_CB; base += 32) {
+        const int idx = base + lane;
+        const int r = idx / BI_CB, c = idx % BI_CB;
+        const int p = p0 + r, q = Q0 + jj0 + c;
+        if (idx < R * BI_CB && q >= p + 2 && q <= n - 1 && !(p == 0 && q == n - 1)) {
+            const float4 rp = __ldg(&rec[p]), rp1 = __ldg(&rec[p + 1]);
+            const float4 c0 = sc[jj0 + c], c1 = sc[jj0 + c + 1];
+            const float qv = (dist32<ATT>(rp.x, rp.y, c0.x, c0.y) - rp.z) + dist32<ATT>(rp1.x, rp1.y, c1.x, c1.y);
+            pass |= qv <= thr + __ldg(&rec[q].z);
+        }
+    }
+    return __any_sync(0xffffffffu, pass);
 }
 
 // BI_THREADS x R rows per tile: 256 x 8 for big instances; smaller blocks (64 / 128 threads, up to 8 per SM) give
@@ -124,8 +194,10 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
 // would spill under the lower cap) keep 8.
 #define TSPB_BI_MINBLOCKS64 10
 #endif
-template <int BI_THREADS, int R, bool ATT, bool EXACT32, bool PRUNED, bool SHUF>
-__global__ void __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 : 384 / BI_THREADS) : (BI_THREADS == 64 && !PRUNED ? TSPB_BI_MINBLOCKS64 : 512 / BI_THREADS))) bi_scan_kernel(const BiArgs A) {
+// PF: stage-1 prefilter (bi_scan_kernel: exhaustive scans with a large share of pairs per rank, engine.cu) or the square-root
+// filter alone (bi_scan_sqrt_kernel: pruned passes, smaller shares, option "prefilter" = 0).
+template <int BI_THREADS, int R, bool ATT, bool EXACT32, bool PRUNED, bool SHUF, bool PF>
+__device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[2];
     __shared__ int s_hint;
@@ -150,6 +222,7 @@ __global__ void __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 
     // tile tables -> shared memory (one coalesced L2 round trip instead of a dependent chain per binary-search step)
     int *s_rs = reinterpret_cast<int *>(scols1 + (TJ + 2));  // [ntr+1] prefix sums of tiles per tile-row
     int *s_rj = s_rs + (A.ntr + 1);                          // [ntr]   first tile column of each tile-row
+    __shared__ float s_pfthr;                                // PF: the block's threshold of the tile's bounds
     for (int k = tid; k <= A.ntr; k += BI_THREADS) {
         s_rs[k] = A.tile_row_start[k];
         if (k < A.ntr) s_rj[k] = A.tile_row_j0[k];
@@ -281,8 +354,12 @@ __global__ void __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 
         const int buf = it & 1;
         const unsigned parity = (unsigned)(it >> 1) & 1u;
         const float4 *sc = buf ? scols1 : scols0;
-        // prefetch the next tile into the other stage (its slot in s_tile / scols was last read two tiles ago)
-        if (tid == 0) draw(buf ^ 1, false);
+        // prefetch the next tile into the other stage (its slot in s_tile / scols was last read two tiles ago; PF: and
+        // written, so the bulk copy is ordered after those generic-proxy stores)
+        if (tid == 0) {
+            if (PF) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            draw(buf ^ 1, false);
+        }
 
         // rows of this thread: p0 .. p0+R-1 in packed pairs (+ successor row p0+R, scalar)
         const int p0 = SHUF ? P0 + (tid >> 5) * (32 * R - 1) + (tid & 31) * R : P0 + tid * R;
@@ -312,64 +389,93 @@ __global__ void __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 
         mbar_wait(&bars[buf], parity);
         if (PRUNED && A.timing == 2 && tid == 0 && it == 0) A.dbg[8192 + 8 * blockIdx.x + 2] = globaltimer_ns();  // rows and columns of the first tile are here
 
+        if (PF) {
+            // prefilter bounds of this tile, from ONE threshold for the whole block (thread 0's snapshot; every thread's thr
+            // is lowered to it, so h bounds every lane's (thr + E) / 2 until the end of the tile, when thr may have fallen:
+            // an older, larger h only admits more pairs).  Column constants go to shared memory once per tile instead of
+            // four FP32 instructions per column and thread: the column record's ds slot (z) takes C_q, so the hot loop is the
+            // same code as the square-root kernel's (the exact path reads ds_q from rec).
+            if (tid == 0) s_pfthr = (float)(*((volatile int *)&s_hint)) + W;
+            __syncthreads();
+            thr = fminf(thr, s_pfthr);
+            const float h = 0.5f * (s_pfthr + A.pf_slack);
+            float4 *scw = buf ? scols1 : scols0;
+            for (int j = tid; j < NCv; j += BI_THREADS) scw[j].z = pf_bound<ATT>(scw[j].z, h);
+#pragma unroll
+            for (int k = 0; k < R / 2; ++k)  // cp2 holds -ds here (padding / masked rows: -BIG -> +inf)
+                cp2[k] = f2pack(-pf_bound<ATT>(-f2lo(cp2[k]), h), -pf_bound<ATT>(-f2hi(cp2[k]), h));
+            __syncthreads();
+        }
+
         // pairs with q < p+2 exist in this tile?  (mask them; they are mirrored / adjacent pairs)
         const bool diag = (Q0 < P0 + TI + 1);
         const int NC = PRUNED ? NCv : TJ;  // columns of this tile
         // first column of the scan: D0 -> U2 (kept per variant so that the regular tile's shared-memory addressing stays uniform)
         float4 c0, cnext;
         f32x2 U2[R / 2];
-#define BI_INIT(JB)                                                                                    \
+        // PF: the prefilter variant — D holds squared distances, U2 = s + cp (row constant), the column term is pf_bound(ds_q)
+        // and a block is a hit when its minimum is <= 0 (see pf_bound above)
+#define BI_INIT(JB, PF)                                                                                \
     {                                                                                                  \
         c0 = sc[(JB)];                                                                                 \
         cnext = sc[(JB) + 1];                                                                          \
         float D0[R + 1];                                                                               \
-        column_dists<R, ATT, SHUF ? 0 : 1>(xr2, yr2, xrl, yrl, c0.x, c0.y, D0);                        \
+        column_dists<R, ATT, SHUF ? 0 : 1, PF>(xr2, yr2, xrl, yrl, c0.x, c0.y, D0);                    \
         _Pragma("unroll") for (int k = 0; k < R / 2; ++k) U2[k] = f2add(f2pack(D0[2 * k], D0[2 * k + 1]), cp2[k]); \
     }
 #define UU(r_) (((r_) & 1) ? f2hi(U2[(r_) >> 1]) : f2lo(U2[(r_) >> 1]))
 
 // one column: R+1 fresh distances -> R move deltas Q[r] = (D[p_r][q] - ds_p) + D[p_r+1][q+1]; the filter quantity
 // min_r Q[r] - ds_q is folded into the running block minimum M (no branch, no per-pair state kept)
-#define BI_COL(DIAG, jj_)                                                                              \
+#define BI_COL(DIAG, jj_, PF)                                                                          \
     {                                                                                                  \
         const float4 c1 = cnext;                                                                       \
         cnext = sc[(jj_) + 2]; /* prefetched one column ahead */                                       \
         float Dn[R + 1];                                                                               \
-        column_dists<R, ATT, SHUF ? 2 : 1>(xr2, yr2, xrl, yrl, c1.x, c1.y, Dn);                        \
+        column_dists<R, ATT, SHUF ? 2 : 1, PF>(xr2, yr2, xrl, yrl, c1.x, c1.y, Dn);                    \
         float m = TSPB_BIG;                                                                            \
         _Pragma("unroll") for (int r = 0; r < R; ++r) {                                                \
             float qv = UU(r) + Dn[r + 1];                                                              \
             if (DIAG) qv = (qrel0 + (jj_) >= r + 2) ? qv : TSPB_BIG;                                   \
             m = fminf(m, qv);                                                                          \
         }                                                                                              \
-        M = fminf(M, m - c0.z);                                                                        \
+        M = fminf(M, m - c0.z); /* PF: c0.z = C_q */                                                   \
         _Pragma("unroll") for (int k = 0; k < R / 2; ++k)                                              \
             U2[k] = f2add(f2pack(Dn[2 * k], Dn[2 * k + 1]), cp2[k]);                                   \
         c0 = c1;                                                                                       \
     }
 
 // BI_CB columns, then ONE filter check per warp (ballot); hits are resolved one lane at a time by the whole warp
-#define BI_BLOCK(DIAG)                                                                                 \
+// (PF: a stage-1 hit first goes through stage 2, the square-root filter, and only its survivors to the exact path)
+#define BI_BLOCK(DIAG, PF)                                                                             \
     for (int jj = 0; jj < NC; jj += BI_CB) {                                                           \
         float M = TSPB_BIG;                                                                            \
-        _Pragma("unroll") for (int c = 0; c < BI_CB; ++c) BI_COL(DIAG, jj + c)                         \
-        unsigned hits = __ballot_sync(0xffffffffu, M <= thr);                                          \
+        _Pragma("unroll") for (int c = 0; c < BI_CB; ++c) BI_COL(DIAG, jj + c, PF)                     \
+        unsigned hits = __ballot_sync(0xffffffffu, M <= (PF ? 0.f : thr));                             \
         while (hits) {                                                                                 \
             const int L = __ffs(hits) - 1;                                                             \
             const float thrL = __shfl_sync(0xffffffffu, thr, L);                                       \
-            const MoveKey nb = bi_cold_warp<R, ATT, EXACT32>(A.inst, rec, sc, n, p0 + (L - (tid & 31)) * R, Q0, jj, thrL); \
-            if ((tid & 31) == L) {                                                                     \
-                atomicAdd(&ctl->cold_calls, 1ull);                                                     \
-                if (key_less(nb, best)) {                                                              \
-                    best = nb;                                                                         \
-                    atomicMin(&s_hint, nb.delta);                                                      \
-                    atomicMin(&ctl->hint, nb.delta);                                                   \
-                }                                                                                      \
+            const int pL = p0 + (L - (tid & 31)) * R;                                                  \
+            bool cold = true;                                                                          \
+            if (PF) {                                                                                  \
+                if ((tid & 31) == L) atomicAdd(&ctl->pf_hits, 1ull);                                   \
+                cold = bi_refilter_warp<R, ATT>(rec, sc, n, pL, Q0, jj, thrL);                         \
             }                                                                                          \
-            /* an exact delta of a real move bounds the minimum for every lane: tighten all, drop stale hits */ \
-            if (nb.delta < 0) thr = fminf(thr, (float)nb.delta + W);                                   \
+            if (cold) {                                                                                \
+                const MoveKey nb = bi_cold_warp<R, ATT, EXACT32, PF>(A.inst, rec, sc, n, pL, Q0, jj, thrL); \
+                if ((tid & 31) == L) {                                                                 \
+                    atomicAdd(&ctl->cold_calls, 1ull);                                                 \
+                    if (key_less(nb, best)) {                                                          \
+                        best = nb;                                                                     \
+                        atomicMin(&s_hint, nb.delta);                                                  \
+                        atomicMin(&ctl->hint, nb.delta);                                               \
+                    }                                                                                  \
+                }                                                                                      \
+                /* an exact delta of a real move bounds the minimum for every lane: tighten all, drop stale hits */ \
+                if (nb.delta < 0) thr = fminf(thr, (float)nb.delta + W);                               \
+            }                                                                                          \
             hits &= hits - 1;                                                                          \
-            hits &= __ballot_sync(0xffffffffu, M <= thr);                                              \
+            if (!PF) hits &= __ballot_sync(0xffffffffu, M <= thr);                                     \
         }                                                                                              \
         /* every 64 columns: pick up what the other warps / blocks found (tid 0 swaps in the ctl->hint value it */ \
         /* requested 64 columns ago, so nobody waits for L2)                                                    */ \
@@ -384,11 +490,11 @@ __global__ void __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 
 
         const int qrel0 = Q0 - p0;  // q - p0 at jj = 0
         if (!diag) {
-            BI_INIT(0)
-            BI_BLOCK(false)
+            BI_INIT(0, PF)
+            BI_BLOCK(false, PF)
         } else {
-            BI_INIT(0)
-            BI_BLOCK(true)
+            BI_INIT(0, PF)
+            BI_BLOCK(true, PF)
         }
 #undef BI_INIT
 #undef BI_BLOCK
@@ -568,6 +674,18 @@ __global__ void __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 
 }
 
 
+#define TSPB_BI_BOUNDS \
+    __launch_bounds__(BI_THREADS, (R >= 16 ? (BI_THREADS == 256 ? 1 : 384 / BI_THREADS) : (BI_THREADS == 64 && !PRUNED ? TSPB_BI_MINBLOCKS64 : 512 / BI_THREADS)))
+template <int BI_THREADS, int R, bool ATT, bool EXACT32, bool PRUNED, bool SHUF>
+__global__ void TSPB_BI_BOUNDS bi_scan_kernel(const BiArgs A) {
+    bi_scan_body<BI_THREADS, R, ATT, EXACT32, PRUNED, SHUF, true>(A);
+}
+template <int BI_THREADS, int R, bool ATT, bool EXACT32, bool PRUNED, bool SHUF>
+__global__ void TSPB_BI_BOUNDS bi_scan_sqrt_kernel(const BiArgs A) {
+    bi_scan_body<BI_THREADS, R, ATT, EXACT32, PRUNED, SHUF, false>(A);
+}
+#undef TSPB_BI_BOUNDS
+
 // ---- host-side launchers -----------------------------------------------------------------------------
 template <int T, int R, bool SHUF>
 static inline cudaError_t launch_bi_tr(const BiArgs &a, int grid, bool pdl, cudaStream_t st) {
@@ -595,16 +713,30 @@ static inline cudaError_t launch_bi_tr(const BiArgs &a, int grid, bool pdl, cuda
         cfg.numAttrs = 1;
         return cudaLaunchKernelEx(&cfg, kern, a);
     };
-    if (a.pruned) {
+#if TSPB_BI_PREFILTER_PRUNED
+    if (a.prefilter && a.pruned) {
         if (att && ex) return go(bi_scan_kernel<T, R, true, true, true, SHUF>);
         if (att) return go(bi_scan_kernel<T, R, true, false, true, SHUF>);
         if (ex) return go(bi_scan_kernel<T, R, false, true, true, SHUF>);
         return go(bi_scan_kernel<T, R, false, false, true, SHUF>);
     }
-    if (att && ex) return go(bi_scan_kernel<T, R, true, true, false, SHUF>);
-    if (att) return go(bi_scan_kernel<T, R, true, false, false, SHUF>);
-    if (ex) return go(bi_scan_kernel<T, R, false, true, false, SHUF>);
-    return go(bi_scan_kernel<T, R, false, false, false, SHUF>);
+#endif
+    if (a.prefilter && !a.pruned) {  // the prefilter serves exhaustive scans only (engine.cu, tspb200_bi_run)
+        if (att && ex) return go(bi_scan_kernel<T, R, true, true, false, SHUF>);
+        if (att) return go(bi_scan_kernel<T, R, true, false, false, SHUF>);
+        if (ex) return go(bi_scan_kernel<T, R, false, true, false, SHUF>);
+        return go(bi_scan_kernel<T, R, false, false, false, SHUF>);
+    }
+    if (a.pruned) {
+        if (att && ex) return go(bi_scan_sqrt_kernel<T, R, true, true, true, SHUF>);
+        if (att) return go(bi_scan_sqrt_kernel<T, R, true, false, true, SHUF>);
+        if (ex) return go(bi_scan_sqrt_kernel<T, R, false, true, true, SHUF>);
+        return go(bi_scan_sqrt_kernel<T, R, false, false, true, SHUF>);
+    }
+    if (att && ex) return go(bi_scan_sqrt_kernel<T, R, true, true, false, SHUF>);
+    if (att) return go(bi_scan_sqrt_kernel<T, R, true, false, false, SHUF>);
+    if (ex) return go(bi_scan_sqrt_kernel<T, R, false, true, false, SHUF>);
+    return go(bi_scan_sqrt_kernel<T, R, false, false, false, SHUF>);
 }
 
 

@@ -60,6 +60,7 @@ struct Ctl {
     MoveKey cand[4];                // runner-up moves of the last BI pass: re-evaluated after the apply to seed `hint`
     int ncand;
     unsigned long long cold_calls;  // statistics: filter hits that went through the exact (cold) path
+    unsigned long long pf_hits;     // statistics: stage-1 prefilter hits (warp ballot blocks), each re-checked by the FP32 filter
     unsigned long long pass_min;    // BI: packed (delta,i,j) minimum of the running pass (one atomicMin per block)
     int done_reason;                // why `done` is set: DONE_OPTIMUM or DONE_CAP (a capped run may be continued)
     // first improvement on several GPUs: 1 = the next search deals its segments over the ranks and exchanges the winner,
@@ -111,6 +112,12 @@ struct TourDev {
 };
 
 #define FI_NONE 0xffffffffffffffffull
+
+#ifndef TSPB_BI_PREFILTER_PRUNED
+// 1: pruned passes run the stage-1 prefilter kernel too.  Measurement builds only (make EXTRA=-DTSPB_BI_PREFILTER_PRUNED=1
+// OUT=...): it is slower there (profiles/r3_prefilter_pruned.jsonl), so the product build keeps it 0.
+#define TSPB_BI_PREFILTER_PRUNED 0
+#endif
 
 __device__ __forceinline__ int node_of(const float4 &r) { return __float_as_int(r.w); }
 
@@ -455,6 +462,8 @@ struct BiArgs {
     int packed_tail; // 1: blocks fold their key into ctl->pass_min with one 64-bit atomicMin (n <= 2^17, seed_hint < 2)
     int pruned;      // 1: tiles come from the live list built by tile_filter_kernel (exact tile pruning)
     int row_shuffle; // 1: SHUF kernels (a warp owns 32 R - 1 rows, the distance below a lane's rows comes from the next lane)
+    int prefilter;   // 1: stage-1 prefilter on squared distances in front of the FP32 filter (kernels_bi_scan.cuh)
+    float pf_slack;  // prefilter: linear slack E of its row and column bounds (4 eps, DESIGN.md §3)
     int timing;      // 1: accumulate the per-pass breakdown in ctl->tm_acc; 2: also dump per-block {start, end} stamps
     unsigned long long *dbg;        // timing == 2: [gridDim.x][2] globaltimer stamps of the last pass
     XchgDev xchg;    // fuse_apply == 0: how this rank's key reaches the other ranks (enabled = 0 -> NCCL allreduce of ctl->packed)
