@@ -8,16 +8,17 @@ binds it now.
 
 FP32_LANE_OPS_PER_COL: FP32-pipe lane operations per thread and column step in the column loop of
 bi_scan_kernel<64, 8, false, true, false, true>, counted from `cuobjdump -sass` between the loop head and the warp ballot,
-which covers 4 column steps (the once-per-tile first column before the loop excluded): per step FADD2 12 x 2, FADD 9,
-FMUL2 4 x 2, FFMA2 4 x 2 = 49 — dx and dy of 4 packed row pairs, s, U2 = s + cp, the 8 pair sums and the fold.  FMNMX3 /
-FMNMX, LDS and SHFL run on other pipes.  A thread evaluates 8 moves per column step, and a warp 32 x 8 - 1 of the rows it
-scans.  The fraction assumes the packed FP32x2 instructions occupy the pipe for two lane-ops each (not measured: no ncu).
+which covers 4 column steps: per step FFMA2 16 x 2 and FADD 1 = 33 — the four-FMA chain A_p + w_p . v_q of 4 packed row pairs
+and the column constant B_q added to the row minimum.  FMNMX3 / FMNMX, LDS and the loop-carried register moves run on other
+pipes.  A thread evaluates 8 moves per column step, and a warp 32 x 8 - 1 of the rows it scans.  The fraction assumes the
+packed FP32x2 instructions occupy the pipe for two lane-ops each (not measured: no ncu).
 
 With --sizes n1,n2,... it times instead exhaustive passes from an NN tour of uniform_instance(n) with the prefilter forced
 off and on (alternating, `passes` each, L2 flushed before every pass): the data behind BI_PREFILTER_MIN_N in csrc/engine.cu.
---world W times one rank's share of W ranks on one GPU (option "debug_shard", rank 0's tiles).
+--world W times one rank's share of W ranks on one GPU (option "debug_shard", rank 0's tiles).  --fractional adds a
+fraction to every coordinate, so that they are not FP32-exact and the kernels for such coordinates (EXACT32 = 0) run.
 
-usage: python tools/prefilter_hits.py [passes] [--sizes n1,n2,... [--world W]]
+usage: python tools/prefilter_hits.py [passes] [--sizes n1,n2,... [--world W] [--fractional]]
 """
 import json
 import os
@@ -29,17 +30,21 @@ import numpy as np
 from tsp_optimization_b200 import Engine
 from tsp_optimization_b200.instances import uniform_instance
 
-FP32_LANE_OPS_PER_COL = 49
+FP32_LANE_OPS_PER_COL = 33
 EVALS_PER_COL = 8 * 255 / 256
 LANES_PER_SM = 128  # FP32 lanes per SM and clock
 
 
-def by_size(passes, sizes, world):
+def by_size(passes, sizes, world, fractional):
     eng = Engine(0)
     eng.set_option("prune", 0)
     eng.set_option("l2_flush_bytes", 256 << 20)
     for n in sizes:
-        eng.set_instance(uniform_instance(n), 0)
+        xy = uniform_instance(n)
+        if fractional:  # decimal coordinates FP32 cannot hold: the kernels for non-FP32-exact coordinates run
+            xy = xy + np.random.default_rng(n).random(xy.shape) * 0.999 + 0.1
+        eng.set_instance(xy, 0)
+        assert eng.info("exact32") == (0 if fractional else 1)
         succ, _ = eng.nn_tour(0)
         eng.set_option("debug_shard", (world << 8) if world > 1 else 0)
         us = {0: [], 1: []}
@@ -49,7 +54,7 @@ def by_size(passes, sizes, world):
                 eng.tour_upload(succ)
                 st = eng.bi_run(passes)
                 us[pf].append(st.gpu_ms * 1e3 / st.passes)
-        print(json.dumps({"n": n, "world": world, "passes": passes, "us_per_pass_off": us[0], "us_per_pass_on": us[1],
+        print(json.dumps({"n": n, "world": world, "fractional": fractional, "passes": passes, "us_per_pass_off": us[0], "us_per_pass_on": us[1],
                           "speedup_median": float(np.median(us[0]) / np.median(us[1]))}), flush=True)
     eng.close()
 
@@ -58,7 +63,8 @@ def main():
     passes = int(sys.argv[1]) if len(sys.argv) > 1 and not sys.argv[1].startswith("--") else 20
     if "--sizes" in sys.argv:
         world = int(sys.argv[sys.argv.index("--world") + 1]) if "--world" in sys.argv else 1
-        return by_size(passes, [int(v) for v in sys.argv[sys.argv.index("--sizes") + 1].split(",")], world)
+        return by_size(passes, [int(v) for v in sys.argv[sys.argv.index("--sizes") + 1].split(",")], world,
+                       "--fractional" in sys.argv)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     succ = np.load(os.path.join(root, "tests", "golden", "nn_uni100000.npz"))["succ"]
     n = len(succ)

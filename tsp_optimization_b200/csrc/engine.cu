@@ -139,6 +139,7 @@ struct tspb200_ctx {
     int opt_nn_grid = -1;             // nearest neighbour on the bucket grid: -1 auto (planar metrics, n >= 256), 0 off, 1 on
     std::vector<double> h_xy;         // host copy of the coordinates of the resident instance (set_instance short cut)
     float eps32 = 0;                  // bound of |FP32 distance - real distance| for this instance
+    float pf_cx = 0, pf_cy = 0;       // translation of the FP32 coordinates for the stage-1 prefilter (BiArgs::pf_cx)
     unsigned long long geo_near = 0;  // GEO matrix entries within 1e-6 of a rounding boundary (last matrix build)
 
     // tour (device buffers are kept across set_instance / tour_upload calls while they are big enough: cudaMalloc is
@@ -547,6 +548,22 @@ int tspb200_set_instance(tspb200_ctx *ctx, const double *xy, int n, int weight_t
     // (round 1 used 2 + 2 eps for every metric: ~2x the exact-path calls on EUC_2D).
     const bool rounds_up = weight_type == TSPB200_CEIL_2D || weight_type == TSPB200_ATT;
     ctx->eps32 = (float)eps;
+    // The stage-1 prefilter's rounding margins scale with the squared norms of the coordinates it reads (DESIGN.md §3), so
+    // it reads them translated to the bounding box's center, rounded to an integer.  The translation must not round any
+    // FP32 coordinate (FP32 differences, hence every filter decision, stay what they are): otherwise none is used.
+    ctx->pf_cx = ctx->pf_cy = 0;
+    if (finite) {
+        const double cx = std::nearbyint(0.5 * (xmin + xmax)), cy = std::nearbyint(0.5 * (ymin + ymax));
+        bool exact = std::fabs(cx) < 16777216.0 && std::fabs(cy) < 16777216.0;  // the center itself is an FP32 value
+        for (int k = 0; k < n && exact; ++k) {
+            const double x = (double)(float)xy[2 * k] - cx, y = (double)(float)xy[2 * k + 1] - cy;
+            exact = (double)(float)x == x && (double)(float)y == y;
+        }
+        if (exact) {
+            ctx->pf_cx = (float)cx;
+            ctx->pf_cy = (float)cy;
+        }
+    }
     ctx->inst.W = metric_fp32 ? (float)((rounds_up ? 0.125 : 1.0) + 4.0 * eps) : (float)(2.0 + 2.0 * eps);
     ctx->inst.band = (float)std::ldexp(1.0, -20);
     if (n > ctx->inst_cap) {
@@ -725,7 +742,7 @@ static void choose_tile_shape(int n, int num_sms, int world, int opt_T, int opt_
 
 // exact tile pruning pays once a pass is deep enough that skipping tiles outweighs the two extra (tiny) launches
 constexpr int PRUNE_AUTO_MIN_N = 3000;
-constexpr int BI_PREFILTER_MIN_N = 40000;  // exhaustive scans with at least this tour size's pairs per rank use the stage-1 prefilter (see tspb200_bi_run)
+constexpr int BI_PREFILTER_MIN_N = 30000;  // exhaustive scans with at least this tour size's pairs per rank use the stage-1 prefilter (see tspb200_bi_run)
 static bool prune_wanted(const tspb200_ctx *ctx) {
     return ctx->opt_prune >= 0 ? ctx->opt_prune == 1 : ctx->n >= PRUNE_AUTO_MIN_N;
 }
@@ -1044,6 +1061,8 @@ int tspb200_bi_run(tspb200_ctx *ctx, int64_t max_passes, tspb200_stats *st) {
     // E: the square-root filter's own FP32 error (< 1.75 eps: two distances, three sums) plus the roundings of the
     // prefilter's a = ds_p + h, b = ds_q + h and h (< 0.75 eps), DESIGN.md §3
     a.pf_slack = 4.0f * ctx->eps32;
+    a.pf_cx = ctx->pf_cx;
+    a.pf_cy = ctx->pf_cy;
     a.timing = ctx->opt_timing;
     if (a.timing == 2 && !ctx->d_dbg) CK(cudaMalloc(&ctx->d_dbg, sizeof(unsigned long long) * (2 + 8) * 4096));  // {start, end} + 8 phase stamps per block
     a.dbg = ctx->d_dbg;
@@ -1051,7 +1070,7 @@ int tspb200_bi_run(tspb200_ctx *ctx, int64_t max_passes, tspb200_stats *st) {
     const bool prune = path == 0 && !ctx->tabu_on && ctx->ntr > 0 && prune_wanted(ctx);
     a.pruned = prune ? 1 : 0;
     // stage-1 prefilter (kernels_bi_scan.cuh): exhaustive scans with a large share of pairs per rank.  Measured on B200
-    // (profiles/r3_prefilter_by_n.jsonl): a pass at n = 100 000 is 15 % faster, one at n = 10 000 slower — a pass of one or a
+    // (profiles/r4_prefilter_by_n_w1.jsonl): a pass at n = 100 000 is 25 % faster, one at n = 10 000 slower — a pass of one or a
     // few waves is latency-bound, and its stage-1 hits (an L2 round trip each) sit on the critical path.  What counts is the
     // work of this rank, n^2 / (2 world) pairs, so the rule compares that with a single-GPU pass at BI_PREFILTER_MIN_N.
     // Pruned passes scan only the tiles that hold improving moves, where stage 1 hits too often to pay (DESIGN.md §4.1).

@@ -16,8 +16,9 @@
 // (delta, i, j) argmin.  Column records are staged in shared memory by TMA bulk copies (UBLKCP),
 // double-buffered across tiles.
 //
-// Stage-1 prefilter (bi_scan_kernel, exhaustive scans of large tours): squared distances against per-row and per-column
-// bounds decide first, without a square root; only its hits meet the square-root filter above (see pf_bound below).
+// Stage-1 prefilter (bi_scan_kernel, exhaustive scans of large tours): a bound on the sum of squared distances, evaluated as
+// a 4-term dot product (four packed FMAs per two moves, no square root), decides first; only its hits meet the square-root
+// filter above (see pf_bound and pf_dot_const below).
 // bi_scan_sqrt_kernel is the square-root filter alone (pruned passes, smaller shares per rank, option "prefilter" = 0).
 //
 // Header: the kernels are templates over the block shape and the instance flags (104 square-root instantiations, 52 prefilter
@@ -45,8 +46,7 @@ __device__ __forceinline__ float dist32(float ax, float ay, float bx, float by) 
 // LAST: how D[R] — the distance from the row just below this thread's rows, i.e. the first row of the next lane — is
 // obtained: 1 = computed here (scalar, the (R+1)-th square root of the column), 2 = taken from the next lane with one
 // shuffle (SHUF kernels: the lanes of a warp own adjacent row groups, so that distance is lane+1's D[0]), 0 = not needed.
-// SQ: return the raw squared distances s = dx^2 + dy^2 (no square root, no ATT scale) for the stage-1 prefilter.
-template <int R, bool ATT, int LAST, bool SQ = false>
+template <int R, bool ATT, int LAST>
 __device__ __forceinline__ void column_dists(const f32x2 (&xr2)[R / 2], const f32x2 (&yr2)[R / 2], float xrl, float yrl,
                                              float cx, float cy, float (&D)[R + 1]) {
     const f32x2 cxx = f2pack(cx, cx), cyy = f2pack(cy, cy);
@@ -55,22 +55,12 @@ __device__ __forceinline__ void column_dists(const f32x2 (&xr2)[R / 2], const f3
         f32x2 dx = f2sub(xr2[k], cxx);
         f32x2 dy = f2sub(yr2[k], cyy);
         f32x2 s = f2fma(dy, dy, f2mul(dx, dx));
-        if (SQ) {
-            D[2 * k] = f2lo(s);
-            D[2 * k + 1] = f2hi(s);
-            continue;
-        }
         if (ATT) s = f2mul(s, f2pack(0.1f, 0.1f));
         D[2 * k] = sqrt_approx(f2lo(s));
         D[2 * k + 1] = sqrt_approx(f2hi(s));
     }
     if (LAST == 1) {
-        if (SQ) {
-            const float dx = xrl - cx, dy = yrl - cy;
-            D[R] = fmaf(dy, dy, dx * dx);
-        } else {
-            D[R] = dist32<ATT>(xrl, yrl, cx, cy);
-        }
+        D[R] = dist32<ATT>(xrl, yrl, cx, cy);
     } else if (LAST == 2) {
         D[R] = __shfl_down_sync(0xffffffffu, D[0], 1);
     } else {
@@ -85,16 +75,23 @@ __device__ __forceinline__ void column_dists(const f32x2 (&xr2)[R / 2], const f3
 // hence, since a + b >= d1 + d2 >= 0,
 //     s1 + s2 = d1^2 + d2^2 <= (d1 + d2)^2 <= (a + b)^2 <= 2 a|a| + 2 b|b|        (s = dx^2 + dy^2; ATT: d^2 = s / 10)
 // — the last step is 2a^2 + 2b^2 - (a+b)^2 = (a-b)^2 >= 0 for a, b >= 0 and, for b < 0 <= a + b, (a - 3b)(a + b) >= 0.
-// Stage 1 tests  (s1 + cp_p) + s2 <= C_q  with the row constant cp_p = -pf_bound(ds_p) and the column constant
-// C_q = pf_bound(ds_q): squared distances only, no MUFU.  pf_bound(x) >= 2g (x + h)|x + h| (g = 1, ATT: 10) with a relative
-// slack PF_REL that covers every FP32 rounding of the squared domain and an absolute one (PF_ABS) for flushed denormals.
-// Padding rows / columns (ds = -BIG) give cp = +inf / C = -inf: never a hit, never a NaN.
+// So every such pair has  s1 + s2 - pf_bound(ds_p) - pf_bound(ds_q) <= 0  in real arithmetic, where
+// pf_bound(x) >= 2g (x + h)|x + h| (g = 1, ATT: 10) is an FP32 value with a relative slack PF_REL over its own roundings and
+// an absolute one (PF_ABS) for flushed denormals.
+// Stage 1 evaluates that left-hand side in expanded form, as a 4-term dot product.  With X' = x - c (the instance's
+// translation BiArgs::pf_cx / pf_cy, exact for every coordinate, so s is unchanged), P = point(p), P1 = point(p+1),
+// Q = point(q), Q1 = point(q+1):
+//     s1 + s2 - pf_p - pf_q = A_p + B_q + w_p . v_q,      w_p = -2 (X'_p, Y'_p, X'_p+1, Y'_p+1),  v_q = (X'_q, Y'_q, X'_q+1, Y'_q+1)
+//     A_p = |P'|^2 + |P1'|^2 - pf_p   (row constant),      B_q = |Q'|^2 + |Q1'|^2 - pf_q   (column constant)
+// The column loop does 4 FMAs per move from A_p, folds the rows with a minimum and adds B_q once per column; a block is a hit
+// when its minimum is <= 0.  pf_dot_const lowers A_p and B_q by the rounding margins of that chain (see there), so no pair
+// the square-root filter can pass is rejected.  Padding rows / columns (ds = -BIG) give pf = -inf, hence A = +inf /
+// B = +inf: never a hit, never a NaN (their coordinates are finite).
 // Stage 2 re-runs the square-root filter on the hitting lane's R x BI_CB block (bi_refilter_warp); only what survives it
 // reaches bi_cold_warp, so the exact path sees the same pairs as without the prefilter.
 //
-// PF_REL: the roundings of s (dx, dx^2, the FMA: < 4.1 ulp relative), of the two sums (< 2.1 ulp of |s1| + |s2| + |cp|) and
-// of each constant (< 3 ulp) add up to < 12 ulp = 2^-20.4 of 2g (a^2 + b^2); inflating both bounds by 2^-16 of themselves
-// gains 2g (a^2 + b^2) 2^-16, ~20x that.  PF_ABS: flush-to-zero can move a product or a sum by < 2^-126 each.
+// PF_REL: each constant rounds < 3 ulp; inflating it by 2^-16 of 2g (x + h)^2 keeps it above 2g (x + h)|x + h|.
+// PF_ABS: flush-to-zero can move a product or a sum by < 2^-126 each.
 constexpr float PF_REL = 0x1p-16f;
 constexpr float PF_ABS = 0x1p-100f;
 
@@ -105,6 +102,20 @@ __device__ __forceinline__ float pf_bound(float ds, float h) {
     return fmaf(a * (ATT ? 20.f : 2.f), fmaf(PF_REL, a, fabsf(a)), PF_ABS);
 }
 
+// DOT_REL: the four roundings of the FMA chain are < 4.01 ulp of |A| + sum |w_i v_i| <= |A| + |P^|^2 + |Q^|^2 (AM-GM,
+// P^ = (P', P1'), Q^ = (Q', Q1')), so that error splits into a row part and a column part.  Each constant also carries the
+// roundings of its norm (< 4.01 ulp), of nrm - pf (1 ulp), of the margin's sum and FMA (< 2 ulp), all relative to
+// K = nrm + |pf|: < 15 ulp of K for the row, < 11 for the column.  Both are lowered by 2^-19 = 32 ulp of K (DESIGN.md §3).
+// DOT_ABS: flushed or gradual-underflow results, < 2^-126 per operation.
+constexpr float DOT_REL = 0x1p-19f;
+constexpr float DOT_ABS = 0x1p-100f;
+
+// stage-1 row / column constant: nrm - pf lowered by its margin; +inf for padding (pf = -inf)
+__device__ __forceinline__ float pf_dot_const(float nrm, float pf) {
+    const float t = nrm - pf;
+    return pf == -INFINITY ? t : fmaf(-DOT_REL, nrm + fabsf(pf), t) - DOT_ABS;
+}
+
 // ---- cold path ------------------------------------------------------------------------------------------
 // Exact re-evaluation of one filter hit: the R x BI_CB pairs (rows p0..p0+R-1) x (columns Q0+jj0 .. +BI_CB-1) of ONE
 // thread whose FP32 block minimum passed the threshold.  WARP-COOPERATIVE: the whole warp is converged at the call (the
@@ -112,10 +123,9 @@ __device__ __forceinline__ float pf_bound(float ds, float h) {
 // from shared memory, row records from L2 — re-apply the FP32 filter, evaluate the survivors exactly (FP64 with the reference's
 // operation order, reference src/tabusearch.c:150 / src/distutil.c) and reduce the best exact (delta, i, j) key with
 // shuffles.  A hit costs a few hundred cycles instead of a serial walk over 32 pairs by a single lane.
-constexpr int BI_CB = 4;  // columns per filter check
+constexpr int BI_CB = 4;  // columns per filter check (the prefilter reads its column constants as one float4 per check)
 
-// PF: called from the prefilter kernel, whose column records hold C_q instead of ds_q (read from rec instead)
-template <int R, bool ATT, bool EXACT32, bool PF>
+template <int R, bool ATT, bool EXACT32>
 __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
                                              int jj0, float thr) {
     const int lane = threadIdx.x & 31;
@@ -128,7 +138,7 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
         if (idx < R * BI_CB && q >= p + 2 && q <= n - 1 && !(p == 0 && q == n - 1)) {  // reference tabusearch.c:134
             const float4 rp = __ldg(&rec[p]), rp1 = __ldg(&rec[p + 1]);  // row records: one L2 round trip for the warp
             const float4 c0 = sc[jj0 + c], c1 = sc[jj0 + c + 1];
-            const float dsq = PF ? __ldg(&rec[q].z) : c0.z;
+            const float dsq = c0.z;
             const float qv = (dist32<ATT>(rp.x, rp.y, c0.x, c0.y) - rp.z) + dist32<ATT>(rp1.x, rp1.y, c1.x, c1.y);
             if (qv <= thr + dsq) {
                 const int u = node_of(rp), v = node_of(c0);
@@ -219,8 +229,14 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
     float4 *scols1 = scols0 + (TJ + 2);
     const unsigned col_bytes = (unsigned)(TJ + 1) * 16u;
 
+    // PF: the stage-1 column operands of the current tile, written after its bulk copy has landed (one stage: the end-of-tile
+    // barrier orders the next tile's writes after this one's reads).  s_v[j] = {X'_j, X'_j, Y'_j, Y'_j}, so one LDS.128 gives
+    // both broadcast pairs of the packed FMAs; s_b[j] = B_j.
+    float4 *s_v = scols1 + (TJ + 2);                                       // [TJ+2] (PF only)
+    float *s_b = reinterpret_cast<float *>(s_v + (TJ + 2));                // [TJ+4] (PF only)
     // tile tables -> shared memory (one coalesced L2 round trip instead of a dependent chain per binary-search step)
-    int *s_rs = reinterpret_cast<int *>(scols1 + (TJ + 2));  // [ntr+1] prefix sums of tiles per tile-row
+    int *s_rs = PF ? reinterpret_cast<int *>(s_b + (TJ + 4))
+                   : reinterpret_cast<int *>(scols1 + (TJ + 2));  // [ntr+1] prefix sums of tiles per tile-row
     int *s_rj = s_rs + (A.ntr + 1);                          // [ntr]   first tile column of each tile-row
     __shared__ float s_pfthr;                                // PF: the block's threshold of the tile's bounds
     for (int k = tid; k <= A.ntr; k += BI_THREADS) {
@@ -273,6 +289,10 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
     MoveKey best = key_none();
     float thr = (float)s_hint + W;
     int pend_hint = 0;  // tid 0: value of ctl->hint fetched 64 columns ago
+    // PF: tid 0 keeps it in shared memory instead: in a register it would be live across the hit handling of every block,
+    // and the 96-register prefilter kernels for coordinates FP32 cannot hold would spill it to local memory
+    __shared__ int s_pend_hint;
+    if (PF && tid == 0) s_pend_hint = 0;
 
     // Tiles are DRAWN, not dealt: ctl->tile_next counts this rank's tiles handed out beyond the first wave (rank r owns
     // the tile ids r, r + world, ...; every tile costs the same — masked and padded pairs are computed too), so the blocks
@@ -354,12 +374,9 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
         const int buf = it & 1;
         const unsigned parity = (unsigned)(it >> 1) & 1u;
         const float4 *sc = buf ? scols1 : scols0;
-        // prefetch the next tile into the other stage (its slot in s_tile / scols was last read two tiles ago; PF: and
-        // written, so the bulk copy is ordered after those generic-proxy stores)
-        if (tid == 0) {
-            if (PF) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            draw(buf ^ 1, false);
-        }
+        // prefetch the next tile into the other stage (its slot in s_tile / scols was last read two tiles ago; only the bulk
+        // copy writes scols, so no proxy fence is needed)
+        if (tid == 0) draw(buf ^ 1, false);
 
         // rows of this thread: p0 .. p0+R-1 in packed pairs (+ successor row p0+R, scalar)
         const int p0 = SHUF ? P0 + (tid >> 5) * (32 * R - 1) + (tid & 31) * R : P0 + tid * R;
@@ -369,19 +386,28 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
         for (int k = 0; k < R / 2; ++k) {
             const float4 v0 = __ldg(&rec[p0 + 2 * k]), v1 = __ldg(&rec[p0 + 2 * k + 1]);
             // "+ 0" is a real FADD2 (not an identity for -0.0, so it is never folded): its 64-bit result is an aligned
-            // register pair that stays live across the column loop, instead of being re-packed with MOVs per step
+            // register pair that stays live across the column loop, instead of being re-packed with MOVs per step.
+            // PF: the translated coordinates X' = x - c (exact, see pf_dot_const)
             const f32x2 zero2 = f2pack(0.f, 0.f);
-            xr2[k] = f2add(f2pack(v0.x, v1.x), zero2);
-            yr2[k] = f2add(f2pack(v0.y, v1.y), zero2);
+            if (PF) {
+                xr2[k] = f2sub(f2pack(v0.x, v1.x), f2pack(A.pf_cx, A.pf_cx));
+                yr2[k] = f2sub(f2pack(v0.y, v1.y), f2pack(A.pf_cy, A.pf_cy));
+            } else {
+                xr2[k] = f2add(f2pack(v0.x, v1.x), zero2);
+                yr2[k] = f2add(f2pack(v0.y, v1.y), zero2);
+            }
             cp2[k] = f2sub(zero2, f2pack(v0.z, v1.z));  // padding rows carry ds = -BIG -> cp = +BIG -> never a candidate
         }
         if (!SHUF) {
             const float4 v = __ldg(&rec[p0 + R]);
-            xrl = v.x;
-            yrl = v.y;
+            xrl = PF ? v.x - A.pf_cx : v.x;
+            yrl = PF ? v.y - A.pf_cy : v.y;
         } else {
-            xrl = yrl = 0.f;
-            // lane 31's last row has its lower neighbour in another warp: never a candidate here (it is the next warp's first row)
+            // PF: the row below this lane's rows is the next lane's first one (lane 31 gets its own: finite, and masked)
+            xrl = PF ? __shfl_down_sync(0xffffffffu, f2lo(xr2[0]), 1) : 0.f;
+            yrl = PF ? __shfl_down_sync(0xffffffffu, f2lo(yr2[0]), 1) : 0.f;
+            // lane 31's last row has its lower neighbour in another warp: never a candidate here (it is the next warp's first
+            // row).  PF: -ds = BIG gives pf = -inf, hence A = +inf (pf_dot_const)
             if ((tid & 31) == 31) cp2[R / 2 - 1] = f2pack(f2lo(cp2[R / 2 - 1]), TSPB_BIG);
         }
         thr = fminf(thr, (float)(*((volatile int *)&s_hint)) + W);
@@ -389,21 +415,41 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
         mbar_wait(&bars[buf], parity);
         if (PRUNED && A.timing == 2 && tid == 0 && it == 0) A.dbg[8192 + 8 * blockIdx.x + 2] = globaltimer_ns();  // rows and columns of the first tile are here
 
+        // PF: stage-1 operands of this tile (see pf_dot_const), from ONE threshold for the whole block (thread 0's snapshot;
+        // every thread's thr is lowered to it, so h bounds every lane's (thr + E) / 2 until the end of the tile, when thr may
+        // have fallen: an older, larger h only admits more pairs).  Row pair k = rows (2k, 2k+1): w0 = -2 X', w1 = -2 Y' of
+        // those rows, w2 = -2 X', w3 = -2 Y' of the rows below them (2k+1, 2k+2), A2 = the row constants.  The column operands
+        // go to s_v / s_b once per tile; the bulk-copied records keep the original coordinates and ds for stages 2 and 3.
+        f32x2 w0[R / 2], w1[R / 2], w2[R / 2], w3[R / 2], A2[R / 2];
         if (PF) {
-            // prefilter bounds of this tile, from ONE threshold for the whole block (thread 0's snapshot; every thread's thr
-            // is lowered to it, so h bounds every lane's (thr + E) / 2 until the end of the tile, when thr may have fallen:
-            // an older, larger h only admits more pairs).  Column constants go to shared memory once per tile instead of
-            // four FP32 instructions per column and thread: the column record's ds slot (z) takes C_q, so the hot loop is the
-            // same code as the square-root kernel's (the exact path reads ds_q from rec).
             if (tid == 0) s_pfthr = (float)(*((volatile int *)&s_hint)) + W;
             __syncthreads();
             thr = fminf(thr, s_pfthr);
             const float h = 0.5f * (s_pfthr + A.pf_slack);
-            float4 *scw = buf ? scols1 : scols0;
-            for (int j = tid; j < NCv; j += BI_THREADS) scw[j].z = pf_bound<ATT>(scw[j].z, h);
+            for (int j = tid; j <= NCv; j += BI_THREADS) {
+                const float4 c = sc[j];
+                const float x = c.x - A.pf_cx, y = c.y - A.pf_cy;
+                s_v[j] = make_float4(x, x, y, y);
+                if (j < NCv) {
+                    const float4 c1 = sc[j + 1];
+                    const float x1 = c1.x - A.pf_cx, y1 = c1.y - A.pf_cy;
+                    s_b[j] = pf_dot_const(fmaf(y, y, x * x) + fmaf(y1, y1, x1 * x1), pf_bound<ATT>(c.z, h));
+                }
+            }
+            const f32x2 m2 = f2pack(-2.f, -2.f);
 #pragma unroll
-            for (int k = 0; k < R / 2; ++k)  // cp2 holds -ds here (padding / masked rows: -BIG -> +inf)
-                cp2[k] = f2pack(-pf_bound<ATT>(-f2lo(cp2[k]), h), -pf_bound<ATT>(-f2hi(cp2[k]), h));
+            for (int k = 0; k < R / 2; ++k) {
+                const f32x2 x1 = f2pack(f2hi(xr2[k]), k + 1 < R / 2 ? f2lo(xr2[(k + 1) % (R / 2)]) : xrl);
+                const f32x2 y1 = f2pack(f2hi(yr2[k]), k + 1 < R / 2 ? f2lo(yr2[(k + 1) % (R / 2)]) : yrl);
+                const f32x2 nrm = f2add(f2fma(yr2[k], yr2[k], f2mul(xr2[k], xr2[k])), f2fma(y1, y1, f2mul(x1, x1)));
+                w0[k] = f2mul(xr2[k], m2);
+                w1[k] = f2mul(yr2[k], m2);
+                w2[k] = f2mul(x1, m2);
+                w3[k] = f2mul(y1, m2);
+                // cp2 holds -ds (padding / masked rows: -BIG -> pf = -inf -> A = +inf)
+                A2[k] = f2pack(pf_dot_const(f2lo(nrm), pf_bound<ATT>(-f2lo(cp2[k]), h)),
+                               pf_dot_const(f2hi(nrm), pf_bound<ATT>(-f2hi(cp2[k]), h)));
+            }
             __syncthreads();
         }
 
@@ -411,35 +457,67 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
         const bool diag = (Q0 < P0 + TI + 1);
         const int NC = PRUNED ? NCv : TJ;  // columns of this tile
         // first column of the scan: D0 -> U2 (kept per variant so that the regular tile's shared-memory addressing stays uniform)
-        float4 c0, cnext;
-        f32x2 U2[R / 2];
-        // PF: the prefilter variant — D holds squared distances, U2 = s + cp (row constant), the column term is pf_bound(ds_q)
-        // and a block is a hit when its minimum is <= 0 (see pf_bound above)
-#define BI_INIT(JB, PF)                                                                                \
-    {                                                                                                  \
+        // PF: the column operands of q (qx, qy: {X'_q, X'_q}, {Y'_q, Y'_q}) and of q + 1 (vnext).  The 64-thread kernels (96
+        // registers) read them from s_v at the start of every BI_CB block and carry them within it only: nothing of the
+        // columns stays live across the hit handling (a noinline call), which keeps them free of spills.  The larger blocks
+        // have registers to spare and carry them from block to block (CARRY), which keeps their addressing uniform.
+        constexpr bool CARRY = BI_THREADS != 64;
+        float4 c0, cnext, vnext;
+        f32x2 U2[R / 2], qx, qy;
+#define BI_INIT(JB)                                                                                    \
+    if constexpr (PF) {                                                                                \
+        if (CARRY) {                                                                                   \
+            const float4 v0 = s_v[(JB)];                                                               \
+            qx = f2pack(v0.x, v0.y);                                                                   \
+            qy = f2pack(v0.z, v0.w);                                                                   \
+            vnext = s_v[(JB) + 1];                                                                     \
+        }                                                                                              \
+    } else {                                                                                           \
         c0 = sc[(JB)];                                                                                 \
         cnext = sc[(JB) + 1];                                                                          \
         float D0[R + 1];                                                                               \
-        column_dists<R, ATT, SHUF ? 0 : 1, PF>(xr2, yr2, xrl, yrl, c0.x, c0.y, D0);                    \
+        column_dists<R, ATT, SHUF ? 0 : 1>(xr2, yr2, xrl, yrl, c0.x, c0.y, D0);                        \
         _Pragma("unroll") for (int k = 0; k < R / 2; ++k) U2[k] = f2add(f2pack(D0[2 * k], D0[2 * k + 1]), cp2[k]); \
     }
 #define UU(r_) (((r_) & 1) ? f2hi(U2[(r_) >> 1]) : f2lo(U2[(r_) >> 1]))
 
 // one column: R+1 fresh distances -> R move deltas Q[r] = (D[p_r][q] - ds_p) + D[p_r+1][q+1]; the filter quantity
-// min_r Q[r] - ds_q is folded into the running block minimum M (no branch, no per-pair state kept)
-#define BI_COL(DIAG, jj_, PF)                                                                          \
-    {                                                                                                  \
+// min_r Q[r] - ds_q is folded into the running block minimum M (no branch, no per-pair state kept).
+// PF: acc = A_p + w_p . v_q, four packed FMAs per row pair; min_r acc + B_q is folded into M (bq: B of this block's columns)
+#define BI_COL(DIAG, jj_, c_)                                                                          \
+    if constexpr (PF) {                                                                                \
+        const float4 v1 = vnext;                                                                       \
+        if (CARRY) vnext = s_v[(jj_) + 2]; /* prefetched one column ahead */                           \
+        else if ((c_) + 1 < BI_CB) vnext = svj[(c_) + 2]; /* ... within the block */                   \
+        const f32x2 q1x = f2pack(v1.x, v1.y), q1y = f2pack(v1.z, v1.w);                                \
+        float m = TSPB_BIG;                                                                            \
+        _Pragma("unroll") for (int k = 0; k < R / 2; ++k) {                                            \
+            f32x2 acc = f2fma(w0[k], qx, A2[k]);                                                       \
+            acc = f2fma(w1[k], qy, acc);                                                               \
+            acc = f2fma(w2[k], q1x, acc);                                                              \
+            acc = f2fma(w3[k], q1y, acc);                                                              \
+            float a0 = f2lo(acc), a1 = f2hi(acc);                                                      \
+            if (DIAG) {                                                                                \
+                a0 = (qrel0 + (jj_) >= 2 * k + 2) ? a0 : TSPB_BIG;                                     \
+                a1 = (qrel0 + (jj_) >= 2 * k + 3) ? a1 : TSPB_BIG;                                     \
+            }                                                                                          \
+            m = fminf(m, fminf(a0, a1));                                                               \
+        }                                                                                              \
+        M = fminf(M, m + bq[(c_)]);                                                                    \
+        qx = q1x;                                                                                      \
+        qy = q1y;                                                                                      \
+    } else {                                                                                           \
         const float4 c1 = cnext;                                                                       \
         cnext = sc[(jj_) + 2]; /* prefetched one column ahead */                                       \
         float Dn[R + 1];                                                                               \
-        column_dists<R, ATT, SHUF ? 2 : 1, PF>(xr2, yr2, xrl, yrl, c1.x, c1.y, Dn);                    \
+        column_dists<R, ATT, SHUF ? 2 : 1>(xr2, yr2, xrl, yrl, c1.x, c1.y, Dn);                        \
         float m = TSPB_BIG;                                                                            \
         _Pragma("unroll") for (int r = 0; r < R; ++r) {                                                \
             float qv = UU(r) + Dn[r + 1];                                                              \
             if (DIAG) qv = (qrel0 + (jj_) >= r + 2) ? qv : TSPB_BIG;                                   \
             m = fminf(m, qv);                                                                          \
         }                                                                                              \
-        M = fminf(M, m - c0.z); /* PF: c0.z = C_q */                                                   \
+        M = fminf(M, m - c0.z);                                                                        \
         _Pragma("unroll") for (int k = 0; k < R / 2; ++k)                                              \
             U2[k] = f2add(f2pack(Dn[2 * k], Dn[2 * k + 1]), cp2[k]);                                   \
         c0 = c1;                                                                                       \
@@ -447,10 +525,20 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
 
 // BI_CB columns, then ONE filter check per warp (ballot); hits are resolved one lane at a time by the whole warp
 // (PF: a stage-1 hit first goes through stage 2, the square-root filter, and only its survivors to the exact path)
-#define BI_BLOCK(DIAG, PF)                                                                             \
+#define BI_BLOCK(DIAG)                                                                                 \
     for (int jj = 0; jj < NC; jj += BI_CB) {                                                           \
         float M = TSPB_BIG;                                                                            \
-        _Pragma("unroll") for (int c = 0; c < BI_CB; ++c) BI_COL(DIAG, jj + c, PF)                     \
+        const float4 b4 = PF ? *reinterpret_cast<const float4 *>(s_b + jj) : make_float4(0.f, 0.f, 0.f, 0.f); \
+        const float bq[BI_CB] = {b4.x, b4.y, b4.z, b4.w};                                              \
+        /* s_v + jj, spelled from s_b + jj: this form keeps the addresses in uniform registers */      \
+        const float4 *svj = reinterpret_cast<const float4 *>(s_b + 4 * jj) - (TJ + 2);                 \
+        if (PF && !CARRY) {                                                                            \
+            const float4 v0 = svj[0];                                                                  \
+            qx = f2pack(v0.x, v0.y);                                                                   \
+            qy = f2pack(v0.z, v0.w);                                                                   \
+            vnext = svj[1];                                                                            \
+        }                                                                                              \
+        _Pragma("unroll") for (int c = 0; c < BI_CB; ++c) { BI_COL(DIAG, jj + c, c) }                  \
         unsigned hits = __ballot_sync(0xffffffffu, M <= (PF ? 0.f : thr));                             \
         while (hits) {                                                                                 \
             const int L = __ffs(hits) - 1;                                                             \
@@ -462,7 +550,7 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
                 cold = bi_refilter_warp<R, ATT>(rec, sc, n, pL, Q0, jj, thrL);                         \
             }                                                                                          \
             if (cold) {                                                                                \
-                const MoveKey nb = bi_cold_warp<R, ATT, EXACT32, PF>(A.inst, rec, sc, n, pL, Q0, jj, thrL); \
+                const MoveKey nb = bi_cold_warp<R, ATT, EXACT32>(A.inst, rec, sc, n, pL, Q0, jj, thrL); \
                 if ((tid & 31) == L) {                                                                 \
                     atomicAdd(&ctl->cold_calls, 1ull);                                                 \
                     if (key_less(nb, best)) {                                                          \
@@ -481,8 +569,10 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
         /* requested 64 columns ago, so nobody waits for L2)                                                    */ \
         if ((jj & 63) == 64 - BI_CB) {                                                                 \
             if (tid == 0) {                                                                            \
-                if (pend_hint < 0) atomicMin(&s_hint, pend_hint);                                      \
-                pend_hint = __ldcg(&ctl->hint);                                                        \
+                const int ph = PF ? s_pend_hint : pend_hint;                                           \
+                if (ph < 0) atomicMin(&s_hint, ph);                                                    \
+                if (PF) s_pend_hint = __ldcg(&ctl->hint);                                              \
+                else pend_hint = __ldcg(&ctl->hint);                                                   \
             }                                                                                          \
             thr = fminf(thr, (float)(*((volatile int *)&s_hint)) + W);                                 \
         }                                                                                              \
@@ -490,11 +580,11 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
 
         const int qrel0 = Q0 - p0;  // q - p0 at jj = 0
         if (!diag) {
-            BI_INIT(0, PF)
-            BI_BLOCK(false, PF)
+            BI_INIT(0)
+            BI_BLOCK(false)
         } else {
-            BI_INIT(0, PF)
-            BI_BLOCK(true, PF)
+            BI_INIT(0)
+            BI_BLOCK(true)
         }
 #undef BI_INIT
 #undef BI_BLOCK
@@ -689,7 +779,9 @@ __global__ void TSPB_BI_BOUNDS bi_scan_sqrt_kernel(const BiArgs A) {
 // ---- host-side launchers -----------------------------------------------------------------------------
 template <int T, int R, bool SHUF>
 static inline cudaError_t launch_bi_tr(const BiArgs &a, int grid, bool pdl, cudaStream_t st) {
-    const size_t smem = (size_t)2 * (a.TJ + 2) * sizeof(float4) + (size_t)(2 * a.ntr + 2) * sizeof(int);
+    // two column stages, the prefilter's column operands (bi_scan_body: s_v, s_b), the tile tables
+    const size_t smem = (size_t)2 * (a.TJ + 2) * sizeof(float4) + (size_t)(2 * a.ntr + 2) * sizeof(int) +
+                        (a.prefilter ? (size_t)(a.TJ + 2) * sizeof(float4) + (size_t)(a.TJ + 4) * sizeof(float) : 0);
     const bool att = (a.inst.metric == M_ATT);
     const bool ex = a.inst.exact32 != 0;
     auto go = [&](auto kern) -> cudaError_t {

@@ -464,6 +464,7 @@ struct BiArgs {
     int row_shuffle; // 1: SHUF kernels (a warp owns 32 R - 1 rows, the distance below a lane's rows comes from the next lane)
     int prefilter;   // 1: stage-1 prefilter on squared distances in front of the FP32 filter (kernels_bi_scan.cuh)
     float pf_slack;  // prefilter: linear slack E of its row and column bounds (4 eps, DESIGN.md §3)
+    float pf_cx, pf_cy;  // prefilter: translation of the coordinates, exact for every one of them (0 if none is)
     int timing;      // 1: accumulate the per-pass breakdown in ctl->tm_acc; 2: also dump per-block {start, end} stamps
     unsigned long long *dbg;        // timing == 2: [gridDim.x][2] globaltimer stamps of the last pass
     XchgDev xchg;    // fuse_apply == 0: how this rank's key reaches the other ranks (enabled = 0 -> NCCL allreduce of ctl->packed)
