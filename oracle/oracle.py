@@ -188,6 +188,30 @@ class Oracle:
                                         row_end, threads, C.byref(sec), C.byref(bd), C.byref(bi), C.byref(bj))
         return ev, sec.value, (bd.value, bi.value, bj.value)
 
+    def bi_pairs_le(self, xy, wt, succ, H, threads=None) -> np.ndarray:
+        """Every legal pair of one best-improvement scan of `succ` whose exact delta is <= H: an (m, 3) int64 array of
+        (i, j, delta), i < j node indices, in (i, j) order."""
+        L = self.L
+        L.orc_bi_pairs_le.restype = C.c_int64
+        L.orc_bi_pairs_le.argtypes = [_f64p, C.c_int, C.c_int, _i32p, C.c_int64, C.c_int, C.POINTER(C.POINTER(OrcMove))]
+        L.orc_free.argtypes = [C.c_void_p]
+        xy = _as_xy(xy)
+        out = C.POINTER(OrcMove)()
+        m = L.orc_bi_pairs_le(xy, len(xy), wt, np.ascontiguousarray(succ, dtype=np.int32), int(H),
+                              threads or os.cpu_count() or 1, C.byref(out))
+        if m < 0:
+            raise MemoryError("orc_bi_pairs_le: out of memory")
+        try:
+            rec = np.ctypeslib.as_array(C.cast(out, C.POINTER(C.c_int32)), shape=(4 * m,)) if m else np.zeros(0, np.int32)
+            rec = rec.reshape(m, 4)
+            res = np.empty((m, 3), dtype=np.int64)
+            res[:, 0] = rec[:, 0]
+            res[:, 1] = rec[:, 1]
+            res[:, 2] = rec[:, 2:4].copy().view(np.int64)[:, 0]
+        finally:
+            L.orc_free(out)
+        return res
+
 
 class _InstanceLib:
     """A library that keeps reference `instance`s through the refshim_* calls and exports the reference's driver symbols."""

@@ -472,3 +472,90 @@ int64_t orc_bi_scan_rows_mt(const double *xy, int n, int weight_type, const int3
     *best_delta = bd; *best_i = bi; *best_j = bj;
     return evals;
 }
+
+/* ---- every pair at or below a threshold (tests of the FP32 filters: the pairs a filter must never reject) ---- */
+typedef struct {
+    const double *xy; int n; int wt; const int32_t *succ; const double *ds; double H;
+    int tid, nthreads;
+    orc_move *buf; int64_t len, cap;
+    int64_t *block_end;  /* len after each of this thread's row blocks */
+    int failed;
+} pairs_job;
+
+static void *pairs_worker(void *arg) {
+    pairs_job *jb = (pairs_job *)arg;
+    int k = 0;
+    for (int r0 = jb->tid * SCAN_BLOCK_ROWS; r0 < jb->n - 1; r0 += jb->nthreads * SCAN_BLOCK_ROWS, k++) {
+        int r1 = r0 + SCAN_BLOCK_ROWS < jb->n - 1 ? r0 + SCAN_BLOCK_ROWS : jb->n - 1;
+        for (int a = r0; a < r1 && !jb->failed; a++) {
+            for (int b = a + 1; b < jb->n; b++) {
+                int a1 = jb->succ[a], b1 = jb->succ[b];
+                if (b == a1 || b1 == a) continue;
+                /* move_delta's operation order; ds[] holds the same orc_dist values it would compute */
+                double delta = orc_dist(jb->xy, jb->wt, 1, a, b) + orc_dist(jb->xy, jb->wt, 1, a1, b1) - jb->ds[a] - jb->ds[b];
+                if (!(delta <= jb->H)) continue;
+                if (jb->len == jb->cap) {
+                    int64_t nc = jb->cap ? 2 * jb->cap : 1024;
+                    orc_move *nb = (orc_move *)realloc(jb->buf, sizeof(orc_move) * (size_t)nc);
+                    if (!nb) { jb->failed = 1; break; }
+                    jb->buf = nb;
+                    jb->cap = nc;
+                }
+                orc_move m = {a, b, (int64_t)delta};
+                jb->buf[jb->len++] = m;
+            }
+        }
+        jb->block_end[k] = jb->len;
+    }
+    return NULL;
+}
+
+int64_t orc_bi_pairs_le(const double *xy, int n, int weight_type, const int32_t *succ, int64_t H, int threads,
+                        orc_move **out) {
+    *out = NULL;
+    if (threads < 1) threads = 1;
+    if (threads > 256) threads = 256;
+    double *ds = (double *)malloc(sizeof(double) * (size_t)(n > 0 ? n : 1));
+    if (!ds) return -1;
+    for (int a = 0; a < n; a++) ds[a] = orc_dist(xy, weight_type, 1, a, succ[a]);
+    const int nblocks = n > 1 ? (n - 1 + SCAN_BLOCK_ROWS - 1) / SCAN_BLOCK_ROWS : 0;
+    const int per_thread = nblocks / threads + 1;
+    pthread_t th[256];
+    pairs_job jobs[256];
+    int failed = 0;
+    for (int t = 0; t < threads; t++) {
+        pairs_job jb = {xy, n, weight_type, succ, ds, (double)H, t, threads, NULL, 0, 0,
+                        (int64_t *)calloc((size_t)per_thread, sizeof(int64_t)), 0};
+        jobs[t] = jb;
+        if (!jobs[t].block_end) { failed = 1; continue; }
+        pthread_create(&th[t], NULL, pairs_worker, &jobs[t]);
+    }
+    int64_t total = 0;
+    for (int t = 0; t < threads; t++) {
+        if (!jobs[t].block_end) continue;
+        pthread_join(th[t], NULL);
+        failed |= jobs[t].failed;
+        total += jobs[t].len;
+    }
+    orc_move *res = failed ? NULL : (orc_move *)malloc(sizeof(orc_move) * (size_t)(total > 0 ? total : 1));
+    if (res) {  /* row block b was scanned by thread b % threads as its (b / threads)-th block */
+        int64_t at = 0;
+        for (int b = 0; b < nblocks; b++) {
+            pairs_job *jb = &jobs[b % threads];
+            const int k = b / threads;
+            const int64_t lo = k ? jb->block_end[k - 1] : 0, hi = jb->block_end[k];
+            memcpy(res + at, jb->buf + lo, sizeof(orc_move) * (size_t)(hi - lo));
+            at += hi - lo;
+        }
+    }
+    for (int t = 0; t < threads; t++) {
+        free(jobs[t].buf);
+        free(jobs[t].block_end);
+    }
+    free(ds);
+    if (!res) return -1;
+    *out = res;
+    return total;
+}
+
+void orc_free(void *p) { free(p); }

@@ -110,6 +110,13 @@ int64_t orc_bi_scan_rows_mt(const double *xy, int n, int weight_type, const int3
                             int row_begin, int row_end, int threads, double *seconds,
                             int64_t *best_delta, int32_t *best_i, int32_t *best_j);
 
+/* Every legal pair (a, b), a < b, of ONE best-improvement scan (same pairs and same delta arithmetic as
+ * orc_bi_scan_rows) whose exact delta is <= H.  *out gets a malloc'ed array (free it with orc_free), in
+ * (a, b) order; returns the number of pairs, -1 when out of memory. */
+int64_t orc_bi_pairs_le(const double *xy, int n, int weight_type, const int32_t *succ, int64_t H, int threads,
+                        orc_move **out);
+void orc_free(void *p);
+
 #ifdef __cplusplus
 }
 #endif

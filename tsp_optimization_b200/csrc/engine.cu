@@ -183,6 +183,12 @@ struct tspb200_ctx {
     int opt_em_global = 0;      // tests: extra mileage keeps its state in the global work buffer even when it fits shared memory
     int opt_batch_kernel = 0;   // batched best improvement: 0 = position-space kernel when applicable, 1 = always the node-space kernel
     unsigned long long *d_dbg = nullptr;  // per-block time stamps of the last pass ("timing" = 2)
+#if TSPB_FILTER_PROBE
+    int probe_H = 0;                      // option "probe": 0 = off, H <= -1 = pin the threshold of the coming passes at H + W
+    ProbeRec *d_probe = nullptr;          // records of the last probed pass (option "probe_cap" entries)
+    unsigned long long *d_probe_count = nullptr;
+    long long probe_cap = 0;
+#endif
     int opt_debug_shard = 0;    // timing experiments only: (world << 8 | rank) -> scan that rank's share of the tiles on one GPU  // -1 auto, 0 never, 1 whenever the tour fits in shared memory
     // benchmark hygiene: write this many bytes (> L2) before every pass and time each pass with its own event pair
     long long opt_flush_bytes = 0;
@@ -358,6 +364,10 @@ void tspb200_destroy(tspb200_ctx *ctx) {
         free_instance(ctx);
         for (int k = 0; k < 16; ++k) cudaFree(ctx->scratch_ptr[k]);
         cudaFree(ctx->d_dbg);
+#if TSPB_FILTER_PROBE
+        cudaFree(ctx->d_probe);
+        cudaFree(ctx->d_probe_count);
+#endif
         cudaFree(ctx->d_ctl);
         cudaFreeHost(ctx->h_ctl);
         cudaEventDestroy(ctx->ev0);
@@ -437,6 +447,24 @@ int tspb200_set_option(tspb200_ctx *ctx, const char *key, int64_t value) {
         ctx->opt_batch = (int)value;
     } else if (k == "time_limit_ms") {
         ctx->opt_time_limit_ms = value;
+#if TSPB_FILTER_PROBE
+    } else if (k == "probe") {
+        if (value > -1 && value != 0) return fail(ctx, TSPB200_E_ARG, "probe must be 0 (off) or a threshold H <= -1");
+        if (value < INT32_MIN) return fail(ctx, TSPB200_E_ARG, "probe threshold out of range");
+        if (value && !ctx->d_probe) return fail(ctx, TSPB200_E_STATE, "set probe_cap first");
+        ctx->probe_H = (int)value;
+    } else if (k == "probe_cap") {
+        if (value < 1) return fail(ctx, TSPB200_E_ARG, "probe_cap must be >= 1");
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaStreamSynchronize(ctx->stream));
+        cudaFree(ctx->d_probe);
+        ctx->d_probe = nullptr;
+        ctx->probe_cap = 0;
+        CK(cudaMalloc(&ctx->d_probe, sizeof(ProbeRec) * (size_t)value));
+        if (!ctx->d_probe_count) CK(cudaMalloc(&ctx->d_probe_count, sizeof(unsigned long long)));
+        CK(cudaMemset(ctx->d_probe_count, 0, sizeof(unsigned long long)));
+        ctx->probe_cap = value;
+#endif
     } else {
         return fail(ctx, TSPB200_E_ARG, "unknown option %s", key);
     }
@@ -476,6 +504,18 @@ int64_t tspb200_get_info(const tspb200_ctx *ctx, const char *key) {
     if (k == "exchange_p2p") return ctx->xchg.enabled && ctx->opt_exchange == 0;
     if (k == "world") return ctx->world;
     if (k == "rank") return ctx->rank;
+#if TSPB_FILTER_PROBE
+    if (k == "window_bits") {  // W exactly, as the kernels read it
+        uint32_t b;
+        memcpy(&b, &ctx->inst.W, sizeof b);
+        return (int64_t)b;
+    }
+    if (k == "probe_count") {  // records appended by the last probed pass (more than probe_cap: the buffer overflowed)
+        unsigned long long c = 0;
+        if (!ctx->d_probe_count || cudaMemcpy(&c, ctx->d_probe_count, sizeof c, cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
+        return (int64_t)c;
+    }
+#endif
     return -1;
 }
 
@@ -532,7 +572,8 @@ int tspb200_set_instance(tspb200_ctx *ctx, const double *xy, int n, int weight_t
     // FP32 filter usable when distances stay well inside the FP32 integer range (exact ds as float)
     const bool fp32_ok = finite && metric_fp32 && dmax < 4.0e6;
     // |D_fp32 - r_true| <= eps: MUFU.SQRT + the FP32 dx/dy/s roundings are < 2^-21 relative, coordinate rounding
-    // contributes <= 2*sqrt(2)*dc; see DESIGN.md §3 for the derivation of W = 2 + 2*eps (EUC needs 1 + 2*eps).
+    // contributes <= 2*sqrt(2)*dc; see DESIGN.md §3 for the derivation of W = 1 + 4*eps (EUC_2D) and 0.125 + 4*eps
+    // (CEIL_2D, ATT) below.
     double eps = dmax * std::ldexp(1.0, -20) + 4.0 * dc;
     ctx->inst = InstDev{};
     ctx->inst.n = n;
@@ -680,6 +721,13 @@ static InstDev inst_for_path(const tspb200_ctx *ctx, int path) {
     if (path == 2) { I.dmat = ctx->d_mat; I.dmat_ld = ctx->mat_ld; }
     else { I.dmat = nullptr; I.dmat_ld = 0; }
     if (path != 0) I.fp32_ok = 0;
+#if TSPB_FILTER_PROBE
+    I.probe_on = ctx->probe_H != 0;
+    I.probe_H = ctx->probe_H;
+    I.probe_rec = ctx->d_probe;
+    I.probe_count = ctx->d_probe_count;
+    I.probe_cap = ctx->probe_cap;
+#endif
     return I;
 }
 
@@ -783,6 +831,16 @@ static void plan_tiles(tspb200_ctx *ctx, std::vector<int> &row_start, std::vecto
 // last best-improvement pass run with option "timing" = 2).
 int tspb200_debug_fetch(tspb200_ctx *ctx, const char *what, void *out, int64_t bytes) {
     if (!ctx || !ctx->stream || !what || !out) return TSPB200_E_ARG;
+#if TSPB_FILTER_PROBE
+    if (std::string(what) == "probe") {  // the records of the last probed pass, at most probe_cap of them
+        if (!ctx->d_probe) return fail(ctx, TSPB200_E_STATE, "nothing recorded for probe");
+        CK(cudaSetDevice(ctx->device));
+        CK(cudaStreamSynchronize(ctx->stream));
+        const int64_t have = (int64_t)sizeof(ProbeRec) * ctx->probe_cap;
+        CK(cudaMemcpy(out, ctx->d_probe, (size_t)(bytes < have ? bytes : have), cudaMemcpyDeviceToHost));
+        return TSPB200_OK;
+    }
+#endif
     const bool phases = std::string(what) == "block_phases";  // [grid][8]: start, drawn, loaded, scanned, folded, tiles, ticket, -
     if ((std::string(what) != "block_times" && !phases) || !ctx->d_dbg) return fail(ctx, TSPB200_E_STATE, "nothing recorded for %s", what);
     const int64_t have = (int64_t)sizeof(unsigned long long) * (phases ? 8 : 2) * 4096;
@@ -1086,9 +1144,19 @@ int tspb200_bi_run(tspb200_ctx *ctx, int64_t max_passes, tspb200_stats *st) {
     // "seed_hint" = 2: the apply launch's last block re-evaluates every block winner of the pass and seeds the next pass's
     // filter with the best one that is still legal.  It halves the exact-path calls of a one-wave pass (n = 10 000: 356 k ->
     // 188 k per run) but lengthens the serial section by ~5 us, a net loss (36.4 vs 32.3 us per pass): off by default.
-    const bool seed_all = path == 0 && !prune && ctx->opt_seed_hint >= 2;
+    bool seed_all = path == 0 && !prune && ctx->opt_seed_hint >= 2;
+    int grid_seed = ctx->grid_bi;  // block winners of the previous pass the pruned mode's tile_boxes_kernel re-evaluates
     int rc = sync_ctl(ctx);
     if (rc) return rc;
+#if TSPB_FILTER_PROBE
+    if (I.probe_on) {  // the threshold starts at H and no seed may lower it (the cold paths return no key)
+        a.seed_hint = 0;
+        seed_all = false;
+        grid_seed = 0;
+        ctx->h_ctl->hint = ctx->probe_H;  // copied to the device by prepare_run
+        CK(cudaMemsetAsync(ctx->d_probe_count, 0, sizeof(unsigned long long), ctx->stream));
+    }
+#endif
     rc = prepare_run(ctx, false, -1);
     if (rc) return rc;
     const long long passes0 = ctx->h_ctl->passes, moves0 = ctx->h_ctl->moves, delta0 = ctx->h_ctl->obj_delta;
@@ -1139,7 +1207,7 @@ int tspb200_bi_run(tspb200_ctx *ctx, int64_t max_passes, tspb200_stats *st) {
                 CK(cudaEventRecord(ctx->pass_events[2 * q], ctx->stream));
             }
             if (prune) {
-                CK(launch_tile_prune(a, bi_tile_rows(ctx->T, ctx->R, ctx->row_shuffle), ctx->grid_bi, pdl, ctx->stream));
+                CK(launch_tile_prune(a, bi_tile_rows(ctx->T, ctx->R, ctx->row_shuffle), grid_seed, pdl, ctx->stream));
                 host_launches += 2;
             }
             if (ctx->tabu_on)
@@ -1441,6 +1509,9 @@ static int run_batch(tspb200_ctx *ctx, int mode, int32_t *succ, double *obj, int
     CK(cudaMemcpyAsync(d_succ, succ, sizeof(int) * (size_t)n * batch, cudaMemcpyHostToDevice, ctx->stream));
     CK(cudaMemsetAsync(d_delta, 0, sizeof(long long) * (size_t)batch, ctx->stream));
     CK(cudaMemsetAsync(d_cnt, 0, sizeof(long long) * 4 * (size_t)batch, ctx->stream));
+#if TSPB_FILTER_PROBE
+    if (I.probe_on) CK(cudaMemsetAsync(ctx->d_probe_count, 0, sizeof(unsigned long long), ctx->stream));
+#endif
     int launched = 0;
     // best improvement on the FP32-filter path: the position-space block kernel; everything else: the node-space one
     cudaError_t le = cudaErrorNotSupported;

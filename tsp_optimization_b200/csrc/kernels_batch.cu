@@ -366,7 +366,8 @@ constexpr int BPOS_THREADS = 128;
 constexpr int BPOS_CB = 4;
 
 template <int R, bool ATT, bool EXACT32>
-__device__ __noinline__ MoveKey bpos_cold_warp(const InstDev I, const float4 *rec, int n, int p0, int q0, float thr) {
+__device__ __noinline__ MoveKey bpos_cold_warp(const InstDev I, const float4 *rec, int n, int p0, int q0, float thr
+                                               TSPB_PROBE_ARG(int own_rows)) {
     const int lane = threadIdx.x & 31;
     MoveKey best = key_none();
 #pragma unroll 1
@@ -377,7 +378,7 @@ __device__ __noinline__ MoveKey bpos_cold_warp(const InstDev I, const float4 *re
         if (idx < R * BPOS_CB && q >= p + 2 && q <= n - 1 && !(p == 0 && q == n - 1)) {  // reference tabusearch.c:134
             const float4 rp = rec[p], rp1 = rec[p + 1], c0 = rec[q], c1 = rec[q + 1];
             const float qv = (bt_dist32<ATT>(rp.x, rp.y, c0.x, c0.y) - rp.z) + bt_dist32<ATT>(rp1.x, rp1.y, c1.x, c1.y);
-            if (qv <= thr + c0.z) {
+            if (qv <= thr + c0.z TSPB_PROBE_OR(I.probe_on)) {
                 const int u = node_of(rp), v = node_of(c0);
                 long long d1, d2;
                 if (EXACT32) {
@@ -388,6 +389,12 @@ __device__ __noinline__ MoveKey bpos_cold_warp(const InstDev I, const float4 *re
                     d2 = exact_dist(I.metric, I.pt64[node_of(rp1)], I.pt64[node_of(c1)]);
                 }
                 const long long delta = d1 + d2 - (long long)rp.z - (long long)c0.z;
+#if TSPB_FILTER_PROBE
+                if (I.probe_on) {  // as bi_cold_warp
+                    if (r < own_rows && delta <= I.probe_H) probe_record(I, u, v, delta, qv, thr, qv <= thr + c0.z);
+                    continue;
+                }
+#endif
                 if (delta < 0) {
                     MoveKey k;
                     k.delta = (int)delta; k.i = min(u, v); k.j = max(u, v); k.pad = 0;
@@ -469,7 +476,7 @@ __device__ __forceinline__ void bpos_scan(const InstDev &I, const float4 *rec, i
         while (hits) {
             const int L = __ffs(hits) - 1;
             const float thrL = __shfl_sync(0xffffffffu, thr, L);
-            const MoveKey nb = bpos_cold_warp<R, ATT, EXACT32>(I, rec, n, p0w + L * R, q4, thrL);
+            const MoveKey nb = bpos_cold_warp<R, ATT, EXACT32>(I, rec, n, p0w + L * R, q4, thrL TSPB_PROBE_ARG(L == 31 ? R - 1 : R));
             if (lane == L) {
                 colds += 1;
                 if (key_less(nb, best)) {
@@ -552,7 +559,11 @@ __global__ void __launch_bounds__(BPOS_THREADS) two_opt_batch_bi_kernel(const In
                 pos[u] = p;
                 rec[p].z = (float)dist_nodes(I, u, v);
             }
+#if TSPB_FILTER_PROBE
+            if (tid == 0) s_hint = I.probe_on ? I.probe_H : 0;  // pinned: bpos_cold_warp returns no key, the pass ends with none
+#else
             if (tid == 0) s_hint = 0;
+#endif
             __syncthreads();
         }
         if (!s_err && n >= 4) {

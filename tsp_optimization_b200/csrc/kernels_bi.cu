@@ -114,8 +114,11 @@ __global__ void __launch_bounds__(256) apply_move_kernel(const InstDev inst, con
 // exceeds `hint` — the exact delta of some legal move, i.e. an upper bound of the pass minimum — can hold neither the
 // argmin nor a tie (a tie needs delta == minimum <= hint), so skipping it cannot change the selected move: the move log
 // stays the reference's bit for bit, only the number of evaluated pairs drops.  The bound is evaluated in FP32 from the
-// FP32 records; W (>= 2 + the FP32 / coordinate-rounding error of a distance, see set_instance) plus 1 is subtracted,
-// far more than the roundings of the few operations below can add up to.
+// FP32 records, and W + 1 is subtracted from it: W = 1 + 4 eps (EUC_2D) or 0.125 + 4 eps (CEIL_2D, ATT), DESIGN.md §3,
+// with eps = dmax 2^-20 + 4 dc (tspb200_set_instance).  The "- 1" of the bound above is the rounding of the two exact
+// distances; the 4 eps of W cover the FP32 side: the coordinate rounding of the boxes (<= 2 sqrt(2) dc per distance) and
+// the roundings of the few operations below (sqrtf and the product 2 bd scale: a few ulp of 2 dmax, then one rounding per
+// subtraction: together < dmax 2^-20 = eps).  The scale constants lie below 1/sqrt(10) and 1.
 __global__ void __launch_bounds__(64) tile_boxes_kernel(const InstDev inst, const TourDev tour, int TI, int TJ, int ntr, int ncb,
                                                         int ncb2, int nseed) {
     __shared__ float s_r[2][5];

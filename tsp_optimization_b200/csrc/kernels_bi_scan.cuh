@@ -127,7 +127,7 @@ constexpr int BI_CB = 4;  // columns per filter check (the prefilter reads its c
 
 template <int R, bool ATT, bool EXACT32>
 __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
-                                             int jj0, float thr) {
+                                             int jj0, float thr TSPB_PROBE_ARG(int own_rows)) {
     const int lane = threadIdx.x & 31;
     MoveKey best = key_none();
 #pragma unroll 1
@@ -140,7 +140,7 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
             const float4 c0 = sc[jj0 + c], c1 = sc[jj0 + c + 1];
             const float dsq = c0.z;
             const float qv = (dist32<ATT>(rp.x, rp.y, c0.x, c0.y) - rp.z) + dist32<ATT>(rp1.x, rp1.y, c1.x, c1.y);
-            if (qv <= thr + dsq) {
+            if (qv <= thr + dsq TSPB_PROBE_OR(I.probe_on)) {
                 const int u = node_of(rp), v = node_of(c0);
                 long long d1, d2;
                 if (EXACT32) {
@@ -151,6 +151,12 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
                     d2 = exact_dist(I.metric, I.pt64[node_of(rp1)], I.pt64[node_of(c1)]);
                 }
                 const long long delta = d1 + d2 - (long long)rp.z - (long long)dsq;
+#if TSPB_FILTER_PROBE
+                if (I.probe_on) {  // every pair, passed or not; rows the calling lane owns only; no key (the threshold stays pinned)
+                    if (r < own_rows && delta <= I.probe_H) probe_record(I, u, v, delta, qv, thr, qv <= thr + dsq);
+                    continue;
+                }
+#endif
                 if (delta < 0) {
                     MoveKey k;
                     k.delta = (int)delta; k.i = min(u, v); k.j = max(u, v); k.pad = 0;
@@ -550,7 +556,8 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
                 cold = bi_refilter_warp<R, ATT>(rec, sc, n, pL, Q0, jj, thrL);                         \
             }                                                                                          \
             if (cold) {                                                                                \
-                const MoveKey nb = bi_cold_warp<R, ATT, EXACT32>(A.inst, rec, sc, n, pL, Q0, jj, thrL); \
+                const MoveKey nb = bi_cold_warp<R, ATT, EXACT32>(A.inst, rec, sc, n, pL, Q0, jj, thrL                   \
+                                                                 TSPB_PROBE_ARG(SHUF && L == 31 ? R - 1 : R)); \
                 if ((tid & 31) == L) {                                                                 \
                     atomicAdd(&ctl->cold_calls, 1ull);                                                 \
                     if (key_less(nb, best)) {                                                          \

@@ -17,6 +17,27 @@
 
 namespace tspb {
 
+#ifndef TSPB_FILTER_PROBE
+// 1: the filter probe build (make OUT=../lib/probe EXTRA=-DTSPB_FILTER_PROBE=1; tests/test_gpu_filter_probe.py).  Option
+// "probe" = H <= -1 pins the threshold of the next best-improvement pass at H + W (nothing lowers it: the cold paths record
+// and return no key, no seed tightens the hint), and the cold paths record every pair of their R x 4 block whose exact
+// delta is <= H.  The product build keeps it 0: none of this exists there.
+#define TSPB_FILTER_PROBE 0
+#endif
+
+#if TSPB_FILTER_PROBE
+struct ProbeRec {  // one pair seen by a cold path: node ids i < j, exact delta, the FP32 filter value, threshold and verdict
+    int i, j, delta;
+    float qv, thr;
+    int passed, pad0, pad1;
+};
+#define TSPB_PROBE_ARG(x) , x
+#define TSPB_PROBE_OR(x) || (x)
+#else
+#define TSPB_PROBE_ARG(x)
+#define TSPB_PROBE_OR(x)
+#endif
+
 struct InstDev {
     int n;
     int metric;             // reference weight_type value
@@ -29,7 +50,26 @@ struct InstDev {
     const float2 *pt32;     // node-indexed FP32 points
     const int *dmat;        // optional n x ld int32 distance matrix (matrix mode), else nullptr
     long long dmat_ld;
+#if TSPB_FILTER_PROBE
+    int probe_on;                    // the threshold is pinned at probe_H + W and the cold paths record
+    int probe_H;
+    ProbeRec *probe_rec;             // [probe_cap]
+    unsigned long long *probe_count; // records appended (beyond probe_cap: counted, not written)
+    long long probe_cap;
+#endif
 };
+
+#if TSPB_FILTER_PROBE
+__device__ __forceinline__ void probe_record(const InstDev &I, int u, int v, long long delta, float qv, float thr, bool passed) {
+    const unsigned long long k = atomicAdd(I.probe_count, 1ull);
+    if ((long long)k < I.probe_cap) {
+        ProbeRec r;
+        r.i = min(u, v); r.j = max(u, v); r.delta = (int)delta;
+        r.qv = qv; r.thr = thr; r.passed = passed ? 1 : 0; r.pad0 = r.pad1 = 0;
+        I.probe_rec[k] = r;
+    }
+}
+#endif
 
 struct MoveRec {  // one applied move, as logged for parity tests
     int i, j;

@@ -75,15 +75,16 @@ class Stats:
                      s.tiles_scanned, s.tiles_total)
 
 
-_lib = None
+_libs = {}
 
 
-def load_library() -> C.CDLL:
-    """Load libtspb200.so (built in-tree by ``__graft_entry__.build()`` / ``make -C tsp_optimization_b200/csrc``)."""
-    global _lib
-    if _lib is not None:
-        return _lib
-    path = os.environ.get("TSPB200_LIB", LIB_PATH)  # development: A/B timing of another build of the same ABI
+def load_library(path: str | None = None) -> C.CDLL:
+    """Load libtspb200.so (built in-tree by ``__graft_entry__.build()`` / ``make -C tsp_optimization_b200/csrc``), or another
+    build of the same ABI at `path` (e.g. the filter probe build, tests/test_gpu_filter_probe.py).  One handle per path."""
+    if path is None:
+        path = os.environ.get("TSPB200_LIB", LIB_PATH)  # development: A/B timing of another build of the same ABI
+    if path in _libs:
+        return _libs[path]
     if not os.path.exists(path):
         raise TspB200Error(-1, f"{path} is missing: build it with `make -C tsp_optimization_b200/csrc` "
                                "(there is no CPU fallback)")
@@ -138,7 +139,7 @@ def load_library() -> C.CDLL:
         L.tspb200_population_two_opt.argtypes = [vp, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(_Stats)]
     if hasattr(L, "tspb200_debug_fetch"):
         L.tspb200_debug_fetch.argtypes = [vp, C.c_char_p, C.c_void_p, i64]
-    _lib = L
+    _libs[path] = L
     return L
 
 
@@ -193,8 +194,8 @@ def _moves_to_array(buf, k: int) -> np.ndarray:
 class Engine:
     """One engine = one CUDA device + stream; holds one instance and one resident tour."""
 
-    def __init__(self, device: int = 0):
-        self.L = load_library()
+    def __init__(self, device: int = 0, lib_path: str | None = None):
+        self.L = load_library(lib_path)
         self.h = C.c_void_p()
         rc = self.L.tspb200_create(device, C.byref(self.h))
         if rc:
