@@ -206,6 +206,20 @@ int tspb200_population_upload(tspb200_ctx *ctx, const int32_t *tours, const int3
 int tspb200_population_download(tspb200_ctx *ctx, int32_t *tours, const int32_t *slots, int count, int as_order);
 int tspb200_population_costs(tspb200_ctx *ctx, const int32_t *slots, int count, double *out);
 int tspb200_population_two_opt(tspb200_ctx *ctx, int mode, const int32_t *slots, int count, double *obj, tspb200_stats *st);
+/* Independent VNS chains on the resident population (reference HEU_VNS, src/vns.c:103-183), one launch for all of them: for
+ * every listed slot b (the first `count` when slots == NULL) and t = 0 .. iters-1: kick the slot's tour with the three tour
+ * indices kicks[(b*iters + t)*3 .. +2] (counted from node 0, any order, the rules of tspb200_vns_kick), run alg_2opt (first
+ * improvement from a fresh sweep) to the local optimum, and keep the result iff its cost is strictly below the slot's
+ * current cost, else go back to the slot's tour.  At return each slot holds its chain's incumbent.  A chain's whole state
+ * is its slot's tour (the cost is recomputed at the start), so iters = K1 and then K2 with the next kicks equals one call
+ * with K1 + K2; iters = 0 returns the current costs.  best = count doubles out (incumbent costs, may be NULL); trace =
+ * count*iters doubles out (cost after each iteration's 2-opt: below the previous incumbent = accepted, may be NULL);
+ * st = moves, sweeps (passes), evals, gpu_ms and launches summed over all chains and iterations.  Every triple is checked
+ * first: a bad one gives TSPB200_E_ARG (naming the chain and the iteration) and leaves the population untouched.  Needs n
+ * to fit one block's shared memory (28 bytes per node, as tspb200_population_two_opt) and distances < 2^24
+ * (TSPB200_E_UNSUPPORTED); a slot that is not one cycle gives TSPB200_E_DEVICE_CHECK. */
+int tspb200_population_vns(tspb200_ctx *ctx, const int32_t *slots, int count, const int32_t *kicks, int iters, double *best,
+                           double *trace, tspb200_stats *st);
 
 /* ---- multi-GPU (one process per GPU; the caller bootstraps the id, e.g. over torch.distributed) ---- */
 /* Neighbourhood sharding: with a communicator attached, tspb200_bi_run deals the pair tiles round-robin over the ranks;

@@ -74,6 +74,7 @@ cudaError_t launch_two_opt_batch(const InstDev &I, int mode, int *succ, const in
 cudaError_t launch_two_opt_batch_bi_pos(const InstDev &I, int *succ, const int *slots, long long *obj, long long *counters, int batch,
                                         int num_sms, cudaStream_t st, int *launched, MoveRec *log, long long log_cap);
 cudaError_t launch_vns_kick(const InstDev &I, const TourDev &T, int idx1, int idx2, int idx3, float4 *scratch, cudaStream_t st);
+cudaError_t launch_vns_chains(const InstDev &I, int count, int num_sms, int *grid, const VnsChainArgs *a, cudaStream_t st);
 cudaError_t launch_tabu_kick_select(const TourDev &T, int *skip, const int *pairs, int count, int iter, int tenure, int *accepted,
                                     cudaStream_t st);
 cudaError_t launch_population_store(const int *staged, int *pop, const int *slots, int n, int count, int as_order, cudaStream_t st);
@@ -2053,6 +2054,80 @@ int tspb200_population_two_opt(tspb200_ctx *ctx, int mode, const int32_t *slots,
     CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
     local.gpu_ms = ms;
     local.launches = launched;
+    local.path = path;
+    local.status = TSPB200_LOCAL_OPTIMUM;
+    if (st) *st = local;
+    return TSPB200_OK;
+}
+
+// Independent VNS chains (HEU_VNS, reference src/vns.c:103-183) on the listed slots, one thread block per chain: kicks[(b*iters +
+// t)*3 ..] are chain b's tour indices of iteration t.  Every triple is checked before anything is launched, so a bad one
+// leaves the population as it was.
+int tspb200_population_vns(tspb200_ctx *ctx, const int32_t *slots, int count, const int32_t *kicks, int iters, double *best,
+                           double *trace, tspb200_stats *st) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (ctx->pop_count < 1 || ctx->pop_n != ctx->n) return fail(ctx, TSPB200_E_STATE, "no resident population");
+    if (count < 1 || (!slots && count > ctx->pop_count) || iters < 0 || (iters > 0 && !kicks)) return fail(ctx, TSPB200_E_ARG, "bad arguments");
+    if (!(ctx->dist_bound < 16777216.0)) return fail(ctx, TSPB200_E_UNSUPPORTED, "distances >= 2^24 are not supported by the 2-opt kernels");
+    const int n = ctx->n;
+    const size_t nk = (size_t)count * (size_t)iters;
+    std::vector<int32_t> sorted(3 * nk);
+    for (size_t q = 0; q < nk; ++q) {  // the rules of tspb200_vns_kick (reference vns.c:25-50)
+        int i1 = kicks[3 * q], i2 = kicks[3 * q + 1], i3 = kicks[3 * q + 2];
+        if (i1 > i2) std::swap(i1, i2);
+        if (i1 > i3) std::swap(i1, i3);
+        if (i2 > i3) std::swap(i2, i3);
+        if (i1 < 0 || i3 >= n || i2 - i1 < 2 || i3 - i2 < 2)
+            return fail(ctx, TSPB200_E_ARG, "chain %d, iteration %d: kick (%d, %d, %d) is not three distinct, non-adjacent tour indices in [0, %d)",
+                        (int)(q / (size_t)iters), (int)(q % (size_t)iters), kicks[3 * q], kicks[3 * q + 1], kicks[3 * q + 2], n);
+        sorted[3 * q] = i1; sorted[3 * q + 1] = i2; sorted[3 * q + 2] = i3;
+    }
+    CK(cudaSetDevice(ctx->device));
+    const int path = select_path(ctx);
+    if (path == 2 && !ctx->d_mat) return fail(ctx, TSPB200_E_STATE, "matrix path selected but no resident matrix");
+    InstDev I = inst_for_path(ctx, path);
+    int grid = 0;
+    cudaError_t le = launch_vns_chains(I, count, ctx->num_sms, &grid, nullptr, ctx->stream);
+    if (le == cudaErrorInvalidValue)
+        return fail(ctx, TSPB200_E_UNSUPPORTED, "VNS chains use the one-block kernel: n=%d does not fit one block's shared memory", n);
+    if (le != cudaSuccess) return fail(ctx, TSPB200_E_CUDA, "VNS chain kernel setup failed: %s", cudaGetErrorString(le));
+    int *d_slots = nullptr;
+    int rc = pop_slots_to_device(ctx, slots, count, &d_slots);
+    if (rc) return rc;
+    SCRATCH(d_image, unsigned *, 0, sizeof(unsigned) * 5 * (size_t)n * (size_t)grid);
+    SCRATCH(d_best, long long *, 1, sizeof(long long) * (size_t)count);
+    SCRATCH(d_cnt, long long *, 2, sizeof(long long) * 4 * (size_t)count);
+    SCRATCH(d_kicks, int *, 3, sizeof(int) * 3 * nk);
+    long long *d_trace = nullptr;
+    if (trace && nk) {
+        SCRATCH(d_t, long long *, 14, sizeof(long long) * nk);
+        d_trace = d_t;
+    }
+    CK(cudaEventRecord(ctx->ev0, ctx->stream));
+    if (nk) CK(cudaMemcpyAsync(d_kicks, sorted.data(), sizeof(int) * 3 * nk, cudaMemcpyHostToDevice, ctx->stream));
+    VnsChainArgs a{ctx->d_pop, d_slots, d_kicks, iters, d_image, d_best, d_trace, d_cnt};
+    le = launch_vns_chains(I, count, ctx->num_sms, &grid, &a, ctx->stream);
+    if (le != cudaSuccess) return fail(ctx, TSPB200_E_CUDA, "VNS chain launch failed: %s", cudaGetErrorString(le));
+    std::vector<long long> h_best((size_t)count), h_cnt((size_t)count * 4), h_trace(d_trace ? nk : 0);
+    CK(cudaMemcpyAsync(h_best.data(), d_best, sizeof(long long) * (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(h_cnt.data(), d_cnt, sizeof(long long) * 4 * (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_trace) CK(cudaMemcpyAsync(h_trace.data(), d_trace, sizeof(long long) * nk, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaEventRecord(ctx->ev1, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    tspb200_stats local;
+    memset(&local, 0, sizeof local);
+    for (int b = 0; b < count; ++b) {
+        if (h_cnt[4 * (size_t)b + 3]) return fail(ctx, TSPB200_E_DEVICE_CHECK, "population slot %d does not hold a single cycle", slots ? slots[b] : b);
+        local.moves += h_cnt[4 * (size_t)b + 0];
+        local.passes += h_cnt[4 * (size_t)b + 1];
+        local.evals += h_cnt[4 * (size_t)b + 2];
+        if (best) best[b] = (double)h_best[(size_t)b];
+    }
+    for (size_t q = 0; q < h_trace.size(); ++q) trace[q] = (double)h_trace[q];
+    float ms = 0;
+    CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    local.gpu_ms = ms;
+    local.launches = 1;
     local.path = path;
     local.status = TSPB200_LOCAL_OPTIMUM;
     if (st) *st = local;

@@ -93,6 +93,149 @@ __device__ __forceinline__ void bt_apply(const InstDev &I, const BatchSmem &S, b
     __syncthreads();
 }
 
+// Loads tour `gsucc` and the coordinates into shared memory and lays out the visiting order from node 0; *err = 1 when
+// gsucc is not one cycle over the n nodes.
+__device__ __forceinline__ void bt_load_tour(const InstDev &I, const BatchSmem &S, const int *gsucc, int n, int *err) {
+    const int tid = threadIdx.x;
+    for (int k = tid; k < n; k += BATCH_THREADS) {
+        float2 p = I.pt32[k];
+        S.sx[k] = p.x; S.sy[k] = p.y;
+        S.succ[k] = gsucc[k];
+    }
+    if (tid == 0) *err = 0;
+    __syncthreads();
+    if (tid == 0) {  // visiting order from node 0; also validates the cycle
+        int at = 0;
+        for (int p = 0; p < n; ++p) {
+            if (at < 0 || at >= n || (p > 0 && at == 0)) { *err = 1; break; }
+            S.order[p] = at;
+            S.pos[at] = p;
+            at = S.succ[at];
+        }
+        if (at != 0) *err = 1;
+    }
+    __syncthreads();
+}
+
+// exact length of every tour edge, in node space (dsn) and position space (dsp)
+__device__ __forceinline__ void bt_edges(const InstDev &I, const BatchSmem &S, bool exact32, int n) {
+    for (int k = threadIdx.x; k < n; k += BATCH_THREADS) {
+        const float d = (float)bt_exact(I, S, exact32, k, S.succ[k]);
+        S.dsn[k] = d;
+        S.dsp[S.pos[k]] = d;
+    }
+    __syncthreads();
+}
+
+// alg_2opt (reference src/heuristics.c:438-502) on the shared-memory tour, from a fresh sweep to the local optimum.
+// moves / passes / evals / objd (sum of the applied deltas) are accumulated, identically in every thread.
+template <bool ATT, bool EXACT32, bool FP32_OK>
+__device__ __forceinline__ void bt_fi_sweep(const InstDev &I, const BatchSmem &S, int n, float W, int *s_hits, MoveRec *log,
+                                            long long log_cap, long long &moves, long long &passes, long long &evals,
+                                            long long &objd) {
+    const int tid = threadIdx.x;
+    const bool ex32 = FP32_OK && EXACT32;
+    // The reference's sweep is a linear scan of the pairs in row-major order from a cursor.  The block scans a
+    // WINDOW of that linear order per step: chunks of 32 consecutive pairs (crossing row ends) are dealt to the
+    // 8 warps round-robin, K chunks per warp, each warp stopping at its first improving pair; the smallest
+    // linear offset over the warps is the reference's "first improving pair at or after the cursor".  K
+    // doubles while nothing is found (long quiet stretches cost few barriers) and resets after a move (tours
+    // far from the optimum improve every few hundred pairs), so the work past the hit is bounded by the gap.
+    constexpr int NW = BATCH_THREADS / 32;
+    const int warp = tid >> 5, lane = tid & 31;
+    int ci = 0, cj = 1;      // cursor (row, column)
+    long long lin_prev = 1;  // statistics: linear index i*n+j of the cursor after the last move / sweep start
+    long long sweep_moves = 0;
+    int K = 1;
+    const float thr = -1.0f + W;
+    // (row, column) of the pair `k` places after the cursor; row >= n-1 means "past the end of the sweep"
+    auto locate = [&](int k, int &row, int &j) {
+        row = ci;
+        long long jj = (long long)cj + k;
+        while (row < n - 1 && jj >= n) {
+            jj -= n;
+            row += 1;
+            jj += row + 1;
+        }
+        j = (int)jj;
+    };
+    for (;;) {
+        int myhit = 0x7fffffff;
+        // this lane's pair of the warp's first chunk; later chunks are 32*NW pairs further along the linear
+        // order, reached by walking (row, column) forward instead of locating from the cursor again
+        int row, j;
+        locate(32 * warp + lane, row, j);
+        for (int q = 0; q < K; ++q) {
+            bool hit = false;
+            const bool valid = row < n - 1;
+            if (valid) {
+                const int si = S.succ[row];
+                long long delta;
+                if (bt_eval<ATT, EXACT32, FP32_OK>(I, S, row, j, S.sx[row], S.sy[row], si, S.sx[si], S.sy[si], S.dsn[row], thr, delta))
+                    hit = delta < 0;
+            }
+            const unsigned m = __ballot_sync(0xffffffffu, hit);
+            if (m) {
+                myhit = 32 * (warp + q * NW) + __ffs(m) - 1;
+                break;
+            }
+            if (!__any_sync(0xffffffffu, valid)) break;  // the whole chunk lies past the end of the sweep
+            long long jj = (long long)j + 32 * NW;
+            while (row < n - 1 && jj >= n) {
+                jj -= n;
+                row += 1;
+                jj += row + 1;
+            }
+            j = (int)jj;
+        }
+        if (lane == 0) s_hits[warp] = myhit;
+        __syncthreads();
+        int first = s_hits[0];
+#pragma unroll
+        for (int w = 1; w < NW; ++w) first = min(first, s_hits[w]);
+        __syncthreads();  // s_hits[] is rewritten by the next step
+        bool sweep_end = false;
+        if (first != 0x7fffffff) {
+            int fi, fj;
+            locate(first, fi, fj);
+            const int si = S.succ[fi], sj = S.succ[fj];
+            const long long fdelta = bt_exact(I, S, ex32, fi, fj) + bt_exact(I, S, ex32, si, sj) - (long long)S.dsn[fi] -
+                                     (long long)S.dsn[fj];
+            evals += (long long)fi * n + fj - lin_prev + 1;  // linear pairs swept, like the grid kernel
+            if (log && tid == 0 && moves < log_cap) {
+                MoveRec mr;
+                mr.i = fi; mr.j = fj; mr.delta = fdelta;
+                log[moves] = mr;
+            }
+            bt_apply(I, S, ex32, n, fi, fj);
+            moves++; sweep_moves++;
+            objd += fdelta;
+            ci = fi; cj = fj + 1;
+            if (cj >= n) { ci = fi + 1; cj = ci + 1; }
+            lin_prev = (long long)ci * n + cj;
+            if (ci >= n - 1) sweep_end = true;
+            K = 1;
+        } else {
+            int nr, nj;
+            locate(32 * NW * K, nr, nj);
+            ci = nr; cj = nj;
+            if (ci >= n - 1) {
+                sweep_end = true;
+                evals += (long long)(n - 1) * n - lin_prev;
+            }
+            if (K < 16) K *= 2;
+        }
+        if (sweep_end) {
+            passes++;
+            if (sweep_moves == 0) break;  // reference heuristics.c:492
+            sweep_moves = 0;
+            ci = 0; cj = 1;
+            lin_prev = 1;
+            K = 1;
+        }
+    }
+}
+
 template <bool ATT, bool EXACT32, bool FP32_OK>
 __global__ void __launch_bounds__(BATCH_THREADS) two_opt_batch_kernel(const InstDev I, int mode, int *succ_all, const int *slots,
                                                                       long long *obj_out, long long *counters, int batch,
@@ -116,32 +259,10 @@ __global__ void __launch_bounds__(BATCH_THREADS) two_opt_batch_kernel(const Inst
 
     for (int b = blockIdx.x; b < batch; b += gridDim.x) {
         int *gsucc = succ_all + (long long)(slots ? slots[b] : b) * n;  // slots: tours of a resident population
-        for (int k = tid; k < n; k += BATCH_THREADS) {
-            float2 p = I.pt32[k];
-            S.sx[k] = p.x; S.sy[k] = p.y;
-            S.succ[k] = gsucc[k];
-        }
-        if (tid == 0) s_err = 0;
-        __syncthreads();
-        if (tid == 0) {  // visiting order from node 0; also validates the cycle
-            int at = 0;
-            for (int p = 0; p < n; ++p) {
-                if (at < 0 || at >= n || (p > 0 && at == 0)) { s_err = 1; break; }
-                S.order[p] = at;
-                S.pos[at] = p;
-                at = S.succ[at];
-            }
-            if (at != 0) s_err = 1;
-        }
-        __syncthreads();
+        bt_load_tour(I, S, gsucc, n, &s_err);
         long long moves = 0, passes = 0, evals = 0, objd = 0;
         if (!s_err && n >= 4) {
-            for (int k = tid; k < n; k += BATCH_THREADS) {
-                const float d = (float)bt_exact(I, S, ex32, k, S.succ[k]);
-                S.dsn[k] = d;
-                S.dsp[S.pos[k]] = d;
-            }
-            __syncthreads();
+            bt_edges(I, S, ex32, n);
             if (mode == 1) {
                 // ---------------- best improvement ----------------
                 for (;;) {
@@ -184,105 +305,7 @@ __global__ void __launch_bounds__(BATCH_THREADS) two_opt_batch_kernel(const Inst
                 evals = passes * ((long long)n * (n - 3) / 2);
             } else {
                 // ---------------- first improvement ----------------
-                // The reference's sweep is a linear scan of the pairs in row-major order from a cursor.  The block scans a
-                // WINDOW of that linear order per step: chunks of 32 consecutive pairs (crossing row ends) are dealt to the
-                // 8 warps round-robin, K chunks per warp, each warp stopping at its first improving pair; the smallest
-                // linear offset over the warps is the reference's "first improving pair at or after the cursor".  K
-                // doubles while nothing is found (long quiet stretches cost few barriers) and resets after a move (tours
-                // far from the optimum improve every few hundred pairs), so the work past the hit is bounded by the gap.
-                constexpr int NW = BATCH_THREADS / 32;
-                const int warp = tid >> 5, lane = tid & 31;
-                int ci = 0, cj = 1;      // cursor (row, column)
-                long long lin_prev = 1;  // statistics: linear index i*n+j of the cursor after the last move / sweep start
-                long long sweep_moves = 0;
-                int K = 1;
-                const float thr = -1.0f + W;
-                // (row, column) of the pair `k` places after the cursor; row >= n-1 means "past the end of the sweep"
-                auto locate = [&](int k, int &row, int &j) {
-                    row = ci;
-                    long long jj = (long long)cj + k;
-                    while (row < n - 1 && jj >= n) {
-                        jj -= n;
-                        row += 1;
-                        jj += row + 1;
-                    }
-                    j = (int)jj;
-                };
-                for (;;) {
-                    int myhit = 0x7fffffff;
-                    // this lane's pair of the warp's first chunk; later chunks are 32*NW pairs further along the linear
-                    // order, reached by walking (row, column) forward instead of locating from the cursor again
-                    int row, j;
-                    locate(32 * warp + lane, row, j);
-                    for (int q = 0; q < K; ++q) {
-                        bool hit = false;
-                        const bool valid = row < n - 1;
-                        if (valid) {
-                            const int si = S.succ[row];
-                            long long delta;
-                            if (bt_eval<ATT, EXACT32, FP32_OK>(I, S, row, j, S.sx[row], S.sy[row], si, S.sx[si], S.sy[si], S.dsn[row], thr, delta))
-                                hit = delta < 0;
-                        }
-                        const unsigned m = __ballot_sync(0xffffffffu, hit);
-                        if (m) {
-                            myhit = 32 * (warp + q * NW) + __ffs(m) - 1;
-                            break;
-                        }
-                        if (!__any_sync(0xffffffffu, valid)) break;  // the whole chunk lies past the end of the sweep
-                        long long jj = (long long)j + 32 * NW;
-                        while (row < n - 1 && jj >= n) {
-                            jj -= n;
-                            row += 1;
-                            jj += row + 1;
-                        }
-                        j = (int)jj;
-                    }
-                    if (lane == 0) s_hits[warp] = myhit;
-                    __syncthreads();
-                    int first = s_hits[0];
-#pragma unroll
-                    for (int w = 1; w < NW; ++w) first = min(first, s_hits[w]);
-                    __syncthreads();  // s_hits[] is rewritten by the next step
-                    bool sweep_end = false;
-                    if (first != 0x7fffffff) {
-                        int fi, fj;
-                        locate(first, fi, fj);
-                        const int si = S.succ[fi], sj = S.succ[fj];
-                        const long long fdelta = bt_exact(I, S, ex32, fi, fj) + bt_exact(I, S, ex32, si, sj) - (long long)S.dsn[fi] -
-                                                 (long long)S.dsn[fj];
-                        evals += (long long)fi * n + fj - lin_prev + 1;  // linear pairs swept, like the grid kernel
-                        if (log && tid == 0 && moves < log_cap) {
-                            MoveRec mr;
-                            mr.i = fi; mr.j = fj; mr.delta = fdelta;
-                            log[moves] = mr;
-                        }
-                        bt_apply(I, S, ex32, n, fi, fj);
-                        moves++; sweep_moves++;
-                        objd += fdelta;
-                        ci = fi; cj = fj + 1;
-                        if (cj >= n) { ci = fi + 1; cj = ci + 1; }
-                        lin_prev = (long long)ci * n + cj;
-                        if (ci >= n - 1) sweep_end = true;
-                        K = 1;
-                    } else {
-                        int nr, nj;
-                        locate(32 * NW * K, nr, nj);
-                        ci = nr; cj = nj;
-                        if (ci >= n - 1) {
-                            sweep_end = true;
-                            evals += (long long)(n - 1) * n - lin_prev;
-                        }
-                        if (K < 16) K *= 2;
-                    }
-                    if (sweep_end) {
-                        passes++;
-                        if (sweep_moves == 0) break;  // reference heuristics.c:492
-                        sweep_moves = 0;
-                        ci = 0; cj = 1;
-                        lin_prev = 1;
-                        K = 1;
-                    }
-                }
+                bt_fi_sweep<ATT, EXACT32, FP32_OK>(I, S, n, W, s_hits, log, log_cap, moves, passes, evals, objd);
             }
         } else if (!s_err) {
             passes = 1;
@@ -347,6 +370,177 @@ cudaError_t launch_two_opt_batch(const InstDev &I, int mode, int *succ, const in
     if (att) return launch_batch_t<true, false, true>(I, mode, succ, slots, obj, counters, batch, num_sms, st, launched, log, log_cap);
     if (ex) return launch_batch_t<false, true, true>(I, mode, succ, slots, obj, counters, batch, num_sms, st, launched, log, log_cap);
     return launch_batch_t<false, false, true>(I, mode, succ, slots, obj, counters, batch, num_sms, st, launched, log, log_cap);
+}
+
+// ---- independent VNS chains (reference HEU_VNS, src/vns.c:103-183), one thread block per chain ------------------------------
+// Per iteration: kick() (vns.c:11-100) on the shared-memory tour, alg_2opt to the local optimum (bt_fi_sweep), keep the result
+// iff its cost is strictly below the incumbent's, else go back to the incumbent.  The incumbent's shared-memory image (succ,
+// dsn, order, pos, dsp: 20 bytes per node, contiguous from S.dsn) lives in a global scratch per RESIDENT block; accepting
+// copies shared -> image, rejecting copies it back.  The slot's successors are written once, at the end of the chain.
+
+// sum over the block of one int64 per thread (s_red: one word per warp); every thread gets the total
+__device__ __forceinline__ long long bt_block_sum(long long v, long long *s_red) {
+    for (int m = 16; m > 0; m >>= 1) v += __shfl_xor_sync(0xffffffffu, v, m);
+    if ((threadIdx.x & 31) == 0) s_red[threadIdx.x >> 5] = v;
+    __syncthreads();
+    long long c = 0;
+#pragma unroll
+    for (int w = 0; w < BATCH_THREADS / 32; ++w) c += s_red[w];
+    __syncthreads();  // s_red[] is rewritten by the next call
+    return c;
+}
+
+// kick() with sorted tour indices i1 < i2 < i3 (i2 - i1 >= 2, i3 - i2 >= 2): tour index t is position (pos[0] + t) mod n.
+// The blocks X = tour[i1+1..i2] and Y = tour[i2+1..i3] trade places by a rotation of order[] (three reversals: X, Y, then
+// the whole range); the inner edges keep their lengths (dsn is node space), only a->d, e->b and c->f are evaluated.  For
+// i3 = n-1, f wraps to tour index 0 (the rule of tspb200_vns_kick).
+__device__ __forceinline__ void bt_kick(const InstDev &I, const BatchSmem &S, bool exact32, int n, int i1, int i2, int i3) {
+    const int tid = threadIdx.x;
+    auto wrap = [n](int p) { return p >= n ? p - n : p; };
+    const int base = S.pos[0];
+    const int pa = wrap(base + i1), sx = wrap(pa + 1), sy = wrap(base + i2 + 1);
+    const int L1 = i2 - i1, L2 = i3 - i2, L = L1 + L2;
+    const int a = S.order[pa], b = S.order[sx], c = S.order[wrap(base + i2)], d = S.order[sy], e = S.order[wrap(base + i3)],
+              f = S.order[wrap(base + i3 + 1)];
+    __syncthreads();  // everybody has read a..f before order[] is rewritten
+    if (tid == 0) {
+        S.dsn[a] = (float)bt_exact(I, S, exact32, a, d);
+        S.dsn[e] = (float)bt_exact(I, S, exact32, e, b);
+        S.dsn[c] = (float)bt_exact(I, S, exact32, c, f);
+    }
+    const int h1 = L1 >> 1, h2 = L2 >> 1;
+    for (int t = tid; t < h1 + h2; t += BATCH_THREADS) {  // reverse X and Y (disjoint ranges)
+        const int s0 = t < h1 ? sx : sy, len = t < h1 ? L1 : L2, u = t < h1 ? t : t - h1;
+        const int A = wrap(s0 + u), B = wrap(s0 + len - 1 - u);
+        const int oa = S.order[A];
+        S.order[A] = S.order[B];
+        S.order[B] = oa;
+    }
+    __syncthreads();
+    for (int t = tid; t < (L >> 1); t += BATCH_THREADS) {  // reverse X'Y' -> Y X
+        const int A = wrap(sx + t), B = wrap(sx + L - 1 - t);
+        const int oa = S.order[A];
+        S.order[A] = S.order[B];
+        S.order[B] = oa;
+    }
+    __syncthreads();
+    for (int t = tid; t <= L; t += BATCH_THREADS) {  // positions of a .. c (new order): successor, position, edge length
+        const int P = wrap(pa + t);
+        const int k = S.order[P];
+        S.pos[k] = P;
+        S.succ[k] = S.order[wrap(P + 1)];
+        S.dsp[P] = S.dsn[k];
+    }
+    __syncthreads();
+}
+
+// the 5n words from S.dsn (dsn, dsp, succ, order, pos) <-> the block's image
+__device__ __forceinline__ void bt_image_copy(unsigned *dst, const unsigned *src, int words) {
+    for (int k = threadIdx.x; k < words; k += BATCH_THREADS) dst[k] = src[k];
+    __syncthreads();
+}
+
+// Blocks per SM that ptxas gives two_opt_batch_kernel (80 registers with the FP32 filter and FP64 points, 64 otherwise): the
+// chain kernel is held to the same occupancy, so that chains run as many at a time as population_two_opt tours.
+template <bool EXACT32, bool FP32_OK>
+constexpr int vns_min_blocks() { return FP32_OK && !EXACT32 ? 3 : 4; }
+
+template <bool ATT, bool EXACT32, bool FP32_OK>
+__global__ void __launch_bounds__(BATCH_THREADS, vns_min_blocks<EXACT32, FP32_OK>()) vns_chains_kernel(const InstDev I, int *succ_all, const int *slots, const int *kicks,
+                                                                   int iters, unsigned *image, long long *best_out,
+                                                                   long long *trace, long long *counters, int count) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ int s_hits[BATCH_THREADS / 32];
+    __shared__ int s_err;
+    __shared__ long long s_red[BATCH_THREADS / 32];
+    __shared__ long long s_best, s_kicked, s_tot[3];
+    const int n = I.n;
+    const int tid = threadIdx.x;
+    BatchSmem S;
+    S.sx = reinterpret_cast<float *>(smem_raw);
+    S.sy = S.sx + n;
+    S.dsn = S.sy + n;
+    S.dsp = S.dsn + n;
+    S.succ = reinterpret_cast<int *>(S.dsp + n);
+    S.order = S.succ + n;
+    S.pos = S.order + n;
+    const bool ex32 = FP32_OK && EXACT32;
+    const float W = I.W;
+    unsigned *img = image + (long long)blockIdx.x * 5 * n;
+    unsigned *sim = reinterpret_cast<unsigned *>(S.dsn);
+
+    for (int b = blockIdx.x; b < count; b += gridDim.x) {
+        int *gsucc = succ_all + (long long)(slots ? slots[b] : b) * n;
+        bt_load_tour(I, S, gsucc, n, &s_err);
+        if (tid == 0) s_tot[0] = s_tot[1] = s_tot[2] = 0;
+        if (!s_err) {
+            bt_edges(I, S, ex32, n);
+            long long cost_part = 0;
+            for (int k = tid; k < n; k += BATCH_THREADS) cost_part += (long long)S.dsn[k];
+            const long long c0 = bt_block_sum(cost_part, s_red);  // reference vns.c:78-86
+            if (tid == 0) s_best = c0;
+            if (iters > 0) bt_image_copy(img, sim, 5 * n);
+            // the chain's state between the steps stays in shared memory (s_best, s_kicked, s_tot): few registers live
+            // across the sweep, so that the kernel runs as many blocks per SM as two_opt_batch_kernel without spilling
+            for (int t = 0; t < iters; ++t) {
+                const int *kk = kicks + 3 * ((long long)b * iters + t);
+                bt_kick(I, S, ex32, n, kk[0], kk[1], kk[2]);
+                cost_part = 0;
+                for (int k = tid; k < n; k += BATCH_THREADS) cost_part += (long long)S.dsn[k];
+                const long long kicked = bt_block_sum(cost_part, s_red);
+                if (tid == 0) s_kicked = kicked;
+                long long moves = 0, passes = 0, evals = 0, objd = 0;
+                bt_fi_sweep<ATT, EXACT32, FP32_OK>(I, S, n, W, s_hits, nullptr, 0, moves, passes, evals, objd);
+                const long long cost = s_kicked + objd;  // reference heuristics.c:486
+                const bool keep = cost < s_best;         // reference vns.c:167-176
+                __syncthreads();                          // everybody has read s_kicked and s_best
+                if (tid == 0) {
+                    if (trace) trace[(long long)b * iters + t] = cost;
+                    if (keep) s_best = cost;
+                    s_tot[0] += moves; s_tot[1] += passes; s_tot[2] += evals;
+                }
+                if (keep) bt_image_copy(img, sim, 5 * n);
+                else bt_image_copy(sim, img, 5 * n);
+            }
+            for (int k = tid; k < n; k += BATCH_THREADS) gsucc[k] = S.succ[k];
+            if (tid == 0) best_out[b] = s_best;
+        }
+        if (tid == 0) {
+            counters[4 * b + 0] = s_tot[0];
+            counters[4 * b + 1] = s_tot[1];
+            counters[4 * b + 2] = s_tot[2];
+            counters[4 * b + 3] = s_err;
+        }
+        __syncthreads();
+    }
+}
+
+template <bool ATT, bool EXACT32, bool FP32_OK>
+static cudaError_t vns_chains_t(const InstDev &I, int count, int num_sms, int *grid, const VnsChainArgs *a, cudaStream_t st) {
+    const size_t smem = (size_t)I.n * 28 + 16;
+    auto kern = vns_chains_kernel<ATT, EXACT32, FP32_OK>;
+    if (smem > 227 * 1024) return cudaErrorInvalidValue;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    int occ = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BATCH_THREADS, smem);
+    if (e != cudaSuccess) return e;
+    if (occ < 1) return cudaErrorInvalidValue;
+    *grid = num_sms * occ < count ? num_sms * occ : count;
+    if (!a) return cudaSuccess;
+    kern<<<*grid, BATCH_THREADS, smem, st>>>(I, a->succ, a->slots, a->kicks, a->iters, a->image, a->best, a->trace, a->counters, count);
+    return cudaGetLastError();
+}
+
+// a == nullptr: only *grid (blocks, hence images of 5 n words, the launch needs); else launch with that grid
+cudaError_t launch_vns_chains(const InstDev &I, int count, int num_sms, int *grid, const VnsChainArgs *a, cudaStream_t st) {
+    const bool att = (I.metric == M_ATT);
+    const bool ex = I.exact32 != 0;
+    if (!I.fp32_ok) return vns_chains_t<false, false, false>(I, count, num_sms, grid, a, st);
+    if (att && ex) return vns_chains_t<true, true, true>(I, count, num_sms, grid, a, st);
+    if (att) return vns_chains_t<true, false, true>(I, count, num_sms, grid, a, st);
+    if (ex) return vns_chains_t<false, true, true>(I, count, num_sms, grid, a, st);
+    return vns_chains_t<false, false, true>(I, count, num_sms, grid, a, st);
 }
 
 }  // namespace tspb

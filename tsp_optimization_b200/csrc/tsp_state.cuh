@@ -76,6 +76,17 @@ struct MoveRec {  // one applied move, as logged for parity tests
     long long delta;
 };
 
+struct VnsChainArgs {  // device buffers of one launch of the VNS chain kernel (kernels_batch.cu)
+    int *succ;             // the resident population
+    const int *slots;      // chain b works on slot slots[b] (b when null)
+    const int *kicks;      // count * iters sorted tour-index triples
+    int iters;
+    unsigned *image;       // grid * 5 n words: the incumbent of every resident block
+    long long *best;       // count incumbent costs
+    long long *trace;      // count * iters costs after each iteration's 2-opt (may be null)
+    long long *counters;   // count * {moves, sweeps, evals, not a cycle}
+};
+
 struct Ctl {
     int done;                       // 1 = local optimum reached (all later launches return at once)
     int error;                      // device-side consistency check failed

@@ -36,6 +36,7 @@ ABI_SYMBOLS = [
     "tspb200_tour_cost", "tspb200_tour_save", "tspb200_tour_restore", "tspb200_vns_kick",
     "tspb200_tabu_begin", "tspb200_tabu_run", "tspb200_tabu_kick", "tspb200_tabu_end",
     "tspb200_population_upload", "tspb200_population_download", "tspb200_population_costs", "tspb200_population_two_opt",
+    "tspb200_population_vns",
 ]
 
 
@@ -137,6 +138,9 @@ def load_library(path: str | None = None) -> C.CDLL:
         L.tspb200_population_download.argtypes = [vp, C.c_void_p, C.c_void_p, C.c_int, C.c_int]
         L.tspb200_population_costs.argtypes = [vp, C.c_void_p, C.c_int, C.c_void_p]
         L.tspb200_population_two_opt.argtypes = [vp, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(_Stats)]
+    if hasattr(L, "tspb200_population_vns"):
+        L.tspb200_population_vns.argtypes = [vp, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                             C.POINTER(_Stats)]
     if hasattr(L, "tspb200_debug_fetch"):
         L.tspb200_debug_fetch.argtypes = [vp, C.c_char_p, C.c_void_p, i64]
     _libs[path] = L
@@ -429,6 +433,22 @@ class Engine:
         st = _Stats()
         self._ck(self.L.tspb200_population_two_opt(self.h, mode, None if sl is None else sl.ctypes.data, k, o.ctypes.data, C.byref(st)))
         return o, Stats.of(st)
+
+    def population_vns(self, kicks, count=None, slots=None, want_trace: bool = True):
+        """Independent VNS chains (reference HEU_VNS, src/vns.c:103-183) on the listed slots (the first `count` when slots is
+        None): kicks[b, t] = chain b's three tour indices of iteration t, shape (chains, iters, 3) (instances.vns_kick_indices).
+        -> (best[chains] incumbent costs, trace[chains, iters] cost after each iteration's 2-opt or None, Stats)."""
+        kicks = np.ascontiguousarray(kicks, dtype=np.int32)
+        sl = None if slots is None else np.ascontiguousarray(slots, dtype=np.int32)
+        k = len(sl) if sl is not None else (int(count) if count is not None else kicks.shape[0])
+        assert kicks.ndim == 3 and kicks.shape[0] == k and kicks.shape[2] == 3, kicks.shape
+        iters = kicks.shape[1]
+        best = np.empty(k, dtype=np.float64)
+        trace = np.empty((k, iters), dtype=np.float64) if want_trace else None
+        st = _Stats()
+        self._ck(self.L.tspb200_population_vns(self.h, None if sl is None else sl.ctypes.data, k, kicks.ctypes.data, iters,
+                                               best.ctypes.data, trace.ctypes.data if want_trace else None, C.byref(st)))
+        return best, trace, Stats.of(st)
 
     # -- multi-GPU
     @staticmethod

@@ -141,6 +141,18 @@ class GlibcRandom:
         return lo + int(self.urand() * (hi - lo))
 
 
+def vns_kick_indices(g: GlibcRandom, n: int):
+    """The three tour indices of one kick() of the reference's VNS, drawn from `g` like src/vns.c:25-31 (the loop of
+    examples/vns_resident.c): idx1, then idx2 until it is neither idx1 nor next to it, then idx3 likewise."""
+    i1 = g.rand_choice(0, n)
+    i2 = i3 = i1
+    while i2 == i1 or abs(i1 - i2) <= 1:
+        i2 = g.rand_choice(0, n)
+    while i3 == i1 or i3 == i2 or abs(i1 - i3) <= 1 or abs(i2 - i3) <= 1:
+        i3 = g.rand_choice(0, n)
+    return i1, i2, i3
+
+
 def reference_random_population(n: int, batch: int, seed: int) -> np.ndarray:
     """`batch` chromosomes generated exactly like reference src/genetic.c:349-364 random_generation(): identity, then n
     random transpositions (idx1, idx2 drawn with rand_choice(0, n) in that order), one generator stream (srandom(seed),
