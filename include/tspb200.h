@@ -220,6 +220,36 @@ int tspb200_population_two_opt(tspb200_ctx *ctx, int mode, const int32_t *slots,
  * (TSPB200_E_UNSUPPORTED); a slot that is not one cycle gives TSPB200_E_DEVICE_CHECK. */
 int tspb200_population_vns(tspb200_ctx *ctx, const int32_t *slots, int count, const int32_t *kicks, int iters, double *best,
                            double *trace, tspb200_stats *st);
+/* Independent tabu searches on the resident population (reference tabu(), src/tabusearch.c:188-320), all chains and
+ * iterations in one launch.  Chain b's state: its current tour in population slot slots[b], its best tour in
+ * best_slots[b], its tabu list (n(n-1)/2 ints, the reference's x_udir_pos layout), its next iteration number and its own
+ * glibc random() stream.  Unlike tspb200_population_vns, the random stream lives on the device: how many pairs a kick
+ * draws depends on the list.
+ * begin: the 2 count slots must be distinct slots of the population; zeroes the lists (CALLOC, tabusearch.c:196), sets
+ * the next iteration number to 1, copies each slot to its best slot and seeds stream b with srandom(seeds[b]).  Needs n to
+ * fit one block's shared memory (28 bytes per node plus one bit), distances < 2^24 and n <= 46340; count * n(n-1)/2 * 4
+ * bytes of lists must fit the device's free memory, else TSPB200_E_UNSUPPORTED naming the bytes, before anything is
+ * allocated.  A begin first ends the previous chain set, so a failed begin leaves none.
+ * tabu: for every chain and t = 0 .. iters-1, with tenure = tenures[b*iters + t] and iter = the chain's next iteration
+ * number: alg_2opt_tabu(list, iter, tenure) to the local optimum (masked best improvement, tabusearch.c:107-178); trace[b*iters
+ * + t] = the recomputed cost; if it is strictly below the best slot's cost the tour is copied there; then the random kick
+ * (:262-309): pairs a = rand_choice(0, n), b = rand_choice(0, n) are drawn until one passes the tests of tspb200_tabu_kick,
+ * which is applied and stamped with iter; draws[b*iters + t] = the pairs drawn; the iteration number then grows by one.  A
+ * kick that would need more than max_draws (>= 1) pairs stops its chain with TSPB200_E_DEVICE_CHECK naming the chain and the
+ * iteration; that chain's state is then unspecified (begin again), the other chains finish normally and the outputs are
+ * filled.  The whole state is kept between calls, so iters = K1 and then K2 (with the matching tenures) equals one call with
+ * K1 + K2; iters = 0 returns the best costs and changes nothing.  best = count doubles (best costs), trace = count*iters
+ * doubles, draws = count*iters ints, each may be NULL; st = moves, passes and evals summed over all chains, gpu_ms, launches.
+ * A slot may be overwritten with tspb200_population_upload(slots = ..): the chain continues from that tour.  No chain set,
+ * a re-created population or a new instance give TSPB200_E_STATE; a slot that is not one cycle TSPB200_E_DEVICE_CHECK.
+ * fetch: chain `chain`'s list (n(n-1)/2 ints, may be NULL) and next iteration number (may be NULL).  There is deliberately
+ * no call that writes a list.  end: frees the chain set (so do tspb200_set_instance with another instance and destroy). */
+int tspb200_population_tabu_begin(tspb200_ctx *ctx, const int32_t *slots, const int32_t *best_slots, int count,
+                                  const uint32_t *seeds);
+int tspb200_population_tabu(tspb200_ctx *ctx, const int32_t *tenures, int iters, int max_draws, double *best,
+                            double *trace, int32_t *draws, tspb200_stats *st);
+int tspb200_population_tabu_fetch(tspb200_ctx *ctx, int chain, int32_t *list_out, int32_t *next_iter);
+int tspb200_population_tabu_end(tspb200_ctx *ctx);
 
 /* ---- multi-GPU (one process per GPU; the caller bootstraps the id, e.g. over torch.distributed) ---- */
 /* Neighbourhood sharding: with a communicator attached, tspb200_bi_run deals the pair tiles round-robin over the ranks;

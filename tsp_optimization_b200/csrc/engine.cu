@@ -75,6 +75,7 @@ cudaError_t launch_two_opt_batch_bi_pos(const InstDev &I, int *succ, const int *
                                         int num_sms, cudaStream_t st, int *launched, MoveRec *log, long long log_cap);
 cudaError_t launch_vns_kick(const InstDev &I, const TourDev &T, int idx1, int idx2, int idx3, float4 *scratch, cudaStream_t st);
 cudaError_t launch_vns_chains(const InstDev &I, int count, int num_sms, int *grid, const VnsChainArgs *a, cudaStream_t st);
+cudaError_t launch_tabu_chains(const InstDev &I, int count, int num_sms, const TabuChainArgs *a, cudaStream_t st);
 cudaError_t launch_tabu_kick_select(const TourDev &T, int *skip, const int *pairs, int count, int iter, int tenure, int *accepted,
                                     cudaStream_t st);
 cudaError_t launch_population_store(const int *staged, int *pop, const int *slots, int n, int count, int as_order, cudaStream_t st);
@@ -215,6 +216,14 @@ struct tspb200_ctx {
     int *d_pop = nullptr;
     long long pop_cap = 0;            // tours the population buffer can hold
     int pop_count = 0, pop_n = 0;
+    long long pop_gen = 0;            // population_upload without slots: a new population
+    // tabu chains on the population (tspb200_population_tabu_begin .. _end)
+    int tc_count = 0;                 // 0 = no chain set
+    long long tc_pop_gen = 0;         // the population they were begun on
+    int *d_tc_lists = nullptr;        // tc_count lists of n(n-1)/2 ints
+    TabuChainState *d_tc_state = nullptr;
+    int *d_tc_slots = nullptr;        // current slots, then best slots
+    std::vector<int> tc_slots;
 
     // comm
     nccl_comm_t comm = nullptr;
@@ -300,8 +309,16 @@ static void free_xchg(tspb200_ctx *c) {
     c->xchg = XchgDev{};
 }
 
+static void free_tabu_chains(tspb200_ctx *c) {
+    cudaFree(c->d_tc_lists); cudaFree(c->d_tc_state); cudaFree(c->d_tc_slots);
+    c->d_tc_lists = nullptr; c->d_tc_state = nullptr; c->d_tc_slots = nullptr;
+    c->tc_count = 0;
+    c->tc_slots.clear();
+}
+
 static void free_instance(tspb200_ctx *c) {
     free_tour(c);
+    free_tabu_chains(c);
     cudaFree(c->d_flush);
     c->d_flush = nullptr;
     c->flush_cap = 0;
@@ -541,6 +558,7 @@ int tspb200_set_instance(tspb200_ctx *ctx, const double *xy, int n, int weight_t
         ctx->has_tour = false;
         ctx->tabu_session = false;  // sessions belong to the instance they were opened on
         ctx->pop_count = 0;
+        free_tabu_chains(ctx);
         ctx->save_n[0] = ctx->save_n[1] = 0;
     }
     ctx->n = n;
@@ -1954,6 +1972,7 @@ int tspb200_population_upload(tspb200_ctx *ctx, const int32_t *tours, const int3
             ctx->pop_n = n;
         }
         ctx->pop_count = count;
+        ctx->pop_gen++;
     } else if (ctx->pop_count < 1 || ctx->pop_n != n) {
         return fail(ctx, TSPB200_E_STATE, "no resident population");
     }
@@ -2131,6 +2150,187 @@ int tspb200_population_vns(tspb200_ctx *ctx, const int32_t *slots, int count, co
     local.path = path;
     local.status = TSPB200_LOCAL_OPTIMUM;
     if (st) *st = local;
+    return TSPB200_OK;
+}
+
+// glibc srandom(seed) followed by the 310 discarded outputs (GlibcRandom in instances.py): the last 31 values of the
+// recurrence, as the chain kernel continues it
+static void glibc_srandom_state(uint32_t seed, TabuChainState &s) {
+    if (seed == 0) seed = 1;
+    uint32_t x[344];
+    x[0] = seed;
+    for (int i = 1; i < 31; ++i) {  // 16807 x mod (2^31 - 1) on the signed value (Schrage), as glibc computes it
+        const int32_t prev = (int32_t)x[i - 1];
+        const int32_t hi = prev / 127773, lo = prev % 127773;
+        int32_t word = 16807 * lo - 2836 * hi;
+        if (word < 0) word += 2147483647;
+        x[i] = (uint32_t)word;
+    }
+    for (int i = 31; i < 34; ++i) x[i] = x[i - 31];
+    for (int i = 34; i < 344; ++i) x[i] = x[i - 31] + x[i - 3];
+    for (int i = 344 - 31; i < 344; ++i) s.rng[i % 31] = x[i];
+    s.rng_pos = 344 % 31;
+}
+
+// Independent tabu searches (reference tabu(), src/tabusearch.c:188-320) on the resident population: begin checks the
+// slots and the memory the lists need, zeroes the lists (CALLOC, tabusearch.c:196), copies every chain's tour to its best
+// slot and seeds the chains' random streams.  A new begin ends the previous chain set first, so that a failed begin leaves
+// no chain set behind (the caller's arrays are sized for the new count).
+int tspb200_population_tabu_begin(tspb200_ctx *ctx, const int32_t *slots, const int32_t *best_slots, int count,
+                                  const uint32_t *seeds) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->stream));
+    free_tabu_chains(ctx);
+    if (ctx->pop_count < 1 || ctx->pop_n != ctx->n) return fail(ctx, TSPB200_E_STATE, "no resident population");
+    if (count < 1 || !slots || !best_slots || !seeds) return fail(ctx, TSPB200_E_ARG, "bad arguments");
+    const int n = ctx->n;
+    if (n > 46340) return fail(ctx, TSPB200_E_UNSUPPORTED, "tabu list index overflows int for n=%d (reference limit)", n);
+    if (!(ctx->dist_bound < 16777216.0)) return fail(ctx, TSPB200_E_UNSUPPORTED, "distances >= 2^24 are not supported by the 2-opt kernels");
+    std::vector<int> all((size_t)2 * count);
+    for (int b = 0; b < count; ++b) { all[(size_t)b] = slots[b]; all[(size_t)count + b] = best_slots[b]; }
+    std::vector<char> used((size_t)ctx->pop_count, 0);
+    for (size_t k = 0; k < all.size(); ++k) {
+        if (all[k] < 0 || all[k] >= ctx->pop_count) return fail(ctx, TSPB200_E_ARG, "population slot %d out of range", all[k]);
+        if (used[(size_t)all[k]]) return fail(ctx, TSPB200_E_ARG, "population slot %d is listed twice (slots and best slots must be 2 count distinct slots)", all[k]);
+        used[(size_t)all[k]] = 1;
+    }
+    int path = select_path(ctx);
+    if (path == 2 && !ctx->d_mat) return fail(ctx, TSPB200_E_STATE, "matrix path selected but no resident matrix");
+    cudaError_t le = launch_tabu_chains(inst_for_path(ctx, path), count, ctx->num_sms, nullptr, ctx->stream);
+    if (le == cudaErrorInvalidValue)
+        return fail(ctx, TSPB200_E_UNSUPPORTED, "tabu chains use the one-block kernel: n=%d does not fit one block's shared memory", n);
+    if (le != cudaSuccess) return fail(ctx, TSPB200_E_CUDA, "tabu chain kernel setup failed: %s", cudaGetErrorString(le));
+    const long long len = (long long)n * (n - 1) / 2;
+    const size_t bytes = sizeof(int) * (size_t)len * (size_t)count;
+    size_t free_b = 0, total_b = 0;
+    CK(cudaMemGetInfo(&free_b, &total_b));
+    if (bytes > free_b)
+        return fail(ctx, TSPB200_E_UNSUPPORTED, "the tabu lists of %d chains need %zu bytes (n(n-1)/2 ints each); the device has %zu bytes free",
+                    count, bytes, free_b);
+    std::vector<TabuChainState> h((size_t)count);
+    memset(h.data(), 0, sizeof(TabuChainState) * (size_t)count);
+    for (int b = 0; b < count; ++b) {
+        glibc_srandom_state(seeds[b], h[(size_t)b]);
+        h[(size_t)b].next_iter = 1;
+    }
+    if (cudaMalloc(&ctx->d_tc_lists, bytes > 0 ? bytes : 4) != cudaSuccess ||
+        cudaMalloc(&ctx->d_tc_state, sizeof(TabuChainState) * (size_t)count) != cudaSuccess ||
+        cudaMalloc(&ctx->d_tc_slots, sizeof(int) * all.size()) != cudaSuccess) {
+        const cudaError_t e = cudaGetLastError();
+        free_tabu_chains(ctx);
+        return fail(ctx, TSPB200_E_CUDA, "cannot allocate the tabu chains (%zu bytes of lists): %s", bytes, cudaGetErrorString(e));
+    }
+    CK(cudaMemsetAsync(ctx->d_tc_lists, 0, bytes, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_tc_state, h.data(), sizeof(TabuChainState) * (size_t)count, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_tc_slots, all.data(), sizeof(int) * all.size(), cudaMemcpyHostToDevice, ctx->stream));
+    for (int b = 0; b < count; ++b)
+        CK(cudaMemcpyAsync(ctx->d_pop + (size_t)best_slots[b] * n, ctx->d_pop + (size_t)slots[b] * n, sizeof(int) * (size_t)n,
+                           cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));  // `all` and `h` are pageable host memory
+    ctx->tc_count = count;
+    ctx->tc_pop_gen = ctx->pop_gen;
+    ctx->tc_slots = all;
+    return TSPB200_OK;
+}
+
+static int tabu_chains_ready(tspb200_ctx *ctx) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (ctx->tc_count < 1) return fail(ctx, TSPB200_E_STATE, "no tabu chain set (tspb200_population_tabu_begin)");
+    if (ctx->pop_gen != ctx->tc_pop_gen || ctx->pop_count < 1 || ctx->pop_n != ctx->n)
+        return fail(ctx, TSPB200_E_STATE, "the population was re-created since tspb200_population_tabu_begin");
+    return TSPB200_OK;
+}
+
+// iters iterations of every chain in one launch (see include/tspb200.h)
+int tspb200_population_tabu(tspb200_ctx *ctx, const int32_t *tenures, int iters, int max_draws, double *best, double *trace,
+                            int32_t *draws, tspb200_stats *st) {
+    int rc = tabu_chains_ready(ctx);
+    if (rc) return rc;
+    if (iters < 0 || (iters > 0 && !tenures) || max_draws < 1) return fail(ctx, TSPB200_E_ARG, "bad arguments (iters >= 0, tenures, max_draws >= 1)");
+    CK(cudaSetDevice(ctx->device));
+    const int n = ctx->n, count = ctx->tc_count;
+    const int path = select_path(ctx);
+    if (path == 2 && !ctx->d_mat) return fail(ctx, TSPB200_E_STATE, "matrix path selected but no resident matrix");
+    InstDev I = inst_for_path(ctx, path);
+    const size_t nk = (size_t)count * (size_t)iters;
+    SCRATCH(d_best, long long *, 1, sizeof(long long) * (size_t)count);
+    SCRATCH(d_cnt, long long *, 2, sizeof(long long) * 4 * (size_t)count);
+    SCRATCH(d_ten, int *, 3, sizeof(int) * nk);
+    long long *d_trace = nullptr;
+    int *d_draws = nullptr;
+    if (trace && nk) {
+        SCRATCH(d_t, long long *, 14, sizeof(long long) * nk);
+        d_trace = d_t;
+    }
+    if (draws && nk) {
+        SCRATCH(d_d, int *, 4, sizeof(int) * nk);
+        d_draws = d_d;
+    }
+    CK(cudaEventRecord(ctx->ev0, ctx->stream));
+    if (nk) CK(cudaMemcpyAsync(d_ten, tenures, sizeof(int) * nk, cudaMemcpyHostToDevice, ctx->stream));
+    TabuChainArgs a{ctx->d_pop, ctx->d_tc_slots, ctx->d_tc_lists, (long long)n * (n - 1) / 2, ctx->d_tc_state, d_ten, iters, max_draws,
+                    d_best, d_trace, d_draws, d_cnt};
+    const cudaError_t le = launch_tabu_chains(I, count, ctx->num_sms, &a, ctx->stream);
+    if (le != cudaSuccess) return fail(ctx, TSPB200_E_CUDA, "tabu chain launch failed: %s", cudaGetErrorString(le));
+    std::vector<long long> h_best((size_t)count), h_cnt((size_t)count * 4), h_trace(d_trace ? nk : 0);
+    std::vector<int> h_draws(d_draws ? nk : 0);
+    CK(cudaMemcpyAsync(h_best.data(), d_best, sizeof(long long) * (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(h_cnt.data(), d_cnt, sizeof(long long) * 4 * (size_t)count, cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_trace) CK(cudaMemcpyAsync(h_trace.data(), d_trace, sizeof(long long) * nk, cudaMemcpyDeviceToHost, ctx->stream));
+    if (d_draws) CK(cudaMemcpyAsync(h_draws.data(), d_draws, sizeof(int) * nk, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaEventRecord(ctx->ev1, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    tspb200_stats local;
+    memset(&local, 0, sizeof local);
+    int bad = -1;
+    for (int b = 0; b < count; ++b) {
+        if (h_cnt[4 * (size_t)b + 3] && bad < 0) bad = b;
+        local.moves += h_cnt[4 * (size_t)b + 0];
+        local.passes += h_cnt[4 * (size_t)b + 1];
+        local.evals += h_cnt[4 * (size_t)b + 2];
+        if (best) best[b] = (double)h_best[(size_t)b];
+    }
+    for (size_t q = 0; q < h_trace.size(); ++q) trace[q] = (double)h_trace[q];
+    for (size_t q = 0; q < h_draws.size(); ++q) draws[q] = h_draws[q];
+    float ms = 0;
+    CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+    local.gpu_ms = ms;
+    local.launches = 1;
+    local.path = path;
+    local.status = TSPB200_LOCAL_OPTIMUM;
+    if (st) *st = local;
+    if (bad >= 0) {
+        const long long e = h_cnt[4 * (size_t)bad + 3];
+        if (e == 1)
+            return fail(ctx, TSPB200_E_DEVICE_CHECK, "chain %d: population slot %d or %d does not hold a single cycle", bad,
+                        ctx->tc_slots[(size_t)bad], ctx->tc_slots[(size_t)count + bad]);
+        return fail(ctx, TSPB200_E_DEVICE_CHECK, "chain %d, iteration %lld: the kick drew max_draws = %d pairs and none passed; the chain's state "
+                    "is unspecified (begin again)", bad, e - 2, max_draws);
+    }
+    return TSPB200_OK;
+}
+
+int tspb200_population_tabu_fetch(tspb200_ctx *ctx, int chain, int32_t *list_out, int32_t *next_iter) {
+    int rc = tabu_chains_ready(ctx);
+    if (rc) return rc;
+    if (chain < 0 || chain >= ctx->tc_count) return fail(ctx, TSPB200_E_ARG, "chain %d out of range", chain);
+    CK(cudaSetDevice(ctx->device));
+    const long long len = (long long)ctx->n * (ctx->n - 1) / 2;
+    if (list_out && len)
+        CK(cudaMemcpyAsync(list_out, ctx->d_tc_lists + (size_t)chain * (size_t)len, sizeof(int) * (size_t)len, cudaMemcpyDeviceToHost, ctx->stream));
+    if (next_iter)
+        CK(cudaMemcpyAsync(next_iter, &ctx->d_tc_state[chain].next_iter, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return TSPB200_OK;
+}
+
+int tspb200_population_tabu_end(tspb200_ctx *ctx) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (ctx->tc_count < 1) return fail(ctx, TSPB200_E_STATE, "no tabu chain set");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->stream));
+    free_tabu_chains(ctx);
     return TSPB200_OK;
 }
 

@@ -38,12 +38,57 @@ __device__ __forceinline__ long long bt_exact(const InstDev &I, const BatchSmem 
     return exact_dist(I.metric, I.pt64[u], I.pt64[v]);
 }
 
-// exact delta of pair (i,j) or "skip" (adjacent) -> returns false
-template <bool ATT, bool EXACT32, bool FP32_OK>
+// The tabu list of one chain of tabu_chains_kernel (reference src/tabusearch.c:137-149), seen by the masked pass.  Only
+// kicks write non-zero entries and lazy expiry only zeroes them, so few entries are non-zero; marks[] (shared memory, one
+// bit per node) has both ends of every entry that may be non-zero set.  An entry with an unmarked end is zero: its
+// check_tenure returns "not tabu" and writes nothing, so it is not read.
+struct TabuMask {
+    int *list;              // n(n-1)/2 ints, x_udir_pos layout (reference src/utility.c:17-30)
+    const unsigned *marks;  // shared memory, (n + 31) / 32 words
+    int n, iter, tenure;
+};
+
+__device__ __forceinline__ bool tm_marked(const unsigned *marks, int x) { return (marks[x >> 5] >> (x & 31)) & 1u; }
+
+__device__ __forceinline__ int tm_index(int x, int y, int n) {  // x_udir_pos; n fits one block, so int is enough
+    if (x > y) { const int t = x; x = y; y = t; }
+    return x * n + y - ((x + 1) * (x + 2)) / 2;
+}
+
+// reference src/tabusearch.c:83-92 check_tenure on entry (x, y), with its lazy expiry.  iter and tenure are fixed during a
+// pass, so whether another thread of the block has already zeroed an expired entry does not change the verdict: the set of
+// zeroed entries is the union over the tested pairs, whatever the order in which the threads test them.
+__device__ __forceinline__ bool tm_check(const TabuMask &M, int x, int y) {
+    int *p = M.list + tm_index(x, y, M.n);
+    const int v = *p;
+    if (v == 0) return false;
+    if (M.iter - v > M.tenure) {
+        *p = 0;
+        return false;
+    }
+    return true;
+}
+
+// the four tests of alg_2opt_tabu for the pair a = i < b = j, in the reference's '||' order (tabusearch.c:137-149; the fourth
+// entry is (a, b1)); rowm = marks of a (bit 0) and a1 (bit 1), the same for the whole row
+__device__ __forceinline__ bool tm_tabu(const TabuMask &M, unsigned rowm, int a, int b, int a1, int b1) {
+    const bool ma = rowm & 1u, mb = tm_marked(M.marks, b);
+    if (!ma && !mb) return false;
+    if (ma && mb && tm_check(M, a, b)) return true;
+    if (ma && (rowm & 2u) && tm_check(M, a, a1)) return true;
+    if (mb && tm_marked(M.marks, b1) && tm_check(M, b, b1)) return true;
+    return ma && tm_marked(M.marks, b1) && tm_check(M, a, b1);
+}
+
+// exact delta of pair (i,j) or "skip" (adjacent; with MASK also tabu) -> returns false.  The tabu tests come after the
+// adjacency test and before, independently of, the FP32 filter: their lazy expiry is a side effect of every tested pair.
+template <bool ATT, bool EXACT32, bool FP32_OK, bool MASK = false>
 __device__ __forceinline__ bool bt_eval(const InstDev &I, const BatchSmem &S, int i, int j, float xi, float yi, int si,
-                                        float xsi, float ysi, float dsi, float thr, long long &delta) {
+                                        float xsi, float ysi, float dsi, float thr, long long &delta,
+                                        const TabuMask *M = nullptr, unsigned rowm = 0) {
     const int sj = S.succ[j];
     if (sj == i || si == j || si == sj) return false;  // reference heuristics.c:471 / tabusearch.c:134
+    if (MASK && tm_tabu(*M, rowm, i, j, si, sj)) return false;
     const float dsj = S.dsn[j];
     if (FP32_OK) {
         float q = bt_dist32<ATT>(xi, yi, S.sx[j], S.sy[j]) + bt_dist32<ATT>(xsi, ysi, S.sx[sj], S.sy[sj]) - dsi - dsj;
@@ -236,6 +281,41 @@ __device__ __forceinline__ void bt_fi_sweep(const InstDev &I, const BatchSmem &S
     }
 }
 
+// One best-improvement pass over the shared-memory tour (reference src/tabusearch.c:126-156: strict '<' argmin == lowest
+// (i, j) among equal deltas); with MASK the pairs that alg_2opt_tabu's list forbids are skipped.  Returns the block's
+// winner (delta >= 0: none), identically in every thread.
+template <bool ATT, bool EXACT32, bool FP32_OK, bool MASK>
+__device__ __forceinline__ MoveKey bt_bi_pass(const InstDev &I, const BatchSmem &S, int n, float W, MoveKey *s_keys,
+                                              const TabuMask *M) {
+    MoveKey best = key_none();
+    float thr = W;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int i = warp; i < n - 1; i += BATCH_THREADS / 32) {
+        const float xi = S.sx[i], yi = S.sy[i], dsi = S.dsn[i];
+        const int si = S.succ[i];
+        const float xsi = S.sx[si], ysi = S.sy[si];
+        const unsigned rowm = MASK ? (tm_marked(M->marks, i) ? 1u : 0u) | (tm_marked(M->marks, si) ? 2u : 0u) : 0u;
+        for (int j = i + 1 + lane; j < n; j += 32) {
+            long long delta;
+            if (!bt_eval<ATT, EXACT32, FP32_OK, MASK>(I, S, i, j, xi, yi, si, xsi, ysi, dsi, thr, delta, M, rowm)) continue;
+            if (delta < 0 && delta <= (long long)best.delta) {
+                MoveKey k;
+                k.delta = (int)delta; k.i = i; k.j = j; k.pad = 0;
+                if (key_less(k, best)) { best = k; thr = (float)k.delta + W; }
+            }
+        }
+    }
+    best = key_warp_min(best);
+    if (lane == 0) s_keys[warp] = best;
+    __syncthreads();
+    best = s_keys[0];
+#pragma unroll
+    for (int w = 1; w < BATCH_THREADS / 32; ++w)
+        if (key_less(s_keys[w], best)) best = s_keys[w];
+    __syncthreads();
+    return best;
+}
+
 template <bool ATT, bool EXACT32, bool FP32_OK>
 __global__ void __launch_bounds__(BATCH_THREADS) two_opt_batch_kernel(const InstDev I, int mode, int *succ_all, const int *slots,
                                                                       long long *obj_out, long long *counters, int batch,
@@ -266,31 +346,7 @@ __global__ void __launch_bounds__(BATCH_THREADS) two_opt_batch_kernel(const Inst
             if (mode == 1) {
                 // ---------------- best improvement ----------------
                 for (;;) {
-                    MoveKey best = key_none();
-                    float thr = W;
-                    const int warp = tid >> 5, lane = tid & 31;
-                    for (int i = warp; i < n - 1; i += BATCH_THREADS / 32) {
-                        const float xi = S.sx[i], yi = S.sy[i], dsi = S.dsn[i];
-                        const int si = S.succ[i];
-                        const float xsi = S.sx[si], ysi = S.sy[si];
-                        for (int j = i + 1 + lane; j < n; j += 32) {
-                            long long delta;
-                            if (!bt_eval<ATT, EXACT32, FP32_OK>(I, S, i, j, xi, yi, si, xsi, ysi, dsi, thr, delta)) continue;
-                            if (delta < 0 && delta <= (long long)best.delta) {
-                                MoveKey k;
-                                k.delta = (int)delta; k.i = i; k.j = j; k.pad = 0;
-                                if (key_less(k, best)) { best = k; thr = (float)k.delta + W; }
-                            }
-                        }
-                    }
-                    best = key_warp_min(best);
-                    if (lane == 0) s_keys[warp] = best;
-                    __syncthreads();
-                    best = s_keys[0];
-#pragma unroll
-                    for (int w = 1; w < BATCH_THREADS / 32; ++w)
-                        if (key_less(s_keys[w], best)) best = s_keys[w];
-                    __syncthreads();
+                    const MoveKey best = bt_bi_pass<ATT, EXACT32, FP32_OK, false>(I, S, n, W, s_keys, nullptr);
                     passes++;
                     if (best.delta >= 0) break;
                     if (log && tid == 0 && moves < log_cap) {
@@ -541,6 +597,239 @@ cudaError_t launch_vns_chains(const InstDev &I, int count, int num_sms, int *gri
     if (att) return vns_chains_t<true, false, true>(I, count, num_sms, grid, a, st);
     if (ex) return vns_chains_t<false, true, true>(I, count, num_sms, grid, a, st);
     return vns_chains_t<false, false, true>(I, count, num_sms, grid, a, st);
+}
+
+// ---- independent tabu chains (reference tabu(), src/tabusearch.c:188-320), one thread block per chain -----------------------
+// Per iteration: alg_2opt_tabu (masked best improvement to the local optimum, bt_bi_pass<MASK>), the cost recomputed, the best
+// tour kept in its own slot when strictly better, then the random kick: pairs (a, b) drawn with rand_choice(0, n) from the
+// chain's own glibc random() stream until one passes the adjacency and check_tenure tests (:262-309).  The draws depend on
+// the list, which lives on the device, so the stream does too.
+//
+// The list is read sparsely.  Only kicks write non-zero entries (two per iteration) and expiry only zeroes them, so the
+// chain's table (TabuChainState::tab, in shared memory during the launch) lists a superset of the non-zero entries: every
+// kick adds its two stamped entries, and before each masked pass the table drops the entries that read zero.  marks[] has
+// both ends of every listed entry set, and the masked pass reads the list only for entries with both ends marked
+// (tm_tabu).  A table that overflows is rebuilt from the whole list before each masked pass until it fits again; meanwhile
+// every node is marked (every entry is read).  Passes at tenure < 0 are unmasked and need neither the table nor the marks.
+
+// glibc random() on a chain's state (x_k = x_{k-31} + x_{k-3}, output x_k >> 1), then rand_choice(0, n) (reference
+// src/utility.c:752-754: URAND() = random() / RAND_MAX in FP64, scaled by n and truncated), as GlibcRandom.rand_choice
+__device__ __forceinline__ int tc_rand_choice(TabuChainState &st, int n) {
+    const int k = st.rng_pos;
+    const unsigned v = st.rng[k] + st.rng[k >= 3 ? k - 3 : k + 28];
+    st.rng[k] = v;
+    st.rng_pos = k == 30 ? 0 : k + 1;
+    return (int)(__ddiv_rn((double)(v >> 1), 2147483647.0) * (double)n);
+}
+
+// check_tenure (src/tabusearch.c:83-92) on the dense list, as the kick tests it
+__device__ __forceinline__ bool tc_check(int *list, int e, int iter, int tenure) {
+    if (iter < 0 || tenure < 0) return false;
+    const int v = list[e];
+    if (v == 0) return false;
+    if (iter - v > tenure) {
+        list[e] = 0;
+        return false;
+    }
+    return true;
+}
+
+// the kick stamped entry (x, y): one thread adds it to the table unless it is listed already (-1 when the table is full)
+__device__ __forceinline__ void tc_add(TabuChainState &st, int x, int y) {
+    if (st.tab_n < 0) return;
+    const unsigned e = (unsigned)min(x, y) << 16 | (unsigned)max(x, y);
+    for (int k = 0; k < st.tab_n; ++k)
+        if (st.tab[k] == e) return;
+    if (st.tab_n == TABU_TAB) st.tab_n = -1;
+    else st.tab[st.tab_n++] = e;
+}
+
+// Before a masked pass: drops the entries that read zero from the table, or rebuilds it from the list when it has
+// overflowed, then sets marks[].  Block-wide.
+__device__ __noinline__ void tc_refresh(TabuChainState &st, const int *list, int n, unsigned *marks, int *s_cnt) {
+    const int tid = threadIdx.x;
+    if (st.tab_n >= 0) {
+        const unsigned v = tid < st.tab_n ? st.tab[tid] : 0u;
+        const bool keep = tid < st.tab_n && list[tm_index(v >> 16, v & 0xffff, n)] != 0;
+        if (tid == 0) s_cnt[0] = 0;
+        __syncthreads();
+        if (keep) st.tab[atomicAdd(&s_cnt[0], 1)] = v;
+        __syncthreads();
+        if (tid == 0) st.tab_n = s_cnt[0];
+        __syncthreads();
+    }
+    if (st.tab_n < 0) {
+        if (tid == 0) s_cnt[0] = 0;
+        __syncthreads();
+        const int warp = tid >> 5, lane = tid & 31;
+        for (int x = warp; x < n - 1; x += BATCH_THREADS / 32) {
+            const int *row = list + tm_index(x, x + 1, n) - (x + 1);  // row[y] = entry (x, y)
+            for (int y = x + 1 + lane; y < n; y += 32)
+                if (row[y] != 0) {
+                    const int k = atomicAdd(&s_cnt[0], 1);
+                    if (k < TABU_TAB) st.tab[k] = (unsigned)x << 16 | (unsigned)y;
+                }
+        }
+        __syncthreads();
+        if (tid == 0) st.tab_n = s_cnt[0] <= TABU_TAB ? s_cnt[0] : -1;
+        __syncthreads();
+    }
+    const unsigned fill = st.tab_n < 0 ? ~0u : 0u;
+    for (int k = tid; k < (n + 31) >> 5; k += BATCH_THREADS) marks[k] = fill;
+    __syncthreads();
+    if (tid < st.tab_n) {
+        const unsigned v = st.tab[tid], x = v >> 16, y = v & 0xffff;
+        atomicOr(&marks[x >> 5], 1u << (x & 31));
+        atomicOr(&marks[y >> 5], 1u << (y & 31));
+    }
+    __syncthreads();
+}
+
+template <bool ATT, bool EXACT32, bool FP32_OK>
+__global__ void __launch_bounds__(BATCH_THREADS, vns_min_blocks<EXACT32, FP32_OK>()) tabu_chains_kernel(const InstDev I, const TabuChainArgs A,
+                                                                                                         int count) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    __shared__ int s_err;
+    __shared__ MoveKey s_keys[BATCH_THREADS / 32];
+    __shared__ long long s_red[BATCH_THREADS / 32];
+    __shared__ long long s_best, s_tot[2];
+    __shared__ int s_kick[3];  // a, b, pairs drawn (0: max_draws reached)
+    __shared__ int s_cnt;
+    __shared__ TabuChainState s_st;
+    const int n = I.n;
+    const int tid = threadIdx.x;
+    BatchSmem S;
+    S.sx = reinterpret_cast<float *>(smem_raw);
+    S.sy = S.sx + n;
+    S.dsn = S.sy + n;
+    S.dsp = S.dsn + n;
+    S.succ = reinterpret_cast<int *>(S.dsp + n);
+    S.order = S.succ + n;
+    S.pos = S.order + n;
+    unsigned *marks = reinterpret_cast<unsigned *>(S.pos + n);
+    const bool ex32 = FP32_OK && EXACT32;
+    const float W = I.W;
+
+    for (int b = blockIdx.x; b < count; b += gridDim.x) {
+        int *gsucc = A.succ + (long long)A.slots[b] * n;
+        int *gbest = A.succ + (long long)A.slots[count + b] * n;
+        int *list = A.lists + (long long)b * A.list_len;
+        // the best tour's cost (the slot may have been overwritten since the last call)
+        bt_load_tour(I, S, gbest, n, &s_err);
+        const bool bad_best = s_err != 0;
+        long long part = 0;
+        if (!bad_best)
+            for (int k = tid; k < n; k += BATCH_THREADS) part += bt_exact(I, S, ex32, k, S.succ[k]);
+        const long long c_best = bt_block_sum(part, s_red);
+        bt_load_tour(I, S, gsucc, n, &s_err);
+        long long err = bad_best || s_err ? 1 : 0;
+        if (tid == 0) { s_best = c_best; s_tot[0] = s_tot[1] = 0; }
+        if (!err) {
+            bt_edges(I, S, ex32, n);
+            const unsigned *gs = reinterpret_cast<const unsigned *>(A.state + b);
+            for (int k = tid; k < (int)(sizeof(TabuChainState) / 4); k += BATCH_THREADS) reinterpret_cast<unsigned *>(&s_st)[k] = gs[k];
+            __syncthreads();
+            for (int t = 0; t < A.iters; ++t) {
+                const long long q = (long long)b * A.iters + t;
+                const int tenure = A.tenures[q], iter = s_st.next_iter;
+                const bool masked = iter >= 0 && tenure >= 0;  // else check_tenure never blocks nor expires
+                if (masked) tc_refresh(s_st, list, n, marks, &s_cnt);
+                const TabuMask M{list, marks, n, iter, tenure};
+                long long moves = 0, passes = 0;
+                for (;;) {  // alg_2opt_tabu (tabusearch.c:123-166)
+                    const MoveKey k = masked ? bt_bi_pass<ATT, EXACT32, FP32_OK, true>(I, S, n, W, s_keys, &M)
+                                             : bt_bi_pass<ATT, EXACT32, FP32_OK, false>(I, S, n, W, s_keys, nullptr);
+                    passes++;
+                    if (k.delta >= 0) break;
+                    bt_apply(I, S, ex32, n, k.i, k.j);
+                    moves++;
+                }
+                part = 0;
+                for (int k = tid; k < n; k += BATCH_THREADS) part += (long long)S.dsn[k];
+                const long long cost = bt_block_sum(part, s_red);  // tabusearch.c:168-172
+                const bool better = cost < s_best;                 // tabusearch.c:241-243
+                __syncthreads();                                   // everybody has read s_best
+                if (better)
+                    for (int k = tid; k < n; k += BATCH_THREADS) gbest[k] = S.succ[k];
+                if (tid == 0) {
+                    if (A.trace) A.trace[q] = cost;
+                    if (better) s_best = cost;
+                    s_tot[0] += moves; s_tot[1] += passes;
+                    // the kick (tabusearch.c:262-309): draw until a pair passes, at most max_draws pairs
+                    s_kick[2] = 0;
+                    for (int d = 1; d <= A.max_draws; ++d) {
+                        const int a = tc_rand_choice(s_st, n), bb = tc_rand_choice(s_st, n);
+                        const int a1 = S.succ[a], b1 = S.succ[bb];
+                        if (a == bb || a1 == bb || b1 == a) continue;
+                        const int e1 = tm_index(a, a1, n), e2 = tm_index(bb, b1, n);
+                        if (!tc_check(list, e1, iter, tenure) && !tc_check(list, e2, iter, tenure) &&
+                            !tc_check(list, tm_index(a, bb, n), iter, tenure) && !tc_check(list, tm_index(a1, b1, n), iter, tenure)) {
+                            list[e1] = iter;
+                            list[e2] = iter;
+                            tc_add(s_st, a, a1);
+                            tc_add(s_st, bb, b1);
+                            s_kick[0] = a; s_kick[1] = bb; s_kick[2] = d;
+                            break;
+                        }
+                    }
+                    if (A.draws) A.draws[q] = s_kick[2];
+                }
+                __syncthreads();
+                if (s_kick[2] == 0) {  // the reference would keep drawing
+                    err = 2 + t;
+                    break;
+                }
+                bt_apply(I, S, ex32, n, s_kick[0], s_kick[1]);
+                if (tid == 0) s_st.next_iter = iter + 1;
+                __syncthreads();
+            }
+            for (int k = tid; k < n; k += BATCH_THREADS) gsucc[k] = S.succ[k];
+            unsigned *gw = reinterpret_cast<unsigned *>(A.state + b);
+            for (int k = tid; k < (int)(sizeof(TabuChainState) / 4); k += BATCH_THREADS) gw[k] = reinterpret_cast<const unsigned *>(&s_st)[k];
+        }
+        if (tid == 0) {
+            A.best[b] = s_best;
+            A.counters[4 * b + 0] = s_tot[0];
+            A.counters[4 * b + 1] = s_tot[1];
+            A.counters[4 * b + 2] = s_tot[1] * ((long long)n * (n - 3) / 2);
+            A.counters[4 * b + 3] = err;
+        }
+        __syncthreads();
+    }
+}
+
+// dynamic shared memory of the tabu chain kernel: the 28-byte-per-node tour image and the marks
+static size_t tabu_chains_smem(int n) { return (size_t)n * 28 + (size_t)4 * ((n + 31) / 32) + 16; }
+
+template <bool ATT, bool EXACT32, bool FP32_OK>
+static cudaError_t tabu_chains_t(const InstDev &I, int count, int num_sms, const TabuChainArgs *a, cudaStream_t st) {
+    const size_t smem = tabu_chains_smem(I.n);
+    auto kern = tabu_chains_kernel<ATT, EXACT32, FP32_OK>;
+    cudaFuncAttributes fa;
+    cudaError_t e = cudaFuncGetAttributes(&fa, kern);
+    if (e != cudaSuccess) return e;
+    if (smem + fa.sharedSizeBytes > 227 * 1024) return cudaErrorInvalidValue;
+    e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return e;
+    int occ = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, BATCH_THREADS, smem);
+    if (e != cudaSuccess) return e;
+    if (occ < 1) return cudaErrorInvalidValue;
+    if (!a) return cudaSuccess;
+    const int grid = num_sms * occ < count ? num_sms * occ : count;
+    kern<<<grid, BATCH_THREADS, smem, st>>>(I, *a, count);
+    return cudaGetLastError();
+}
+
+// a == nullptr: only checks that n fits one block (cudaErrorInvalidValue when not); else launch
+cudaError_t launch_tabu_chains(const InstDev &I, int count, int num_sms, const TabuChainArgs *a, cudaStream_t st) {
+    const bool att = (I.metric == M_ATT);
+    const bool ex = I.exact32 != 0;
+    if (!I.fp32_ok) return tabu_chains_t<false, false, false>(I, count, num_sms, a, st);
+    if (att && ex) return tabu_chains_t<true, true, true>(I, count, num_sms, a, st);
+    if (att) return tabu_chains_t<true, false, true>(I, count, num_sms, a, st);
+    if (ex) return tabu_chains_t<false, true, true>(I, count, num_sms, a, st);
+    return tabu_chains_t<false, false, true>(I, count, num_sms, a, st);
 }
 
 }  // namespace tspb

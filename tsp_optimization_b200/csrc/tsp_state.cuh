@@ -87,6 +87,31 @@ struct VnsChainArgs {  // device buffers of one launch of the VNS chain kernel (
     long long *counters;   // count * {moves, sweeps, evals, not a cycle}
 };
 
+constexpr int TABU_TAB = 256;  // entries of a tabu chain's table of possibly non-zero list entries (one per thread)
+
+struct TabuChainState {  // what a tabu chain keeps between calls besides its two tours and its list (kernels_batch.cu)
+    unsigned rng[31];    // glibc random() (TYPE_3): the last 31 outputs of the recurrence, x_k in rng[k mod 31]
+    int rng_pos;         // k mod 31 of the next x_k
+    int next_iter;       // the reference's `iter` of the next iteration
+    int tab_n;           // entries in tab[]; -1 = too many to list: the table is rebuilt from the list
+    int pad[2];
+    unsigned tab[TABU_TAB];  // x << 16 | y (x < y): a superset of the list's non-zero entries
+};
+
+struct TabuChainArgs {   // device buffers of one launch of the tabu chain kernel (kernels_batch.cu)
+    int *succ;             // the resident population
+    const int *slots;      // 2 count: chain b's current tour in slot slots[b], its best tour in slots[count + b]
+    int *lists;            // count lists of list_len ints
+    long long list_len;    // n(n-1)/2
+    TabuChainState *state; // count states
+    const int *tenures;    // count * iters
+    int iters, max_draws;
+    long long *best;       // count best costs
+    long long *trace;      // count * iters costs after each iteration's masked 2-opt (may be null)
+    int *draws;            // count * iters pairs drawn by each kick (may be null)
+    long long *counters;   // count * {moves, passes, evals, error: 1 = not a cycle, 2 + t = kick t drew max_draws pairs}
+};
+
 struct Ctl {
     int done;                       // 1 = local optimum reached (all later launches return at once)
     int error;                      // device-side consistency check failed

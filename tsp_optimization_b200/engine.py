@@ -36,7 +36,8 @@ ABI_SYMBOLS = [
     "tspb200_tour_cost", "tspb200_tour_save", "tspb200_tour_restore", "tspb200_vns_kick",
     "tspb200_tabu_begin", "tspb200_tabu_run", "tspb200_tabu_kick", "tspb200_tabu_end",
     "tspb200_population_upload", "tspb200_population_download", "tspb200_population_costs", "tspb200_population_two_opt",
-    "tspb200_population_vns",
+    "tspb200_population_vns", "tspb200_population_tabu_begin", "tspb200_population_tabu", "tspb200_population_tabu_fetch",
+    "tspb200_population_tabu_end",
 ]
 
 
@@ -141,6 +142,12 @@ def load_library(path: str | None = None) -> C.CDLL:
     if hasattr(L, "tspb200_population_vns"):
         L.tspb200_population_vns.argtypes = [vp, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                              C.POINTER(_Stats)]
+    if hasattr(L, "tspb200_population_tabu"):
+        L.tspb200_population_tabu_begin.argtypes = [vp, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]
+        L.tspb200_population_tabu.argtypes = [vp, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                              C.POINTER(_Stats)]
+        L.tspb200_population_tabu_fetch.argtypes = [vp, C.c_int, C.c_void_p, C.POINTER(C.c_int32)]
+        L.tspb200_population_tabu_end.argtypes = [vp]
     if hasattr(L, "tspb200_debug_fetch"):
         L.tspb200_debug_fetch.argtypes = [vp, C.c_char_p, C.c_void_p, i64]
     _libs[path] = L
@@ -449,6 +456,52 @@ class Engine:
         self._ck(self.L.tspb200_population_vns(self.h, None if sl is None else sl.ctypes.data, k, kicks.ctypes.data, iters,
                                                best.ctypes.data, trace.ctypes.data if want_trace else None, C.byref(st)))
         return best, trace, Stats.of(st)
+
+    def population_tabu_begin(self, seeds, slots=None, best_slots=None):
+        """Independent tabu searches (reference tabu(), src/tabusearch.c:188-320) on the resident population, one per seed:
+        chain b works on slot slots[b] (default b) and keeps its best tour in best_slots[b] (default count + b); its random
+        stream is srandom(seeds[b])."""
+        seeds = np.ascontiguousarray(seeds, dtype=np.uint32)
+        k = len(seeds)
+        sl = np.arange(k, dtype=np.int32) if slots is None else np.ascontiguousarray(slots, dtype=np.int32)
+        bs = np.arange(k, 2 * k, dtype=np.int32) if best_slots is None else np.ascontiguousarray(best_slots, dtype=np.int32)
+        if sl.shape != (k,) or bs.shape != (k,):
+            raise TspB200Error(2, f"need {k} slots and {k} best slots, got {sl.shape} and {bs.shape}")
+        self._tabu_chains = 0  # a begin, even a failed one, ends the previous chain set
+        self._ck(self.L.tspb200_population_tabu_begin(self.h, sl.ctypes.data, bs.ctypes.data, k, seeds.ctypes.data))
+        self._tabu_chains = k
+
+    def population_tabu(self, tenures, max_draws: int = 1 << 20):
+        """`iters` iterations of every chain in one launch; tenures[b, t] = chain b's tenure of iteration t, shape (chains,
+        iters).  -> (best[chains], trace[chains, iters] recomputed cost after each masked 2-opt, draws[chains, iters] pairs
+        drawn by each kick, Stats)."""
+        tenures = np.ascontiguousarray(tenures, dtype=np.int32)
+        k = getattr(self, "_tabu_chains", 0)
+        if k == 0:
+            # no chain set begun through this binding: no array crosses (the library sizes them by its own chain count)
+            self._ck(self.L.tspb200_population_tabu(self.h, None, 0, int(max_draws), None, None, None, None))
+            raise TspB200Error(3, "no tabu chain set (population_tabu_begin)")
+        if tenures.ndim != 2 or tenures.shape[0] != k:
+            raise TspB200Error(2, f"tenures must have shape ({k}, iters), got {tenures.shape}")
+        iters = tenures.shape[1]
+        best = np.empty(k, dtype=np.float64)
+        trace = np.empty((k, iters), dtype=np.float64)
+        draws = np.empty((k, iters), dtype=np.int32)
+        st = _Stats()
+        self._ck(self.L.tspb200_population_tabu(self.h, tenures.ctypes.data, iters, int(max_draws), best.ctypes.data,
+                                                trace.ctypes.data, draws.ctypes.data, C.byref(st)))
+        return best, trace, draws, Stats.of(st)
+
+    def population_tabu_list(self, chain: int):
+        """-> (chain's tabu list, n(n-1)/2 int32 in the reference's x_udir_pos layout, its next iteration number)"""
+        out = np.empty(self.n * (self.n - 1) // 2, dtype=np.int32)
+        it = C.c_int32(0)
+        self._ck(self.L.tspb200_population_tabu_fetch(self.h, int(chain), out.ctypes.data, C.byref(it)))
+        return out, it.value
+
+    def population_tabu_end(self):
+        self._ck(self.L.tspb200_population_tabu_end(self.h))
+        self._tabu_chains = 0
 
     # -- multi-GPU
     @staticmethod
