@@ -251,6 +251,31 @@ int tspb200_population_tabu(tspb200_ctx *ctx, const int32_t *tenures, int iters,
 int tspb200_population_tabu_fetch(tspb200_ctx *ctx, int chain, int32_t *list_out, int32_t *next_iter);
 int tspb200_population_tabu_end(tspb200_ctx *ctx);
 
+/* One tabu search (reference tabu(), src/tabusearch.c:188-320) on the resident tour, every iteration of a call on the device:
+ * the semantics of tspb200_population_tabu with one chain, for any tour the list allows (n <= 46340), not only those that
+ * fit one thread block.  The masked 2-opt passes are grid-wide: the FP32-filter scan with the tabu test in its exact path
+ * (the exact scan for GEO, a resident matrix or coordinates FP32 cannot hold), each preceded by the pass's lazy expiry.
+ * begin: zeroes the list (CALLOC, tabusearch.c:196; an allocation of its own, shared with no other entry point), sets the
+ * next iteration number to 1, seeds the search's stream with srandom(seed) and copies the resident tour to the search's
+ * best tour.  Needs an uploaded tour, n <= 46340, distances < 2^24 and one GPU, else TSPB200_E_UNSUPPORTED.
+ * search: for t = 0 .. iters-1, with tenure = tenures[t] and iter = the next iteration number: alg_2opt_tabu(list, iter,
+ * tenure) on the resident tour to the local optimum; trace[t] = the recomputed cost; a strictly cheaper tour is copied to
+ * the best tour; then the kick of tspb200_population_tabu (pairs rand_choice(0, n) twice, drawn until one passes the tests
+ * of tspb200_tabu_kick; applied and stamped with iter), draws[t] = the pairs drawn; the iteration number grows by one.  A
+ * kick that would need more than max_draws (>= 1) pairs gives TSPB200_E_DEVICE_CHECK naming the iteration (the search's
+ * state is then unspecified: begin again).  The list, table, stream, next iteration number and best tour persist until
+ * end, so iters = K1 then K2 equals one call of K1 + K2; iters = 0 changes nothing.  The current tour is the resident tour:
+ * other calls may replace it (tspb200_tour_upload ..) and the search continues from the new one.  The host synchronises
+ * once per batch of launches.  best (may be NULL) = the best tour's cost; trace, draws = iters entries each (may be NULL);
+ * st = moves, passes, evals (passes n(n-3)/2), gpu_ms, launches.  Without begin: TSPB200_E_STATE.
+ * fetch: the list (n(n-1)/2 ints), the next iteration number and the best tour's successor array; each may be NULL.
+ * end: frees the search (so do tspb200_set_instance with another instance and destroy). */
+int tspb200_tabu_search_begin(tspb200_ctx *ctx, uint32_t seed);
+int tspb200_tabu_search(tspb200_ctx *ctx, const int32_t *tenures, int iters, int max_draws, double *best, double *trace,
+                        int32_t *draws, tspb200_stats *st);
+int tspb200_tabu_search_fetch(tspb200_ctx *ctx, int32_t *list_out, int32_t *next_iter, int32_t *best_succ);
+int tspb200_tabu_search_end(tspb200_ctx *ctx);
+
 /* ---- multi-GPU (one process per GPU; the caller bootstraps the id, e.g. over torch.distributed) ---- */
 /* Neighbourhood sharding: with a communicator attached, tspb200_bi_run deals the pair tiles round-robin over the ranks;
  * per pass every rank's packed (delta, i, j) key is stored into every peer's exchange slots over NVLink by the scan kernel

@@ -16,6 +16,7 @@
 
 #include "../../include/tspb200.h"
 #include "tsp_state.cuh"
+#include "tabu_common.cuh"
 
 namespace tspb {
 
@@ -29,6 +30,14 @@ cudaError_t launch_bi_scan_exact(const InstDev &inst, const TourDev &tour, int r
 cudaError_t launch_bi_scan_tabu(const InstDev &inst, const TourDev &tour, int *skip, int iter, int tenure, long long *zl,
                                 unsigned long long *zl_count, long long zl_cap, int grid, cudaStream_t st);
 cudaError_t launch_bi_decode_packed(const TourDev &tour, cudaStream_t st);
+cudaError_t launch_bi_scan_exact_search(const InstDev &inst, const TourDev &tour, TabuSearchDev *S, int *list, int grid,
+                                        cudaStream_t st);
+cudaError_t launch_bi_scan_tabu_fp32(const BiArgs &a, const int *list, const TabuSearchDev *S, int grid, cudaStream_t st);
+int ts_scan_threads();
+int ts_scan_rows();
+cudaError_t launch_ts_init(const TabuSearchArgs &a, Ctl *ctl, int iters, int max_draws, cudaStream_t st);
+cudaError_t launch_ts_expire(const TabuSearchArgs &a, const TourDev &T, int num_sms, cudaStream_t st);
+cudaError_t launch_ts_step(const TabuSearchArgs &a, const InstDev &I, const TourDev &T, cudaStream_t st);
 cudaError_t launch_apply_move(const InstDev &inst, const TourDev &tour, int num_sms, int seed, int timing, bool pdl, bool node_space,
                               int fi_late, cudaStream_t st);
 cudaError_t launch_tile_prune(const BiArgs &a, int TI, int grid_bi, bool pdl, cudaStream_t st);
@@ -224,6 +233,14 @@ struct tspb200_ctx {
     TabuChainState *d_tc_state = nullptr;
     int *d_tc_slots = nullptr;        // current slots, then best slots
     std::vector<int> tc_slots;
+    // the resident tabu search (tspb200_tabu_search_begin .. _end): its list, device state, best tour and the tile plan of
+    // its masked scan
+    bool ts_on = false;
+    int *d_ts_list = nullptr;
+    TabuSearchDev *d_ts = nullptr;
+    int *d_ts_best = nullptr;
+    int *d_ts_tiles = nullptr;        // tile-row prefix sums [ntr + 1], then first tile columns [ntr]
+    int ts_TJ = 0, ts_ntr = 0, ts_ntiles = 0, ts_grid = 0;
 
     // comm
     nccl_comm_t comm = nullptr;
@@ -316,9 +333,16 @@ static void free_tabu_chains(tspb200_ctx *c) {
     c->tc_slots.clear();
 }
 
+static void free_tabu_search(tspb200_ctx *c) {
+    cudaFree(c->d_ts_list); cudaFree(c->d_ts); cudaFree(c->d_ts_best); cudaFree(c->d_ts_tiles);
+    c->d_ts_list = nullptr; c->d_ts = nullptr; c->d_ts_best = nullptr; c->d_ts_tiles = nullptr;
+    c->ts_on = false;
+}
+
 static void free_instance(tspb200_ctx *c) {
     free_tour(c);
     free_tabu_chains(c);
+    free_tabu_search(c);
     cudaFree(c->d_flush);
     c->d_flush = nullptr;
     c->flush_cap = 0;
@@ -559,6 +583,7 @@ int tspb200_set_instance(tspb200_ctx *ctx, const double *xy, int n, int weight_t
         ctx->tabu_session = false;  // sessions belong to the instance they were opened on
         ctx->pop_count = 0;
         free_tabu_chains(ctx);
+        free_tabu_search(ctx);
         ctx->save_n[0] = ctx->save_n[1] = 0;
     }
     ctx->n = n;
@@ -2153,25 +2178,6 @@ int tspb200_population_vns(tspb200_ctx *ctx, const int32_t *slots, int count, co
     return TSPB200_OK;
 }
 
-// glibc srandom(seed) followed by the 310 discarded outputs (GlibcRandom in instances.py): the last 31 values of the
-// recurrence, as the chain kernel continues it
-static void glibc_srandom_state(uint32_t seed, TabuChainState &s) {
-    if (seed == 0) seed = 1;
-    uint32_t x[344];
-    x[0] = seed;
-    for (int i = 1; i < 31; ++i) {  // 16807 x mod (2^31 - 1) on the signed value (Schrage), as glibc computes it
-        const int32_t prev = (int32_t)x[i - 1];
-        const int32_t hi = prev / 127773, lo = prev % 127773;
-        int32_t word = 16807 * lo - 2836 * hi;
-        if (word < 0) word += 2147483647;
-        x[i] = (uint32_t)word;
-    }
-    for (int i = 31; i < 34; ++i) x[i] = x[i - 31];
-    for (int i = 34; i < 344; ++i) x[i] = x[i - 31] + x[i - 3];
-    for (int i = 344 - 31; i < 344; ++i) s.rng[i % 31] = x[i];
-    s.rng_pos = 344 % 31;
-}
-
 // Independent tabu searches (reference tabu(), src/tabusearch.c:188-320) on the resident population: begin checks the
 // slots and the memory the lists need, zeroes the lists (CALLOC, tabusearch.c:196), copies every chain's tour to its best
 // slot and seeds the chains' random streams.  A new begin ends the previous chain set first, so that a failed begin leaves
@@ -2331,6 +2337,181 @@ int tspb200_population_tabu_end(tspb200_ctx *ctx) {
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
     free_tabu_chains(ctx);
+    return TSPB200_OK;
+}
+
+// ---- the resident tabu search (reference tabu(), src/tabusearch.c:188-320) on the resident tour, DESIGN.md §4.9 ----------
+// The semantics of tspb200_population_tabu with one chain, for tours of any size the list allows.  A call enqueues batches of
+// (expiry, masked scan, apply, step) launches and synchronises once per batch (kernels_tabu_search.cu).
+int tspb200_tabu_search_begin(tspb200_ctx *ctx, uint32_t seed) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (!ctx->has_tour) return fail(ctx, TSPB200_E_STATE, "no tour uploaded");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->stream));
+    free_tabu_search(ctx);
+    const int n = ctx->n;
+    if (n > 46340) return fail(ctx, TSPB200_E_UNSUPPORTED, "tabu list index overflows int for n=%d (reference limit)", n);
+    if (!(ctx->dist_bound < 16777216.0)) return fail(ctx, TSPB200_E_UNSUPPORTED, "distances >= 2^24 are not supported by the 2-opt kernels");
+    if (ctx->world > 1) return fail(ctx, TSPB200_E_UNSUPPORTED, "the tabu search is single-GPU");
+    const int path = select_path(ctx);
+    if (path == 2 && !ctx->d_mat) return fail(ctx, TSPB200_E_STATE, "matrix path selected but no resident matrix");
+    const long long len = (long long)n * (n - 1) / 2;
+    // the masked FP32 scan's own tile plan: its one shape (kernels_bi_tabu.cu), exhaustive, one GPU
+    std::vector<int> row_start, row_j0;
+    int T = 0, R = 0, TJ = 0;
+    choose_tile_shape(n, ctx->num_sms, 1, ts_scan_threads(), ts_scan_rows(), 0, true, &T, &R, &TJ);
+    const long long ntiles = tile_plan(n, bi_tile_rows(T, R, 1), TJ, &row_start, &row_j0);
+    double cost = 0;
+    int rc = tspb200_tour_download(ctx, nullptr, &cost);  // the current tour -> ctx->d_succ
+    if (rc) return rc;
+    TabuSearchDev h;
+    memset(&h, 0, sizeof h);
+    glibc_srandom_state(seed, h.s);
+    h.s.next_iter = 1;
+    h.finished = 1;
+    h.best = (long long)cost;
+    if (cudaMalloc(&ctx->d_ts_list, sizeof(int) * (size_t)(len > 0 ? len : 1)) != cudaSuccess ||
+        cudaMalloc(&ctx->d_ts, sizeof(TabuSearchDev)) != cudaSuccess ||
+        cudaMalloc(&ctx->d_ts_best, sizeof(int) * (size_t)n) != cudaSuccess ||
+        cudaMalloc(&ctx->d_ts_tiles, sizeof(int) * (row_start.size() + row_j0.size() + 1)) != cudaSuccess) {
+        const cudaError_t e = cudaGetLastError();
+        free_tabu_search(ctx);
+        return fail(ctx, TSPB200_E_CUDA, "cannot allocate the tabu search (%lld ints of list): %s", len, cudaGetErrorString(e));
+    }
+    CK(cudaMemsetAsync(ctx->d_ts_list, 0, sizeof(int) * (size_t)(len > 0 ? len : 1), ctx->stream));  // CALLOC, tabusearch.c:196
+    CK(cudaMemcpyAsync(ctx->d_ts, &h, sizeof h, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_ts_best, ctx->d_succ, sizeof(int) * (size_t)n, cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->d_ts_tiles, row_start.data(), sizeof(int) * row_start.size(), cudaMemcpyHostToDevice, ctx->stream));
+    if (!row_j0.empty())
+        CK(cudaMemcpyAsync(ctx->d_ts_tiles + row_start.size(), row_j0.data(), sizeof(int) * row_j0.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));  // h and the tile plan are host memory
+    ctx->ts_TJ = TJ;
+    ctx->ts_ntr = (int)row_j0.size();
+    ctx->ts_ntiles = (int)ntiles;
+    long long grid = (long long)ctx->num_sms * bi_blocks_per_sm(T, R);
+    if (grid > ntiles) grid = ntiles > 0 ? ntiles : 1;
+    if (grid > 4096) grid = 4096;  // block_best[] capacity
+    ctx->ts_grid = (int)grid;
+    ctx->ts_on = true;
+    return TSPB200_OK;
+}
+
+int tspb200_tabu_search(tspb200_ctx *ctx, const int32_t *tenures, int iters, int max_draws, double *best, double *trace,
+                        int32_t *draws, tspb200_stats *st) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (!ctx->ts_on) return fail(ctx, TSPB200_E_STATE, "no tabu search (tspb200_tabu_search_begin)");
+    if (!ctx->has_tour) return fail(ctx, TSPB200_E_STATE, "no tour uploaded");
+    if (iters < 0 || (iters > 0 && !tenures) || max_draws < 1) return fail(ctx, TSPB200_E_ARG, "bad arguments (iters >= 0, tenures, max_draws >= 1)");
+    if (ctx->world > 1) return fail(ctx, TSPB200_E_UNSUPPORTED, "the tabu search is single-GPU");
+    CK(cudaSetDevice(ctx->device));
+    const int n = ctx->n;
+    const int path = select_path(ctx);
+    if (path == 2 && !ctx->d_mat) return fail(ctx, TSPB200_E_STATE, "matrix path selected but no resident matrix");
+    const InstDev I = inst_for_path(ctx, path);
+    SCRATCH(d_ten, int *, 3, sizeof(int) * (size_t)(iters > 0 ? iters : 1));
+    SCRATCH(d_trace, long long *, 14, sizeof(long long) * (size_t)(iters > 0 ? iters : 1));
+    SCRATCH(d_draws, int *, 4, sizeof(int) * (size_t)(iters > 0 ? iters : 1));
+    TabuSearchArgs A{ctx->d_ts, ctx->d_ts_list, d_ten, d_trace, d_draws, ctx->d_ts_best};
+    BiArgs a = {};
+    a.inst = I;
+    a.tour = ctx->tour;
+    a.tile_row_start = ctx->d_ts_tiles;
+    a.tile_row_j0 = ctx->d_ts_tiles + ctx->ts_ntr + 1;
+    a.ntr = ctx->ts_ntr;
+    a.ntiles = ctx->ts_ntiles;
+    a.TJ = ctx->ts_TJ;
+    a.rank = 0;
+    a.world = 1;
+    a.fuse_apply = 1;  // the last block publishes the move, the apply launch applies it
+    a.seed_hint = 0;   // a seed could be a tabu move: it would bound the pass below its masked argmin
+    a.packed_tail = (n <= KEY_PACK_MAX_N && 2.0 * ctx->dist_bound < (double)KEY_PACK_MAX_DELTA) ? 1 : 0;
+    a.row_shuffle = 1;
+    int exact_grid = 4 * ctx->num_sms;
+    if (exact_grid > n) exact_grid = n > 0 ? n : 1;
+    int rc = sync_ctl(ctx);
+    if (rc) return rc;
+    const long long passes0 = ctx->h_ctl->passes, moves0 = ctx->h_ctl->moves;
+    CK(cudaEventRecord(ctx->ev0, ctx->stream));
+    if (iters > 0) CK(cudaMemcpyAsync(d_ten, tenures, sizeof(int) * (size_t)iters, cudaMemcpyHostToDevice, ctx->stream));
+    CK(launch_ts_init(A, ctx->d_ctl, iters, max_draws, ctx->stream));
+    long long host_launches = 1;
+    TabuSearchDev h;
+    memset(&h, 0, sizeof h);
+    h.finished = iters == 0;
+    long long batch = 8;
+    const long long batch_cap = n >= 5000 ? 64 : 256;
+    while (!h.finished) {
+        for (long long q = 0; q < batch; ++q) {
+            CK(launch_ts_expire(A, ctx->tour, ctx->num_sms, ctx->stream));
+            if (path == 0) CK(launch_bi_scan_tabu_fp32(a, ctx->d_ts_list, ctx->d_ts, ctx->ts_grid, ctx->stream));
+            else CK(launch_bi_scan_exact_search(I, ctx->tour, ctx->d_ts, ctx->d_ts_list, exact_grid, ctx->stream));
+            CK(launch_apply_move(I, ctx->tour, ctx->num_sms, 0, 0, false, false, 0, ctx->stream));
+            CK(launch_ts_step(A, I, ctx->tour, ctx->stream));
+            host_launches += 4;
+        }
+        if (batch < batch_cap) batch = batch * 2 < batch_cap ? batch * 2 : batch_cap;
+        CK(cudaMemcpyAsync(&h, ctx->d_ts, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+        rc = sync_ctl(ctx);  // (synchronises the stream)
+        if (rc) return rc;
+    }
+    CK(cudaEventRecord(ctx->ev1, ctx->stream));
+    CK(cudaMemcpyAsync(&h, ctx->d_ts, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+    std::vector<long long> h_trace((size_t)iters);
+    std::vector<int> h_draws((size_t)iters);
+    if (iters > 0) {
+        CK(cudaMemcpyAsync(h_trace.data(), d_trace, sizeof(long long) * (size_t)iters, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaMemcpyAsync(h_draws.data(), d_draws, sizeof(int) * (size_t)iters, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    rc = sync_ctl(ctx);
+    if (rc) return rc;
+    ctx->tour_changed = true;         // ctl->done was left set by the search: the next 2-opt run starts afresh
+    if (iters > 0) {
+        ctx->node_dirty = true;       // the tour moved: first improvement rebuilds its node-space tables
+        ctx->fi_cursor_stale = true;
+    }
+    const int done_iters = h.err ? h.err - 2 : iters;  // a failed kick leaves its iteration's trace entry, not its draws
+    if (best) *best = (double)h.best;
+    for (int t = 0; t < iters; ++t) {
+        if (trace) trace[t] = t < done_iters + (h.err ? 1 : 0) ? (double)h_trace[(size_t)t] : 0.0;
+        if (draws) draws[t] = t < done_iters ? h_draws[(size_t)t] : 0;
+    }
+    if (st) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        memset(st, 0, sizeof *st);
+        st->passes = ctx->h_ctl->passes - passes0;
+        st->moves = ctx->h_ctl->moves - moves0;
+        st->evals = st->passes * ((long long)n * (n - 3) / 2);
+        st->launches = host_launches;
+        st->gpu_ms = ms;
+        st->cost = (double)h.best;
+        st->status = TSPB200_LOCAL_OPTIMUM;
+        st->path = path;
+    }
+    if (h.err)
+        return fail(ctx, TSPB200_E_DEVICE_CHECK, "iteration %d: the kick drew max_draws = %d pairs and none passed; the search's state "
+                    "is unspecified (begin again)", h.err - 2, max_draws);
+    return TSPB200_OK;
+}
+
+int tspb200_tabu_search_fetch(tspb200_ctx *ctx, int32_t *list_out, int32_t *next_iter, int32_t *best_succ) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (!ctx->ts_on) return fail(ctx, TSPB200_E_STATE, "no tabu search (tspb200_tabu_search_begin)");
+    CK(cudaSetDevice(ctx->device));
+    const long long len = (long long)ctx->n * (ctx->n - 1) / 2;
+    if (list_out && len) CK(cudaMemcpyAsync(list_out, ctx->d_ts_list, sizeof(int) * (size_t)len, cudaMemcpyDeviceToHost, ctx->stream));
+    if (next_iter) CK(cudaMemcpyAsync(next_iter, &ctx->d_ts->s.next_iter, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    if (best_succ) CK(cudaMemcpyAsync(best_succ, ctx->d_ts_best, sizeof(int) * (size_t)ctx->n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return TSPB200_OK;
+}
+
+int tspb200_tabu_search_end(tspb200_ctx *ctx) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (!ctx->ts_on) return fail(ctx, TSPB200_E_STATE, "no tabu search");
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaStreamSynchronize(ctx->stream));
+    free_tabu_search(ctx);
     return TSPB200_OK;
 }
 

@@ -12,6 +12,7 @@
 // Evaluation is in node space (the enumeration order IS the node order); FP32 filter + FP64 exact check
 // as in the grid-wide kernels.
 #include "tsp_state.cuh"
+#include "tabu_common.cuh"
 
 namespace tspb {
 
@@ -611,38 +612,6 @@ cudaError_t launch_vns_chains(const InstDev &I, int count, int num_sms, int *gri
 // both ends of every listed entry set, and the masked pass reads the list only for entries with both ends marked
 // (tm_tabu).  A table that overflows is rebuilt from the whole list before each masked pass until it fits again; meanwhile
 // every node is marked (every entry is read).  Passes at tenure < 0 are unmasked and need neither the table nor the marks.
-
-// glibc random() on a chain's state (x_k = x_{k-31} + x_{k-3}, output x_k >> 1), then rand_choice(0, n) (reference
-// src/utility.c:752-754: URAND() = random() / RAND_MAX in FP64, scaled by n and truncated), as GlibcRandom.rand_choice
-__device__ __forceinline__ int tc_rand_choice(TabuChainState &st, int n) {
-    const int k = st.rng_pos;
-    const unsigned v = st.rng[k] + st.rng[k >= 3 ? k - 3 : k + 28];
-    st.rng[k] = v;
-    st.rng_pos = k == 30 ? 0 : k + 1;
-    return (int)(__ddiv_rn((double)(v >> 1), 2147483647.0) * (double)n);
-}
-
-// check_tenure (src/tabusearch.c:83-92) on the dense list, as the kick tests it
-__device__ __forceinline__ bool tc_check(int *list, int e, int iter, int tenure) {
-    if (iter < 0 || tenure < 0) return false;
-    const int v = list[e];
-    if (v == 0) return false;
-    if (iter - v > tenure) {
-        list[e] = 0;
-        return false;
-    }
-    return true;
-}
-
-// the kick stamped entry (x, y): one thread adds it to the table unless it is listed already (-1 when the table is full)
-__device__ __forceinline__ void tc_add(TabuChainState &st, int x, int y) {
-    if (st.tab_n < 0) return;
-    const unsigned e = (unsigned)min(x, y) << 16 | (unsigned)max(x, y);
-    for (int k = 0; k < st.tab_n; ++k)
-        if (st.tab[k] == e) return;
-    if (st.tab_n == TABU_TAB) st.tab_n = -1;
-    else st.tab[st.tab_n++] = e;
-}
 
 // Before a masked pass: drops the entries that read zero from the table, or rebuilds it from the list when it has
 // overflowed, then sets marks[].  Block-wide.

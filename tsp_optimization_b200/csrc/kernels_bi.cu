@@ -316,8 +316,8 @@ __device__ __forceinline__ bool tabu_check(const TabuArgs &T, long long e) {
 }
 
 template <bool MASK>
-__global__ void __launch_bounds__(256) bi_scan_exact_kernel(const InstDev inst, const TourDev tour, int rank, int world,
-                                                            int fuse_apply, const TabuArgs tabu) {
+__device__ __forceinline__ void bi_scan_exact_body(const InstDev &inst, const TourDev &tour, int rank, int world, int fuse_apply,
+                                                   const TabuArgs &tabu) {
     __shared__ MoveKey s_keys[8];
     __shared__ int s_last;
     Ctl *ctl = tour.ctl;
@@ -395,6 +395,21 @@ __global__ void __launch_bounds__(256) bi_scan_exact_kernel(const InstDev inst, 
 }
 
 
+template <bool MASK>
+__global__ void __launch_bounds__(256) bi_scan_exact_kernel(const InstDev inst, const TourDev tour, int rank, int world,
+                                                            int fuse_apply, const TabuArgs tabu) {
+    bi_scan_exact_body<MASK>(inst, tour, rank, world, fuse_apply, tabu);
+}
+
+// The resident tabu search's masked pass for instances without the FP32 path: iter and tenure of the running call come from
+// the search's device state.  The pass's own lazy expiry finds nothing left to zero (ts_expire_kernel ran before it).
+__global__ void __launch_bounds__(256) bi_scan_exact_search_kernel(const InstDev inst, const TourDev tour, TabuArgs tabu,
+                                                                   const TabuSearchDev *S) {
+    tabu.iter = S->cur_iter;
+    tabu.tenure = S->cur_tenure;
+    bi_scan_exact_body<true>(inst, tour, 0, 1, 1, tabu);
+}
+
 // ---- host-side launchers -----------------------------------------------------------------------------
 // rows (moves) of one tile for a block of `threads` threads with `rows_per_thread` rows each
 int bi_tile_rows(int threads, int rows_per_thread, int row_shuffle) {
@@ -438,6 +453,14 @@ cudaError_t launch_bi_scan_tabu(const InstDev &inst, const TourDev &tour, int *s
     TabuArgs t;
     t.skip = skip; t.iter = iter; t.tenure = tenure; t.zl = zl; t.zl_count = zl_count; t.zl_cap = zl_cap;
     bi_scan_exact_kernel<true><<<grid, 256, 0, st>>>(inst, tour, 0, 1, 1, t);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_bi_scan_exact_search(const InstDev &inst, const TourDev &tour, TabuSearchDev *S, int *list, int grid,
+                                        cudaStream_t st) {
+    TabuArgs t;
+    t.skip = list; t.iter = 0; t.tenure = 0; t.zl = nullptr; t.zl_count = &S->zl_count; t.zl_cap = 0;
+    bi_scan_exact_search_kernel<<<grid, 256, 0, st>>>(inst, tour, t, S);
     return cudaGetLastError();
 }
 

@@ -125,9 +125,22 @@ __device__ __forceinline__ float pf_dot_const(float nrm, float pf) {
 // shuffles.  A hit costs a few hundred cycles instead of a serial walk over 32 pairs by a single lane.
 constexpr int BI_CB = 4;  // columns per filter check (the prefilter reads its column constants as one float4 per check)
 
-template <int R, bool ATT, bool EXACT32>
-__device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
-                                             int jj0, float thr TSPB_PROBE_ARG(int own_rows)) {
+//
+// MASK (the resident tabu search, kernels_bi_tabu.cu): a pair with delta < 0 whose four edges (a,b), (a,a1), (b,b1), (a,b1)
+// (a = min(u,v), a1 / b1 the successors of a / b, the order of bi_scan_exact_kernel<true>) include one of the list's blocking
+// entries (non-zero, iter - v <= tenure) is not a candidate.  Within one alg_2opt_tabu call that set is fixed, and only pairs
+// with delta < 0 can change the argmin (it starts at 0 with a strict '<'), so testing them here, after the filter, gives the
+// masked argmin.  The list is only read: the lazy expiry of the pass is done before it, exactly, by ts_expire_kernel.
+__device__ __forceinline__ bool bi_tabu_blocks(const int *list, int x, int y, int n, int iter, int tenure) {
+    if (x > y) { const int t = x; x = y; y = t; }
+    const int v = __ldg(&list[(long long)x * n + y - ((long long)(x + 1) * (x + 2)) / 2]);  // x_udir_pos
+    return v != 0 && iter - v <= tenure;
+}
+
+template <int R, bool ATT, bool EXACT32, bool MASK>
+__device__ __forceinline__ MoveKey bi_cold_warp_body(const InstDev &I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
+                                                     int jj0, float thr, const int *list, int iter, int tenure
+                                                     TSPB_PROBE_ARG(int own_rows)) {
     const int lane = threadIdx.x & 31;
     MoveKey best = key_none();
 #pragma unroll 1
@@ -160,6 +173,13 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
                 if (delta < 0) {
                     MoveKey k;
                     k.delta = (int)delta; k.i = min(u, v); k.j = max(u, v); k.pad = 0;
+                    if (MASK) {
+                        const int u1 = node_of(rp1), v1 = node_of(c1);
+                        const int a1 = u < v ? u1 : v1, b1 = u < v ? v1 : u1;
+                        if (bi_tabu_blocks(list, k.i, k.j, n, iter, tenure) || bi_tabu_blocks(list, k.i, a1, n, iter, tenure) ||
+                            bi_tabu_blocks(list, k.j, b1, n, iter, tenure) || bi_tabu_blocks(list, k.i, b1, n, iter, tenure))
+                            k = key_none();
+                    }
                     if (key_less(k, best)) best = k;
                 }
             }
@@ -167,6 +187,30 @@ __device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec,
     }
     __syncwarp();
     return key_warp_min(best);
+}
+
+template <int R, bool ATT, bool EXACT32>
+__device__ __noinline__ MoveKey bi_cold_warp(const InstDev I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
+                                             int jj0, float thr TSPB_PROBE_ARG(int own_rows)) {
+    return bi_cold_warp_body<R, ATT, EXACT32, false>(I, rec, sc, n, p0, Q0, jj0, thr, nullptr, 0, 0 TSPB_PROBE_ARG(own_rows));
+}
+
+// the masked cold path: iter and tenure of the running call come from the search's device state
+template <int R, bool ATT, bool EXACT32>
+__device__ __noinline__ MoveKey bi_cold_warp_tabu(const InstDev I, const float4 *rec, const float4 *sc, int n, int p0, int Q0,
+                                                  int jj0, float thr, const int *list, const TabuSearchDev *S
+                                                  TSPB_PROBE_ARG(int own_rows)) {
+    const int iter = S->cur_iter, tenure = S->cur_tenure;
+    if (iter < 0 || tenure < 0)  // check_tenure neither blocks nor expires: the unmasked pass
+        return bi_cold_warp_body<R, ATT, EXACT32, false>(I, rec, sc, n, p0, Q0, jj0, thr, nullptr, 0, 0 TSPB_PROBE_ARG(own_rows));
+    return bi_cold_warp_body<R, ATT, EXACT32, true>(I, rec, sc, n, p0, Q0, jj0, thr, list, iter, tenure TSPB_PROBE_ARG(own_rows));
+}
+
+template <int R, bool ATT, bool EXACT32, bool MASK>
+__device__ __forceinline__ MoveKey bi_cold_call(const InstDev &I, const float4 *rec, const float4 *sc, int n, int p0, int Q0, int jj0,
+                                                float thr, const int *list, const TabuSearchDev *S TSPB_PROBE_ARG(int own_rows)) {
+    if constexpr (MASK) return bi_cold_warp_tabu<R, ATT, EXACT32>(I, rec, sc, n, p0, Q0, jj0, thr, list, S TSPB_PROBE_ARG(own_rows));
+    else return bi_cold_warp<R, ATT, EXACT32>(I, rec, sc, n, p0, Q0, jj0, thr TSPB_PROBE_ARG(own_rows));
 }
 
 // Stage 2 of the prefilter: does any pair of the R x BI_CB block pass bi_cold_warp's square-root filter?  Same pairs,
@@ -212,8 +256,9 @@ __device__ __forceinline__ bool bi_refilter_warp(const float4 *rec, const float4
 #endif
 // PF: stage-1 prefilter (bi_scan_kernel: exhaustive scans with a large share of pairs per rank, engine.cu) or the square-root
 // filter alone (bi_scan_sqrt_kernel: pruned passes, smaller shares, option "prefilter" = 0).
-template <int BI_THREADS, int R, bool ATT, bool EXACT32, bool PRUNED, bool SHUF, bool PF>
-__device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
+// MASK: the resident tabu search's masked pass (bi_cold_call; exhaustive, one GPU, seed_hint 0: a seed could be tabu)
+template <int BI_THREADS, int R, bool ATT, bool EXACT32, bool PRUNED, bool SHUF, bool PF, bool MASK = false>
+__device__ __forceinline__ void bi_scan_body(const BiArgs &A, const int *tabu_list = nullptr, const TabuSearchDev *tabu = nullptr) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ __align__(8) unsigned long long bars[2];
     __shared__ int s_hint;
@@ -556,8 +601,8 @@ __device__ __forceinline__ void bi_scan_body(const BiArgs &A) {
                 cold = bi_refilter_warp<R, ATT>(rec, sc, n, pL, Q0, jj, thrL);                         \
             }                                                                                          \
             if (cold) {                                                                                \
-                const MoveKey nb = bi_cold_warp<R, ATT, EXACT32>(A.inst, rec, sc, n, pL, Q0, jj, thrL                   \
-                                                                 TSPB_PROBE_ARG(SHUF && L == 31 ? R - 1 : R)); \
+                const MoveKey nb = bi_cold_call<R, ATT, EXACT32, MASK>(A.inst, rec, sc, n, pL, Q0, jj, thrL, tabu_list, tabu \
+                                                                       TSPB_PROBE_ARG(SHUF && L == 31 ? R - 1 : R)); \
                 if ((tid & 31) == L) {                                                                 \
                     atomicAdd(&ctl->cold_calls, 1ull);                                                 \
                     if (key_less(nb, best)) {                                                          \

@@ -112,6 +112,31 @@ struct TabuChainArgs {   // device buffers of one launch of the tabu chain kerne
     long long *counters;   // count * {moves, passes, evals, error: 1 = not a cycle, 2 + t = kick t drew max_draws pairs}
 };
 
+// The resident tabu search (tspb200_tabu_search_*, kernels_tabu_search.cu): what persists between calls (random stream, next
+// iteration number, table, best cost) and the progress of the running call, which every launch of it reads on the device.
+struct TabuSearchDev {
+    TabuChainState s;        // random stream, next iteration number, table of the list entries that may be non-zero
+    int cur_iter, cur_tenure;  // iter and tenure of the running alg_2opt_tabu call (the masked scans read them)
+    int t, iters;            // iterations of this call done / asked for
+    int max_draws;
+    int finished;            // 1: this call's iterations are done or a kick failed: every launch returns at once
+    int err;                 // 0, or 2 + t: the kick of iteration t drew max_draws pairs and none passed
+    unsigned scan_cnt;       // table rebuild from the whole list: non-zero entries found so far
+    unsigned scan_ticket;    // ... blocks of that launch done
+    int pad;
+    unsigned long long zl_count;  // exact-path scans: entries their own lazy expiry zeroed (counted, not logged)
+    long long best;          // cost of the best tour
+};
+
+struct TabuSearchArgs {      // device buffers of the resident tabu search
+    TabuSearchDev *S;
+    int *list;               // n(n-1)/2 ints, x_udir_pos layout
+    const int *tenures;      // iters tenures of the running call
+    long long *trace;        // iters costs after each masked 2-opt
+    int *draws;              // iters pairs drawn by each kick
+    int *best_succ;          // successor array of the best tour
+};
+
 struct Ctl {
     int done;                       // 1 = local optimum reached (all later launches return at once)
     int error;                      // device-side consistency check failed

@@ -37,7 +37,8 @@ ABI_SYMBOLS = [
     "tspb200_tabu_begin", "tspb200_tabu_run", "tspb200_tabu_kick", "tspb200_tabu_end",
     "tspb200_population_upload", "tspb200_population_download", "tspb200_population_costs", "tspb200_population_two_opt",
     "tspb200_population_vns", "tspb200_population_tabu_begin", "tspb200_population_tabu", "tspb200_population_tabu_fetch",
-    "tspb200_population_tabu_end",
+    "tspb200_population_tabu_end", "tspb200_tabu_search_begin", "tspb200_tabu_search", "tspb200_tabu_search_fetch",
+    "tspb200_tabu_search_end",
 ]
 
 
@@ -148,6 +149,12 @@ def load_library(path: str | None = None) -> C.CDLL:
                                               C.POINTER(_Stats)]
         L.tspb200_population_tabu_fetch.argtypes = [vp, C.c_int, C.c_void_p, C.POINTER(C.c_int32)]
         L.tspb200_population_tabu_end.argtypes = [vp]
+    if hasattr(L, "tspb200_tabu_search"):
+        L.tspb200_tabu_search_begin.argtypes = [vp, C.c_uint32]
+        L.tspb200_tabu_search.argtypes = [vp, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_double), C.c_void_p, C.c_void_p,
+                                          C.POINTER(_Stats)]
+        L.tspb200_tabu_search_fetch.argtypes = [vp, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]
+        L.tspb200_tabu_search_end.argtypes = [vp]
     if hasattr(L, "tspb200_debug_fetch"):
         L.tspb200_debug_fetch.argtypes = [vp, C.c_char_p, C.c_void_p, i64]
     _libs[path] = L
@@ -502,6 +509,35 @@ class Engine:
     def population_tabu_end(self):
         self._ck(self.L.tspb200_population_tabu_end(self.h))
         self._tabu_chains = 0
+
+    def tabu_search_begin(self, seed: int):
+        """One tabu search (reference tabu(), src/tabusearch.c:188-320) on the resident tour: zeroes its list, next
+        iteration 1, random stream srandom(seed), best tour = the resident tour."""
+        self._ck(self.L.tspb200_tabu_search_begin(self.h, int(seed) & 0xffffffff))
+
+    def tabu_search(self, tenures, max_draws: int = 1 << 20):
+        """len(tenures) iterations on the device (tenures[t] = the tenure of iteration t).  -> (best cost, trace[iters]
+        recomputed cost after each masked 2-opt, draws[iters] pairs drawn by each kick, Stats)."""
+        tenures = np.ascontiguousarray(tenures, dtype=np.int32).reshape(-1)
+        iters = len(tenures)
+        best = C.c_double(0.0)
+        trace = np.empty(iters, dtype=np.float64)
+        draws = np.empty(iters, dtype=np.int32)
+        st = _Stats()
+        self._ck(self.L.tspb200_tabu_search(self.h, tenures.ctypes.data, iters, int(max_draws), C.byref(best), trace.ctypes.data,
+                                            draws.ctypes.data, C.byref(st)))
+        return best.value, trace, draws, Stats.of(st)
+
+    def tabu_search_fetch(self):
+        """-> (tabu list, n(n-1)/2 int32 in the reference's x_udir_pos layout, next iteration number, best tour's successors)"""
+        out = np.empty(self.n * (self.n - 1) // 2, dtype=np.int32)
+        it = C.c_int32(0)
+        best = np.empty(self.n, dtype=np.int32)
+        self._ck(self.L.tspb200_tabu_search_fetch(self.h, out.ctypes.data, C.byref(it), best.ctypes.data))
+        return out, it.value, best
+
+    def tabu_search_end(self):
+        self._ck(self.L.tspb200_tabu_search_end(self.h))
 
     # -- multi-GPU
     @staticmethod
