@@ -276,6 +276,20 @@ int tspb200_tabu_search(tspb200_ctx *ctx, const int32_t *tenures, int iters, int
 int tspb200_tabu_search_fetch(tspb200_ctx *ctx, int32_t *list_out, int32_t *next_iter, int32_t *best_succ);
 int tspb200_tabu_search_end(tspb200_ctx *ctx);
 
+/* One VNS search (HEU_VNS, reference src/vns.c:103-183) on the resident tour, every iteration of a call on the device: the
+ * semantics of tspb200_population_vns with one chain, for tours of any size (not only those that fit one thread block).
+ * For t = 0 .. iters-1: the kick of tspb200_vns_kick with kicks[3t .. 3t+2] on the incumbent; alg_2opt (the first-improvement
+ * run of tspb200_fi_run, from a fresh sweep) to the local optimum; trace[t] = the kicked cost plus the deltas; a cost strictly
+ * below the incumbent's makes that tour the incumbent, else the search goes back to the incumbent.  The incumbent at entry is
+ * the resident tour (its cost is recomputed); at return the resident tour is the incumbent and *best (may be NULL) its cost.
+ * Nothing else persists, so iters = K1 then K2 (with the next kicks) equals one call of K1 + K2; iters = 0 returns the
+ * current cost and changes nothing.  The copy of the incumbent is the call's own (tspb200_tour_save slots are untouched).
+ * Every triple is checked before anything is enqueued: a bad one gives TSPB200_E_ARG naming the iteration, with the tour
+ * unchanged.  The host synchronises once per batch of launches.  trace = iters entries (may be NULL); st = moves, passes
+ * (FI sweeps), evals (pairs swept), gpu_ms, launches, summed over the call.  No tour: TSPB200_E_STATE; the matrix path forced
+ * without a resident matrix: TSPB200_E_STATE; several GPUs: TSPB200_E_UNSUPPORTED. */
+int tspb200_vns_search(tspb200_ctx *ctx, const int32_t *kicks, int iters, double *best, double *trace, tspb200_stats *st);
+
 /* ---- multi-GPU (one process per GPU; the caller bootstraps the id, e.g. over torch.distributed) ---- */
 /* Neighbourhood sharding: with a communicator attached, tspb200_bi_run deals the pair tiles round-robin over the ranks;
  * per pass every rank's packed (delta, i, j) key is stored into every peer's exchange slots over NVLink by the scan kernel

@@ -38,6 +38,8 @@ int ts_scan_rows();
 cudaError_t launch_ts_init(const TabuSearchArgs &a, Ctl *ctl, int iters, int max_draws, cudaStream_t st);
 cudaError_t launch_ts_expire(const TabuSearchArgs &a, const TourDev &T, int num_sms, cudaStream_t st);
 cudaError_t launch_ts_step(const TabuSearchArgs &a, const InstDev &I, const TourDev &T, cudaStream_t st);
+cudaError_t launch_vns_step(const VnsSearchArgs &a, const InstDev &I, const TourDev &T, int start, int iters, int num_sms,
+                            cudaStream_t st);
 cudaError_t launch_apply_move(const InstDev &inst, const TourDev &tour, int num_sms, int seed, int timing, bool pdl, bool node_space,
                               int fi_late, cudaStream_t st);
 cudaError_t launch_tile_prune(const BiArgs &a, int TI, int grid_bi, bool pdl, cudaStream_t st);
@@ -2104,6 +2106,20 @@ int tspb200_population_two_opt(tspb200_ctx *ctx, int mode, const int32_t *slots,
     return TSPB200_OK;
 }
 
+// The rules of tspb200_vns_kick (reference vns.c:25-50) for `count` triples: sorted copies go to `sorted`; -1 when all pass,
+// else the index of the first triple that is not three distinct, non-adjacent tour indices in [0, n).
+static long long sort_vns_kicks(const int32_t *kicks, size_t count, int n, int32_t *sorted) {
+    for (size_t q = 0; q < count; ++q) {
+        int i1 = kicks[3 * q], i2 = kicks[3 * q + 1], i3 = kicks[3 * q + 2];
+        if (i1 > i2) std::swap(i1, i2);
+        if (i1 > i3) std::swap(i1, i3);
+        if (i2 > i3) std::swap(i2, i3);
+        if (i1 < 0 || i3 >= n || i2 - i1 < 2 || i3 - i2 < 2) return (long long)q;
+        sorted[3 * q] = i1; sorted[3 * q + 1] = i2; sorted[3 * q + 2] = i3;
+    }
+    return -1;
+}
+
 // Independent VNS chains (HEU_VNS, reference src/vns.c:103-183) on the listed slots, one thread block per chain: kicks[(b*iters +
 // t)*3 ..] are chain b's tour indices of iteration t.  Every triple is checked before anything is launched, so a bad one
 // leaves the population as it was.
@@ -2116,15 +2132,11 @@ int tspb200_population_vns(tspb200_ctx *ctx, const int32_t *slots, int count, co
     const int n = ctx->n;
     const size_t nk = (size_t)count * (size_t)iters;
     std::vector<int32_t> sorted(3 * nk);
-    for (size_t q = 0; q < nk; ++q) {  // the rules of tspb200_vns_kick (reference vns.c:25-50)
-        int i1 = kicks[3 * q], i2 = kicks[3 * q + 1], i3 = kicks[3 * q + 2];
-        if (i1 > i2) std::swap(i1, i2);
-        if (i1 > i3) std::swap(i1, i3);
-        if (i2 > i3) std::swap(i2, i3);
-        if (i1 < 0 || i3 >= n || i2 - i1 < 2 || i3 - i2 < 2)
-            return fail(ctx, TSPB200_E_ARG, "chain %d, iteration %d: kick (%d, %d, %d) is not three distinct, non-adjacent tour indices in [0, %d)",
-                        (int)(q / (size_t)iters), (int)(q % (size_t)iters), kicks[3 * q], kicks[3 * q + 1], kicks[3 * q + 2], n);
-        sorted[3 * q] = i1; sorted[3 * q + 1] = i2; sorted[3 * q + 2] = i3;
+    const long long bad = sort_vns_kicks(kicks, nk, n, sorted.data());
+    if (bad >= 0) {
+        const size_t q = (size_t)bad;
+        return fail(ctx, TSPB200_E_ARG, "chain %d, iteration %d: kick (%d, %d, %d) is not three distinct, non-adjacent tour indices in [0, %d)",
+                    (int)(q / (size_t)iters), (int)(q % (size_t)iters), kicks[3 * q], kicks[3 * q + 1], kicks[3 * q + 2], n);
     }
     CK(cudaSetDevice(ctx->device));
     const int path = select_path(ctx);
@@ -2512,6 +2524,96 @@ int tspb200_tabu_search_end(tspb200_ctx *ctx) {
     CK(cudaSetDevice(ctx->device));
     CK(cudaStreamSynchronize(ctx->stream));
     free_tabu_search(ctx);
+    return TSPB200_OK;
+}
+
+// ---- the resident VNS search (reference HEU_VNS, src/vns.c:103-183) on the resident tour, DESIGN.md §4.9 -------------------
+// The semantics of tspb200_population_vns with one chain, for tours of any size.  A call enqueues batches of the launches of
+// tspb200_fi_run (search, apply) each followed by a step launch, and synchronises once per batch (kernels_vns_search.cu).
+// The incumbent lives in scratch of its own for the length of the call: nothing persists between calls.
+int tspb200_vns_search(tspb200_ctx *ctx, const int32_t *kicks, int iters, double *best, double *trace, tspb200_stats *st) {
+    if (!ctx || !ctx->stream) return fail(ctx, TSPB200_E_CUDA, "context has no CUDA device");
+    if (!ctx->has_tour) return fail(ctx, TSPB200_E_STATE, "no tour uploaded");
+    if (iters < 0 || (iters > 0 && !kicks)) return fail(ctx, TSPB200_E_ARG, "bad arguments (iters >= 0, kicks)");
+    if (ctx->world > 1) return fail(ctx, TSPB200_E_UNSUPPORTED, "the VNS search is single-GPU");
+    const int n = ctx->n;
+    std::vector<int32_t> sorted(3 * (size_t)iters);
+    const long long bad = sort_vns_kicks(kicks, (size_t)iters, n, sorted.data());
+    if (bad >= 0)
+        return fail(ctx, TSPB200_E_ARG, "iteration %lld: kick (%d, %d, %d) is not three distinct, non-adjacent tour indices in [0, %d)",
+                    bad, kicks[3 * bad], kicks[3 * bad + 1], kicks[3 * bad + 2], n);
+    CK(cudaSetDevice(ctx->device));
+    const int path = select_path(ctx);
+    if (path == 2 && !ctx->d_mat) return fail(ctx, TSPB200_E_STATE, "matrix path selected but no resident matrix");
+    const InstDev I = inst_for_path(ctx, path);
+    if (iters == 0) {
+        double cost = 0;
+        int rc = tspb200_tour_cost(ctx, &cost);
+        if (rc) return rc;
+        if (best) *best = cost;
+        if (st) { memset(st, 0, sizeof *st); st->cost = cost; st->status = TSPB200_LOCAL_OPTIMUM; st->path = path; }
+        return TSPB200_OK;
+    }
+    SCRATCH(d_inc_rec, float4 *, 20, sizeof(float4) * (size_t)(n + 1));
+    SCRATCH(d_inc_pos, int *, 21, sizeof(int) * (size_t)n);
+    SCRATCH(d_kscr, float4 *, 22, sizeof(float4) * (size_t)n);
+    SCRATCH(d_state, long long *, 23, sizeof(VnsSearchDev) + sizeof(long long) * (size_t)ctx->num_sms);
+    SCRATCH(d_kicks, int *, 3, sizeof(int) * 3 * (size_t)iters);
+    SCRATCH(d_trace, long long *, 14, sizeof(long long) * (size_t)iters);
+    VnsSearchDev *d_S = reinterpret_cast<VnsSearchDev *>(d_state);
+    VnsSearchArgs A{d_S, d_kicks, d_trace, d_inc_rec, d_inc_pos, d_kscr, d_state + sizeof(VnsSearchDev) / sizeof(long long)};
+    int grid = ctx->opt_grid > 0 ? ctx->opt_grid : 2 * ctx->num_sms;  // the search launches of tspb200_fi_run
+    if (grid > n - 1) grid = n - 1;
+    const bool pdl = ctx->opt_pdl != 0;
+    int rc = sync_ctl(ctx);
+    if (rc) return rc;
+    const long long passes0 = ctx->h_ctl->passes, moves0 = ctx->h_ctl->moves, swept0 = ctx->h_ctl->pairs_swept;
+    CK(cudaEventRecord(ctx->ev0, ctx->stream));
+    CK(cudaMemcpyAsync(d_kicks, sorted.data(), sizeof(int) * 3 * (size_t)iters, cudaMemcpyHostToDevice, ctx->stream));
+    CK(launch_vns_step(A, I, ctx->tour, 1, iters, ctx->num_sms, ctx->stream));
+    long long host_launches = 1;
+    ctx->fi_parity = 0;
+    VnsSearchDev h;
+    memset(&h, 0, sizeof h);
+    long long batch = ctx->opt_batch > 0 ? ctx->opt_batch : 8;  // grows: a call of a few iterations on a small tour stops early
+    const long long batch_cap = ctx->opt_batch > 0 ? ctx->opt_batch : 64;
+    while (!h.finished) {
+        for (long long q = 0; q < batch; ++q) {
+            const int late = ctx->opt_fi_late ? 1 + (int)(ctx->fi_parity++ & 1) : 0;
+            CK(launch_fi_search(I, ctx->tour, 0, 1, nullptr, late, grid, pdl, ctx->stream));
+            CK(launch_apply_move(I, ctx->tour, ctx->num_sms, 0, 0, pdl, true, late, ctx->stream));
+            CK(launch_vns_step(A, I, ctx->tour, 0, iters, ctx->num_sms, ctx->stream));
+            host_launches += 3;
+        }
+        if (batch < batch_cap) batch = batch * 2 < batch_cap ? batch * 2 : batch_cap;
+        CK(cudaMemcpyAsync(&h, d_S, sizeof h, cudaMemcpyDeviceToHost, ctx->stream));
+        rc = sync_ctl(ctx);  // (synchronises the stream)
+        if (rc) return rc;
+    }
+    CK(cudaEventRecord(ctx->ev1, ctx->stream));
+    std::vector<long long> h_trace((size_t)iters);
+    CK(cudaMemcpyAsync(h_trace.data(), d_trace, sizeof(long long) * (size_t)iters, cudaMemcpyDeviceToHost, ctx->stream));
+    rc = sync_ctl(ctx);
+    if (rc) return rc;
+    ctx->tour_changed = true;         // ctl->done was left set by the search: the next 2-opt run starts afresh
+    ctx->node_dirty = true;           // the tour went back to the incumbent: first improvement rebuilds its node-space tables
+    ctx->fi_cursor_stale = true;
+    if (best) *best = (double)h.best;
+    if (trace)
+        for (int t = 0; t < iters; ++t) trace[t] = (double)h_trace[(size_t)t];
+    if (st) {
+        float ms = 0;
+        CK(cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1));
+        memset(st, 0, sizeof *st);
+        st->passes = ctx->h_ctl->passes - passes0;
+        st->moves = ctx->h_ctl->moves - moves0;
+        st->evals = ctx->h_ctl->pairs_swept - swept0;
+        st->launches = host_launches;
+        st->gpu_ms = ms;
+        st->cost = (double)h.best;
+        st->status = TSPB200_LOCAL_OPTIMUM;
+        st->path = path;
+    }
     return TSPB200_OK;
 }
 

@@ -137,6 +137,26 @@ struct TabuSearchArgs {      // device buffers of the resident tabu search
     int *best_succ;          // successor array of the best tour
 };
 
+// The resident VNS search (tspb200_vns_search, kernels_vns_search.cu): the progress of the running call, which every step
+// launch reads on the device.  Nothing persists between calls.
+struct VnsSearchDev {
+    int t;                   // the running iteration
+    int iters;               // iterations asked for
+    int finished;            // 1: this call's iterations are done: every step launch returns at once
+    int pad;
+    long long best;          // cost of the incumbent
+};
+
+struct VnsSearchArgs {       // device buffers of the resident VNS search
+    VnsSearchDev *S;
+    const int *kicks;        // iters sorted tour-index triples
+    long long *trace;        // iters costs after each iteration's 2-opt
+    float4 *inc_rec;         // the incumbent: records 0..n (rec[n] mirrors rec[0]) ...
+    int *inc_pos;            // ... and positions
+    float4 *scratch;         // the kick's blocks X and Y
+    long long *part;         // per-block partial sums of the tour cost
+};
+
 struct Ctl {
     int done;                       // 1 = local optimum reached (all later launches return at once)
     int error;                      // device-side consistency check failed

@@ -38,7 +38,7 @@ ABI_SYMBOLS = [
     "tspb200_population_upload", "tspb200_population_download", "tspb200_population_costs", "tspb200_population_two_opt",
     "tspb200_population_vns", "tspb200_population_tabu_begin", "tspb200_population_tabu", "tspb200_population_tabu_fetch",
     "tspb200_population_tabu_end", "tspb200_tabu_search_begin", "tspb200_tabu_search", "tspb200_tabu_search_fetch",
-    "tspb200_tabu_search_end",
+    "tspb200_tabu_search_end", "tspb200_vns_search",
 ]
 
 
@@ -155,6 +155,8 @@ def load_library(path: str | None = None) -> C.CDLL:
                                           C.POINTER(_Stats)]
         L.tspb200_tabu_search_fetch.argtypes = [vp, C.c_void_p, C.POINTER(C.c_int32), C.c_void_p]
         L.tspb200_tabu_search_end.argtypes = [vp]
+    if hasattr(L, "tspb200_vns_search"):
+        L.tspb200_vns_search.argtypes = [vp, C.c_void_p, C.c_int, C.POINTER(C.c_double), C.c_void_p, C.POINTER(_Stats)]
     if hasattr(L, "tspb200_debug_fetch"):
         L.tspb200_debug_fetch.argtypes = [vp, C.c_char_p, C.c_void_p, i64]
     _libs[path] = L
@@ -538,6 +540,18 @@ class Engine:
 
     def tabu_search_end(self):
         self._ck(self.L.tspb200_tabu_search_end(self.h))
+
+    def vns_search(self, kicks):
+        """One VNS search (reference HEU_VNS, src/vns.c:103-183) on the resident tour: kicks[t] = the three tour indices of
+        iteration t, shape (iters, 3) (instances.vns_kick_indices).  The resident tour is left as the incumbent.
+        -> (incumbent cost, trace[iters] cost after each iteration's 2-opt, Stats)."""
+        kicks = np.ascontiguousarray(kicks, dtype=np.int32).reshape(-1, 3)
+        iters = len(kicks)
+        best = C.c_double(0.0)
+        trace = np.empty(iters, dtype=np.float64)
+        st = _Stats()
+        self._ck(self.L.tspb200_vns_search(self.h, kicks.ctypes.data, iters, C.byref(best), trace.ctypes.data, C.byref(st)))
+        return best.value, trace, Stats.of(st)
 
     # -- multi-GPU
     @staticmethod
